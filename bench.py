@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- throughput of the sparse-A x dense-B hot path on B200 (one JSON line on stdout).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c4|c5] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c2|c1|c3|c4|c5] [--impl b200|reference] [--dump-outputs DIR]
 
 Headline workload (BASELINE.json configs[1], "C2"): libxsmm_spmdm, bf16 inputs / fp32 accumulate,
 M = K = N = 4096, A 99 % zeros, beta = 0.  One STEP = one whole multiply the way samples/spmdm/spmdm.c:88-111
@@ -27,6 +27,11 @@ the barriers and the max-over-ranks of the device time only.
     scaling; reported device-resident and end to end at every N, so that the 1/2/4/8 curve can be read off.
 
 --impl reference times the reference CPU implementation on the same workload (rank 0 only).
+
+--dump-outputs DIR writes what the last timed step of the headline workload computed (C) as DIR/<name>.npy, so that two
+builds can be compared output for output: the inputs are seeded, identical from run to run for the same arguments.  An output
+larger than DUMP_BYTES is written as a fixed sample of its elements, see dump_outputs().  With N > 1 only rank 0 writes: its
+own C for the replicated C2, its own column panel of C for the column-sharded fsspmdm workloads.
 """
 import argparse
 import importlib
@@ -82,6 +87,7 @@ WORKLOADS["soa-b"] = dict(kind="soa", case="bsp_tet4_4_stiffV_0_d", sparse="B", 
                           desc="dcsr_soa, B sparse: [9][35][8] tensors x EDGE tet4 order 4 stiffV_0 (35x35, 108 nnz), 65536 elements, beta=1")
 FP32_FMA_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12      # 74.4: 148 SMs x 128 FMA lanes at the 1965 MHz the CUDA-core kernels run at (nominal; no measured figure in MEASURED_PEAKS.json)
 L2_BYTES = 126 << 20
+DUMP_BYTES = 48 << 20      # --dump-outputs writes at most this much (a dump stays below 64 MB)
 
 
 def peaks():
@@ -229,7 +235,7 @@ def fs_operator(xs, wl):
                                          np.float64 if wl["dtype"] == "f64" else np.float32, seed=1)
 
 
-def run_soa_gpu(xs, wl, steps, warmup):
+def run_soa_gpu(xs, wl, steps, warmup, dump=False):
     d = np.load(os.path.join(ROOT, "tests", "golden", "csr_soa.npz"))
     key = wl["case"]
     M, K, N, soa, _ = (int(x) for x in d[key + "_shape"])
@@ -260,6 +266,7 @@ def run_soa_gpu(xs, wl, steps, warmup):
     st.synchronize()
     total_ms = t0.elapsed_ms(t1)
     xs.check()
+    outputs = {"C": ring[(warmup + steps - 1) % nsets][1].to_numpy(va.dtype, (E, M, N, soa))} if dump else None
     nnz = len(va)
     if bsp:      # A [M][K][soa]: the rows k with nonzeros in B are read.  beta = 0: columns 0 .. ncols-1 of C are written (ncols =
         k_used = int(np.count_nonzero(np.diff(rp)))       # 1 + the largest column index of B); beta = 1: a column without nonzeros
@@ -273,11 +280,23 @@ def run_soa_gpu(xs, wl, steps, warmup):
         bytes_ = esz * E * N * soa * (cols_used + rows_touched * (2 if float(wl["beta"]) != 0.0 else 1))
         flops = 2.0 * nnz * N * soa * E
     yield dict(total_ms=total_ms, launches=xs.launch_count() - l0, nnz=nnz, flops=flops, geo=dict(baked=op.is_baked, M=M, K=K, N=N, soa=soa, elements=E, sparse_operand="B" if bsp else "A"),
-               kernel_ms=total_ms / steps, kernel_bytes=bytes_, kernel_name=xs.last_compute_kernel(), parts={}, step_bytes=bytes_, ring_sets=nsets, ring_bytes=nsets * (bB + bC))
+               kernel_ms=total_ms / steps, kernel_bytes=bytes_, kernel_name=xs.last_compute_kernel(), parts={}, step_bytes=bytes_, ring_sets=nsets, ring_bytes=nsets * (bB + bC),
+               outputs=outputs)
     for bufs in ring:
         for b in bufs:
             b.free()
     op.destroy()
+
+
+def dump_outputs(directory, outputs):
+    """writes each output array as <directory>/<name>.npy.  One larger than its share of DUMP_BYTES is written as the 1-D sample
+    a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]: the same positions for the same shape."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in outputs.items():
+        n = DUMP_BYTES // len(outputs) // a.itemsize
+        if a.size > n:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, n, replace=False))]
+        np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def fill_device_random(xs, dbuf, nbytes, dtype, seed):
@@ -295,7 +314,7 @@ def fill_device_random(xs, dbuf, nbytes, dtype, seed):
 # ------------------------------------------------------------------------------------------------------
 # GPU arm
 # ------------------------------------------------------------------------------------------------------
-def run_spmdm_gpu(xs, wl, steps, warmup, want_e2e=True):
+def run_spmdm_gpu(xs, wl, steps, warmup, want_e2e=True, dump=False):
     bf16 = wl["dtype"] == "bf16"
     dt = xs.LIBXSMM_SPMDM_DATATYPE_BFLOAT16 if bf16 else xs.LIBXSMM_SPMDM_DATATYPE_F32
     ta, tb, tc = wl["trans"]
@@ -342,6 +361,7 @@ def run_spmdm_gpu(xs, wl, steps, warmup, want_e2e=True):
     st.synchronize()
     launches = xs.launch_count() - l0
     total_ms = t_first.elapsed_ms(t_last)
+    outputs = {"C": ring[(warmup + steps - 1) % nsets][2].to_numpy(np.float32, C0.shape)} if dump else None
     for i in range(steps):
         step(warmup + steps + i, ev[i])
     st.synchronize()
@@ -351,7 +371,7 @@ def run_spmdm_gpu(xs, wl, steps, warmup, want_e2e=True):
     res = dict(total_ms=total_ms, launches=launches, nnz=nnz, flops=2.0 * nnz * N, geo=geo,
                kernel_ms=comp_ms, kernel_bytes=b_compute, kernel_name=xs.last_compute_kernel(), dense_flops=2.0 * M * N * K,
                parts={"slice_ms": slice_ms, "compute_ms": comp_ms, "slice_bytes": b_slice, "compute_bytes": b_compute},
-               step_bytes=b_slice + b_compute, ring_sets=nsets, ring_bytes=nsets * set_bytes)
+               step_bytes=b_slice + b_compute, ring_sets=nsets, ring_bytes=nsets * set_bytes, outputs=outputs)
     yield res
     # ---- e2e: host pointers through the C ABI -------------------------------------------------------
     if want_e2e:
@@ -377,7 +397,7 @@ def run_spmdm_gpu(xs, wl, steps, warmup, want_e2e=True):
     p.destroy()
 
 
-def run_fs_gpu(xs, wl, steps, warmup, world, want_e2e=True, rank=0):
+def run_fs_gpu(xs, wl, steps, warmup, world, want_e2e=True, rank=0, dump=False):
     """C3 / C5: the N columns of ONE global problem split into contiguous panels (sharding.column_panels: multiples of 16), one
     per rank; every rank holds its own dense B / C panel (ld = panel width) and a replica of the operator."""
     dbl = wl["dtype"] == "f64"
@@ -426,9 +446,10 @@ def run_fs_gpu(xs, wl, steps, warmup, world, want_e2e=True, rank=0):
     launches = xs.launch_count() - l0
     total_ms = t_first.elapsed_ms(t_last)
     xs.check()
+    outputs = {"C": ring[(warmup + steps - 1) % nsets][1].to_numpy(dtype, (wl["M"], N))} if dump else None
     yield dict(total_ms=total_ms, launches=launches, nnz=nnz, flops=2.0 * nnz * N, geo=dict(sparse=op.is_sparse, baked=op.is_baked, first_column=n0, columns_per_rank=N),
                kernel_ms=total_ms / steps, kernel_bytes=fs_bytes(wl, N), kernel_name=xs.last_compute_kernel(),
-               parts={}, step_bytes=fs_bytes(wl, N), ring_sets=nsets, ring_bytes=nsets * (bB + bC))
+               parts={}, step_bytes=fs_bytes(wl, N), ring_sets=nsets, ring_bytes=nsets * (bB + bC), outputs=outputs)
     if want_e2e:
         Ne = min(N, 1 << 20)                      # host panel of at most 2^20 columns per step (537 MB + 1.26 GB for fp64)
         ope = make_operator(Ne) if Ne != N else op
@@ -566,7 +587,10 @@ def main():
     ap.add_argument("--cpu-budget", type=float, default=12.0, help="seconds of reference CPU time for the headline cpu_baseline (a quarter of it per secondary workload)")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the headline workload's last timed step to DIR/<name>.npy (rank 0's part when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     args.warmup = max(args.warmup, 3)
     wl = WORKLOADS[args.workload]
     rank = int(os.environ.get("RANK", "0"))
@@ -629,7 +653,7 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.SUM)
         return float(t.item())
 
-    def run(wl_, want_e2e, sample_clocks, shard=1):
+    def run(wl_, want_e2e, sample_clocks, shard=1, dump=False):
         """one workload on this rank.  shard = 1: the whole problem on every rank (replicas).  shard = world: this rank's
         N / world column panel of ONE global problem (fsspmdm; SURVEY.md section 8e)."""
         # the clock sampler (nvidia-smi every 200 ms) runs from before the warm-up until after the end-to-end
@@ -640,10 +664,10 @@ def main():
             time.sleep(0.3)
         if wl_["kind"] == "soa":
             want_e2e = False
-            gen = run_soa_gpu(xs, wl_, args.steps, args.warmup)
+            gen = run_soa_gpu(xs, wl_, args.steps, args.warmup, dump)
         else:
-            gen = run_spmdm_gpu(xs, wl_, args.steps, args.warmup, want_e2e) if wl_["kind"] == "spmdm" else \
-                run_fs_gpu(xs, wl_, args.steps, args.warmup, shard, want_e2e, rank if shard > 1 else 0)
+            gen = run_spmdm_gpu(xs, wl_, args.steps, args.warmup, want_e2e, dump) if wl_["kind"] == "spmdm" else \
+                run_fs_gpu(xs, wl_, args.steps, args.warmup, shard, want_e2e, rank if shard > 1 else 0, dump)
         assert next(gen) == "ready"
         barrier()
         res = next(gen)
@@ -690,7 +714,9 @@ def main():
                 "h2d_bytes_per_step": int(e["h2d"]), "d2h_bytes_per_step": int(e["d2h"]),
                 "api": "libxsmm_spmdm_exec_host" if wl_["kind"] == "spmdm" else "libxsmm_[sd]fsspmdm_execute (host pointers)"}
 
-    res, e2e, clocks = run(wl, not args.no_e2e, rank == 0, shard=(world if wl["kind"] == "fsspmdm" else 1))
+    res, e2e, clocks = run(wl, not args.no_e2e, rank == 0, shard=(world if wl["kind"] == "fsspmdm" else 1), dump=bool(args.dump_outputs) and rank == 0)
+    if res["outputs"] is not None:
+        dump_outputs(args.dump_outputs, res.pop("outputs"))
     ms_per_step = res["total_ms"] / args.steps
     value = res["flops_all"] / (ms_per_step * 1e6)
     achieved = res["kernel_bytes"] / (res["kernel_ms"] * 1e6)
