@@ -413,7 +413,11 @@ bool fs_tc_launch(const FsTc* t, const void* dB, void* dC, long long ncols, long
   // C as a tensor of (ncols, M) for the store engine: rows past M and columns past ncols of a box are clipped by the hardware
   CUtensorMap cmap = map;
   int epi = t->epi;
-  if (2 == epi && !make_tensor_map_2d(&cmap, dC, 4, (unsigned long long)ncols, (unsigned long long)t->M, (unsigned long long)ldc * 4, FT_BN, FT_CBOX_ROWS)) { cmap = map; epi = 1; }   // unaligned C
+  // The store engine clips a box at the tensor's last column only to a 16-byte boundary: with ncols not a multiple of four
+  // it would write (beta = 0: zeros) or read-modify-write (beta = 1) up to three columns past the panel, which belong to the
+  // caller (the dense dispatch entry takes any column count).  Per-thread stores write exactly [0, ncols).
+  if (0 != (ncols & 3)) epi = (0 == epi) ? 0 : 1;
+  if (2 == epi &&!make_tensor_map_2d(&cmap, dC, 4, (unsigned long long)ncols, (unsigned long long)t->M, (unsigned long long)ldc * 4, FT_BN, FT_CBOX_ROWS)) { cmap = map; epi = 1; }   // unaligned C
   if (2 == epi) fsspmdm_tc_kernel<2><<<grid, FT_THREADS, t->smem, stream>>>(map, cmap, a);
   else if (1 == epi) fsspmdm_tc_kernel<1><<<grid, FT_THREADS, t->smem, stream>>>(map, cmap, a);
   else fsspmdm_tc_kernel<0><<<grid, FT_THREADS, t->smem, stream>>>(map, cmap, a);

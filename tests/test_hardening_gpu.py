@@ -238,7 +238,7 @@ def test_concurrent_execute_on_host_panels(gpu, oracle):
     xs.check()
 
 
-@pytest.mark.parametrize("kind", ["spmdm-f32", "spmdm-bf16", "fsspmdm-regs", "fsspmdm-strip", "csr-soa"])
+@pytest.mark.parametrize("kind", ["spmdm-f32", "spmdm-bf16", "fsspmdm-regs", "fsspmdm-strip", "fsspmdm-tc", "csr-soa"])
 def test_guard_bands_stay_intact(gpu, oracle, monkeypatch, kind):
     """compute-sanitizer is closed on this GPU pool (profiles/r02_compute_sanitizer_closed.log), so out-of-bounds WRITES are
     hunted the plain way: every output (and every input, which must not be written at all) sits between two 64 KiB guard
@@ -247,15 +247,16 @@ def test_guard_bands_stay_intact(gpu, oracle, monkeypatch, kind):
     xs = gpu
     G = 1 << 16
 
-    def guarded(arr):
-        raw = np.full(2 * G + arr.nbytes, 0xA5, np.uint8)
-        raw[G:G + arr.nbytes] = arr.view(np.uint8).ravel()
+    def guarded(arr, shift=0):
+        raw = np.full(2 * G + shift + arr.nbytes, 0xA5, np.uint8)
+        raw[G + shift:G + shift + arr.nbytes] = arr.view(np.uint8).ravel()
         d = xs.DeviceBuffer.from_numpy(raw)
         return d, raw
 
-    def check(d, raw, nbytes, changed_ok):
+    def check(d, raw, nbytes, changed_ok, shift=0):
         got = d.to_numpy(np.uint8, raw.shape)
-        assert np.array_equal(got[:G], raw[:G]) and np.array_equal(got[G + nbytes:], raw[G + nbytes:]), "guard band overwritten"
+        lo, hi = G + shift, G + shift + nbytes
+        assert np.array_equal(got[:lo], raw[:lo]) and np.array_equal(got[hi:], raw[hi:]), "guard band overwritten"
         if not changed_ok:
             assert np.array_equal(got, raw), "input buffer was written"
         d.free()
@@ -274,6 +275,28 @@ def test_guard_bands_stay_intact(gpu, oracle, monkeypatch, kind):
                 xs.synchronize()
                 p.destroy()
                 check(dA, rA, A.nbytes, False); check(dB, rB, B.nbytes, False); check(dC, rC, C0.nbytes, True)
+    elif kind == "fsspmdm-tc":
+        # dense fp32 operator on the tensor-core kernel: one tile, a panel of a wider matrix, several tiles per CTA, and a C
+        # the store engine cannot address (4 bytes past an aligned base: per-thread stores)
+        from test_fsspmdm_tc_gpu import K4F, persistent_n, sm_count
+        monkeypatch.setenv("LIBXSMM_B200_FSSPMDM_TC", "1")
+        monkeypatch.delenv("LIBXSMM_B200_K4F_EPI", raising=False)
+        M, K = 150, 64
+        a = rng.uniform(-1, 1, (M, K)).astype(np.float32)
+        Nbig = persistent_n(sm_count())[0]
+        for beta in (0.0, 1.0):
+            for (N, ld, shift) in ((16, 16, 0), (48, 112, 0), (Nbig, Nbig + 64, 0), (48, 112, 4)):
+                B = rng.uniform(-1, 1, (K, ld)).astype(np.float32); C0 = rng.uniform(-1, 1, (M, ld)).astype(np.float32)
+                (dB, rB), (dC, rC) = guarded(B), guarded(C0, shift)
+                op = xs.Fsspmdm(a, N, ldb=ld, ldc=ld, beta=beta)
+                assert op.is_tensor_core
+                op.execute_stream(dB.ptr + G, dC.ptr + G + shift)
+                xs.synchronize()
+                assert xs.last_compute_kernel() == K4F
+                got = dC.to_numpy(np.uint8, rC.shape)[G + shift:G + shift + C0.nbytes].view(np.float32).reshape(C0.shape)
+                assert np.array_equal(got[:, N:], C0[:, N:]), "columns past N were written"
+                op.destroy()
+                check(dB, rB, B.nbytes, False); check(dC, rC, C0.nbytes, True, shift)
     elif kind.startswith("fsspmdm"):
         for dt in (np.float64, np.float32):
             M, K = (150, 125) if kind.endswith("strip") else (47, 33)
