@@ -420,8 +420,7 @@ void libxsmm_spmdm_init(int M, int N, int K, int max_threads, libxsmm_spmdm_hand
   const size_t col_bytes = ns * cap * 2, val_bytes = ns * cap * 4;
   c->arena_base = 0; c->staging = 0; c->table = 0;
   const size_t nnz_bytes = ((ns * 4) + 255) & ~(size_t)255;
-  const size_t lb_bytes = ((ns * 4 * 8) + 255) & ~(size_t)255;     // look-back words of the split slicing kernels + {epoch, done counter}
-  XB_CUDA(cudaMalloc(&c->arena_base, row_bytes + col_bytes + val_bytes + val_bytes + nnz_bytes + lb_bytes + 256 + nnz_bytes));
+  XB_CUDA(cudaMalloc(&c->arena_base, row_bytes + col_bytes + val_bytes + val_bytes + nnz_bytes + nnz_bytes));
   // per-tid staging slab for the legacy per-block entries on HOST matrices: an A block, or a B panel
   // (k x bn) followed by a C tile (bm x bn); the reference's slab holds the latter two (:148-155)
   {
@@ -445,10 +444,8 @@ void libxsmm_spmdm_init(int M, int N, int K, int max_threads, libxsmm_spmdm_hand
   c->arena.tcoff = (uint16_t*)((char*)c->arena_base + row_bytes + col_bytes + val_bytes);
   c->arena.tcpk = (uint32_t*)c->arena.tcoff;     // 4 bytes per entry: bf16 slices keep a 32-bit word per nonzero
   c->arena.slice_nnz = (uint32_t*)((char*)c->arena_base + row_bytes + col_bytes + val_bytes + val_bytes);
-  c->arena.lookback = (unsigned long long*)((char*)c->arena.slice_nnz + nnz_bytes);
-  c->arena.epoch = (uint32_t*)((char*)c->arena.lookback + lb_bytes);
-  c->arena.slice_ovf = (uint32_t*)((char*)c->arena.epoch + 256);
-  XB_CUDA(cudaMemset(c->arena.slice_nnz, 0, nnz_bytes + lb_bytes + 256 + nnz_bytes));
+  c->arena.slice_ovf = (uint32_t*)((char*)c->arena.slice_nnz + nnz_bytes);
+  XB_CUDA(cudaMemset(c->arena.slice_nnz, 0, nnz_bytes + nnz_bytes));
   c->h_nnz = 0; c->d_nnz = 0; c->d_acc = 0; c->aux_written = false; c->dense_written = false; c->sp_written = false; c->d_seen = -1.f; c->d_seen_prev = -1.f; c->captured = false; c->dense_bytes = 0; c->arena.dense = 0; c->arena.tcsp = 0; c->arena.ovf_list = 0;
   if (cudaSuccess == cudaHostAlloc((void**)&c->h_nnz, sizeof(unsigned long long), cudaHostAllocMapped)) {
     *c->h_nnz = ~0ull;

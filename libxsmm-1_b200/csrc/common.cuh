@@ -39,8 +39,6 @@ struct SliceArena {
   uint16_t* rowidx;
   uint16_t* colidx;
   float* values;
-  unsigned long long* lookback;   // auxiliary: per slice four words {launch epoch << 32 | nonzeros of that quarter of the slice} (k1_scan)
-  uint32_t* epoch;                // auxiliary: {launch epoch, CTAs finished} of the split slicing kernels
   uint32_t* slice_nnz;   // auxiliary: true nonzero count of every slice (the u16 row pointers wrap at 65536)
   uint16_t* tcoff;   // auxiliary (not part of the reference's slice), same indexing as colidx: where the nonzero
                      // goes in the tensor-core branch's shared-memory A tile (fp32 slices: xb_tc_pack)
@@ -233,10 +231,9 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream);
 void launch_compute(const ComputeArgs& args, cudaStream_t stream);
 bool launch_compute_tma(const ComputeArgs& args, bool partial, cudaStream_t stream);
-bool launch_compute_sp(const ComputeArgs& args, cudaStream_t stream);    // K2s: cluster-multicast order-preserving kernel (spmdm_compute_sp.cu)
+bool launch_compute_sp(const ComputeArgs& args, cudaStream_t stream);    // K2s: order-preserving TMA-ring kernel (spmdm_compute_sp.cu)
 bool launch_compute_tc(const ComputeArgs& args, cudaStream_t stream);
-bool launch_compute_tc16(const ComputeArgs& args, cudaStream_t stream);   // tcgen05 branch for bf16 inputs
-bool launch_compute_tc16p(const ComputeArgs& args, cudaStream_t stream);
+bool launch_compute_tc16p(const ComputeArgs& args, cudaStream_t stream);  // tcgen05 branch for bf16 inputs: CTA-pair kernel
 bool launch_compute_tc16s(const ComputeArgs& args, cudaStream_t stream);  // 2:4 structured-sparse CTA-pair kernel (needs SliceArena::tcsp)
 bool slices_get_sp_words(const SliceArgs& args);                          // would launch_slices() write tcsp for these arguments?
 bool launch_compute_tcq(const ComputeArgs& args, cudaStream_t stream);    // fp32 CTA-pair kernel (needs the slices' dense image)  // CTA-pair (cta_group::2) persistent form of it

@@ -7,13 +7,10 @@
 // src/template/libxsmm_spmdm_compute_fp32_thread.tpl.c:309-370, ..._bfloat16_thread.tpl.c:309-370) -- so the
 // result is bit-identical to the reference's full-width blocks.  What changed is everything around the fma:
 //
-//  * CTAs that work on the same column panel form a thread-block CLUSTER (CL row tiles of 128 rows).  A B tile
-//    (128 k x BN columns, 64 KiB) is fetched from L2 once per cluster: CTA r issues the TMA copy of k-rows
-//    [r*128/CL, (r+1)*128/CL) with .multicast::cluster, the data lands in every CTA's ring slot and every CTA's
-//    "full" barrier counts the bytes.  K2 re-read B from L2 once per 128 rows (M/128 x 33.5 MB = 1.07 GB on
-//    4096^3 bf16, which alone bounded it at ~125 us); with CL = 4 it is a quarter of that.  A slot is refilled
-//    when all CL x 16 consumer warps of the cluster have released it (remote mbarrier arrives).
-//  * a dedicated producer warp, so no consumer ever waits inside the producer's empty-slot wait.
+//  * B tiles (128 k x BN columns, 64 KiB) arrive by TMA in a 3-deep ring, fed by a dedicated producer warp, so no
+//    consumer ever waits inside the producer's empty-slot wait; a slot is refilled when all 16 consumer warps have
+//    released it.  Each CTA fetches its own tiles: sharing them over a thread-block cluster by TMA multicast measured
+//    slower (4096^3 bf16 at 1 %, B tile loads alone: 106 us per CTA, 161 us for pairs, 178 us for quads).
 //  * bf16: the nonzero travels as ONE word (bf16 value << 16 | column * 512), one shuffle per nonzero, and the
 //    multiply-add is the mixed-precision instruction fma.rn.f32.bf16 (SASS FHFMA.BF16 with .H0/.H1 operand
 //    selectors): bf16 x bf16 is exact in fp32, the sum is rounded once, so it equals fmaf(widen(a), widen(b), c)
@@ -47,34 +44,6 @@ constexpr int SP_THREADS = (SP_CW + 4) * 32;   // 16 consumer warps + one produc
 constexpr int SP_WSCRATCH = 384;               // bytes of per-warp list space: 33 x {1, 2} words of nonzeros (+ pad), 16 row offsets
 constexpr int SP_SMEM = SP_STAGES * SP_STAGEB + 64 + SP_CW * SP_WSCRATCH;
 
-__device__ __forceinline__ uint32_t cluster_ctarank()
-{
-  uint32_t r;
-  asm volatile("mov.u32 %0, %%cluster_ctarank;\n" : "=r"(r));
-  return r;
-}
-__device__ __forceinline__ void cluster_sync_all()
-{
-  __syncwarp();
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;\n" ::: "memory");
-}
-// arrive on the mbarrier at the same shared-memory offset in CTA `rank` of this cluster
-__device__ __forceinline__ void mbar_arrive_cluster(uint64_t* bar, uint32_t rank)
-{
-  asm volatile(
-    "{\n\t.reg .b32 ra;\n\t"
-    "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-    "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}\n"
-    ::"r"(smem_u32(bar)), "r"(rank) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_cluster_u32(uint32_t bar, uint32_t rank)
-{
-  asm volatile(
-    "{\n\t.reg .b32 ra;\n\t"
-    "mapa.shared::cluster.u32 ra, %0, %1;\n\t"
-    "mbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}\n"
-    ::"r"(bar), "r"(rank) : "memory");
-}
 __device__ __forceinline__ void mbar_arrive_u32(uint32_t bar) { asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];\n" ::"r"(bar) : "memory"); }
 __device__ __forceinline__ void mbar_wait_u32(uint32_t bar, uint32_t parity)
 {
@@ -87,13 +56,6 @@ __device__ __forceinline__ void mbar_wait_u32(uint32_t bar, uint32_t parity)
     "SP_DONE:\n\t}\n"
     ::"r"(bar), "r"(parity), "r"(0x989680) : "memory");
 }
-__device__ __forceinline__ void tma_load_2d_multicast(void* smem_dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar, uint16_t mask)
-{
-  asm volatile(
-    "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster [%0], [%1, {%2, %3}], [%4], %5;\n"
-    ::"r"(smem_u32(smem_dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)), "h"(mask) : "memory");
-}
-
 // One nonzero of the warp's rows as it is kept in registers between its (prefetched) load and the moment it is put on the
 // warp's shared-memory list.  A list entry is 8 bytes {address of the B tile row in shared memory, w}: for bf16 slices w
 // holds the value in its high half (the widened fp32 value has 16 zero bits below it), for fp32 slices w is the value.
@@ -164,15 +126,13 @@ template <> struct RowWalk<false> {
   }
 };
 
-template <bool BF16, int CL>
+template <bool BF16>
 __global__ void __launch_bounds__(SP_THREADS, 1)
 spmdm_compute_sp_kernel(const __grid_constant__ CUtensorMap tmB, const ComputeArgs p)
 {
   constexpr int VEC = BF16 ? 8 : 4;
   constexpr int BN = 32 * VEC;
   constexpr int R = SP_R;
-  constexpr int SLICE_ROWS = 128 / CL;                 // k-rows of a tile fetched by one CTA of the cluster
-  constexpr int SLICEB = SLICE_ROWS * SP_ROWB;
   extern __shared__ __align__(128) unsigned char smem[];
   uint64_t* full = (uint64_t*)(smem + (size_t)SP_STAGES * SP_STAGEB);
   uint64_t* empty = full + SP_STAGES;
@@ -181,27 +141,25 @@ spmdm_compute_sp_kernel(const __grid_constant__ CUtensorMap tmB, const ComputeAr
   pdl_wait();     // launched with programmatic stream serialization: the CTAs of the first wave are in place when the slicing kernel ends
   if (p.tc_twin > 0 && xb_total_nnz(p.sl.slice_nnz, g.mb * g.kb) >= p.tc_min_nnz) return;   // the tensor-core twin does this multiply (uniform over the grid)
   const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const uint32_t crank = (CL > 1) ? cluster_ctarank() : 0u;
   const int n0 = (int)blockIdx.y * BN;
 
   if (0 == tid) {
 #pragma unroll
-    for (int s = 0; s < SP_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], CL * SP_CW); }
+    for (int s = 0; s < SP_STAGES; ++s) { mbar_init(&full[s], 1); mbar_init(&empty[s], SP_CW); }
     mbar_fence_init();
   }
-  if (CL > 1) cluster_sync_all(); else __syncthreads();
+  __syncthreads();
 
   if (warp >= SP_CW) {
-    // ---------------- producer warp group: one lane streams this CTA's share of every B tile ----------------
+    // ---------------- producer warp group: one lane streams the B tiles ----------------
     asm volatile("setmaxnreg.dec.sync.aligned.u32 24;\n");
     if (SP_CW == warp && 0 == lane) {
       tma_prefetch_desc(&tmB);
       for (int t = 0; t < g.kb && !(p.debug_flags & 2); ++t) {
         const int s = t % SP_STAGES, f = t / SP_STAGES;
-        if (f > 0) mbar_wait(&empty[s], (f - 1) & 1);          // every consumer warp of the cluster is done with the slot
-        mbar_arrive_expect_tx(&full[s], SP_STAGEB);            // the whole tile: CL shares, one from each CTA
-        if (CL > 1) tma_load_2d_multicast(smem + (size_t)s * SP_STAGEB + (size_t)crank * SLICEB, &tmB, n0, t * g.bk + (int)crank * SLICE_ROWS, &full[s], (uint16_t)((1u << CL) - 1u));
-        else tma_load_2d(smem + (size_t)s * SP_STAGEB, &tmB, n0, t * g.bk, &full[s]);
+        if (f > 0) mbar_wait(&empty[s], (f - 1) & 1);          // every consumer warp is done with the slot
+        mbar_arrive_expect_tx(&full[s], SP_STAGEB);
+        tma_load_2d(smem + (size_t)s * SP_STAGEB, &tmB, n0, t * g.bk, &full[s]);
       }
     }
     __syncwarp();
@@ -216,10 +174,9 @@ spmdm_compute_sp_kernel(const __grid_constant__ CUtensorMap tmB, const ComputeAr
     asm volatile("" : "+r"(lane_off));
     const int tiles_per_mb = (g.bm + SP_TM - 1) / SP_TM;
     const int rt = (int)blockIdx.x;
-    const bool live = rt < p.mb_count * tiles_per_mb;          // grid.x is padded to a multiple of CL: a padding CTA only keeps the protocol going
-    const int mbi = p.mb_first + (live ? rt / tiles_per_mb : 0);
-    const int ml0 = live ? (rt % tiles_per_mb) * SP_TM : 0;
-    const int rows_in_block = live ? min(g.bm, g.m - mbi * g.bm) : 0;
+    const int mbi = p.mb_first + rt / tiles_per_mb;
+    const int ml0 = (rt % tiles_per_mb) * SP_TM;
+    const int rows_in_block = min(g.bm, g.m - mbi * g.bm);
     const int mycol = n0 + lane * VEC;
     const int wrow0 = ml0 + warp * R;
     const int nvalid = max(0, min(R, rows_in_block - wrow0));
@@ -342,11 +299,10 @@ spmdm_compute_sp_kernel(const __grid_constant__ CUtensorMap tmB, const ComputeAr
           }
         }
       }
-      // ---- release the slot to every producer of the cluster (not needed for the last tiles: nobody refills) ----
+      // ---- release the slot to the producer (not needed for the last tiles: nobody refills) ----
       if (kb + SP_STAGES < kbn && !(p.debug_flags & 2)) {
         __syncwarp();
-        if (CL > 1) { if (ulane < CL) mbar_arrive_cluster_u32(fullb + 8u * SP_STAGES, ulane); }
-        else if (0 == ulane) mbar_arrive_u32(fullb + 8u * SP_STAGES);
+        if (0 == ulane) mbar_arrive_u32(fullb + 8u * SP_STAGES);
       }
       stage += SP_STAGEB; fullb += 8u;
       if (++slot == SP_STAGES) { slot = 0; stage -= SP_STAGES * SP_STAGEB; fullb -= 8u * SP_STAGES; phase ^= 1u; }
@@ -371,67 +327,39 @@ spmdm_compute_sp_kernel(const __grid_constant__ CUtensorMap tmB, const ComputeAr
       }
     }
   }
-  if (CL > 1) cluster_sync_all();   // no CTA leaves while a peer may still signal its barriers
 }
 
-template <bool BF16, int CL>
+template <bool BF16>
 bool launch_sp(const ComputeArgs& a, cudaStream_t stream)
 {
   constexpr int ESZ = BF16 ? 2 : 4;
   constexpr int BN = SP_ROWB / ESZ;
-  constexpr size_t smem = (size_t)SP_SMEM;
   CUtensorMap map;
   if (!make_tensor_map_2d(&map, a.b, ESZ, (unsigned long long)a.ncols, (unsigned long long)a.g.k,
-                          (unsigned long long)a.ldb * ESZ, BN, 128 / CL)) return false;
-  auto kern = spmdm_compute_sp_kernel<BF16, CL>;
-  ensure_smem_optin((const void*)kern, (int)smem);
+                          (unsigned long long)a.ldb * ESZ, BN, 128)) return false;
+  auto kern = spmdm_compute_sp_kernel<BF16>;
+  ensure_smem_optin((const void*)kern, SP_SMEM);
   const int tiles_per_mb = (a.g.bm + SP_TM - 1) / SP_TM;
-  const int row_tiles = a.mb_count * tiles_per_mb;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)((row_tiles + CL - 1) / CL * CL), (unsigned)((a.ncols + BN - 1) / BN), 1);
-  cfg.blockDim = dim3(SP_THREADS, 1, 1);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[2];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = CL; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization; attr[1].val.programmaticStreamSerializationAllowed = 1;
-  static const bool pdl = [] { const char* e = getenv("LIBXSMM_B200_PDL"); return !(e && '0' == *e); }();
-  cfg.attrs = attr; cfg.numAttrs = pdl ? 2 : 1;
+  const dim3 grid((unsigned)(a.mb_count * tiles_per_mb), (unsigned)((a.ncols + BN - 1) / BN), 1);
   count_launch(1);
   note_compute_kernel("spmdm_compute_sp_kernel");
-  XB_CUDA(cudaLaunchKernelEx(&cfg, kern, map, a));
+  XB_CUDA(launch_pdl(kern, grid, dim3(SP_THREADS), (size_t)SP_SMEM, stream, map, a));
   return true;
 }
 
 }  // namespace
 
-// LIBXSMM_B200_K2S: "0" = keep the first-generation kernel (K2), "1" / "2" / "4" = cluster size.  Default 1: measured on
-// 4096^3 bf16 at 1 % the multicast forms are SLOWER (B tile loads alone: 106 us unicast, 161 us for pairs, 178 us for
-// quads), so they stay an experiment
+// returns false when the panel does not qualify (caller then uses K2 or the generic kernel)
 bool launch_compute_sp(const ComputeArgs& a_in, cudaStream_t stream)
 {
   if (a_in.transb || a_in.transc) return false;
   if (0 != ((uintptr_t)a_in.c & 15) || 0 != (a_in.ldc & 3)) return false;
   if (a_in.ncols <= 32) return false;
   if ((unsigned long long)a_in.g.mb * a_in.g.kb * a_in.g.bm * a_in.g.bk >= (1ull << 31)) return false;   // the kernel indexes the slice arena with 32-bit element offsets
-  static const int cl = [] { const char* e = getenv("LIBXSMM_B200_K2S"); return (e && *e) ? atoi(e) : 1; }();
   static const int dbg = [] { const char* e = getenv("LIBXSMM_B200_K2S_DEBUG"); return (e && *e) ? atoi(e) : 0; }();
-  if (cl <= 0) return false;
   ComputeArgs a = a_in;
   a.debug_flags = dbg;
-  if (a.is_bf16) {
-    switch (cl) {
-      case 1: return launch_sp<true, 1>(a, stream);
-      case 2: return launch_sp<true, 2>(a, stream);
-      default: return launch_sp<true, 4>(a, stream);
-    }
-  }
-  switch (cl) {
-    case 1: return launch_sp<false, 1>(a, stream);
-    case 2: return launch_sp<false, 2>(a, stream);
-    default: return launch_sp<false, 4>(a, stream);
-  }
+  return a.is_bf16 ? launch_sp<true>(a, stream) : launch_sp<false>(a, stream);
 }
 
 }  // namespace xb

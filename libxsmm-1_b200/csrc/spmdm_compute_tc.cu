@@ -18,7 +18,6 @@
 // in a way that changes finite results: dropped (zero) entries of A are exact zeros in the dense tile.
 #include "common.cuh"
 #include "tc_common.cuh"
-#include <cstdlib>
 
 namespace xb {
 
@@ -361,9 +360,8 @@ bool launch_compute_tc(const ComputeArgs& a, cudaStream_t stream)
   }
   else if (!make_tensor_map_2d_sw128(&map, a.b, 4, (unsigned long long)a.ncols, (unsigned long long)a.g.k, (unsigned long long)a.ldb * 4, 32, TC_KC, true)) return false;
   // performance-only choice (every instantiation is complete): the host's estimate is one call old at most
-  bool sparse_variant = a.density_hint >= 0.f && a.density_hint < 0.25f;
-  { const char* e = getenv("LIBXSMM_B200_K4_VARIANT"); if (e && 's' == *e) sparse_variant = true; else if (e && 'd' == *e) sparse_variant = false; }   // developer switch
-  const bool image = 0 != a.dense_valid && 0 != a.sl.dense && !(getenv("LIBXSMM_B200_K4_VARIANT") && 0 != a.aux_valid);   // the slicing pass left the A image: nothing to rebuild
+  const bool sparse_variant = a.density_hint >= 0.f && a.density_hint < 0.25f;
+  const bool image = 0 != a.dense_valid && 0 != a.sl.dense;   // the slicing pass left the A image: nothing to rebuild
   if (!image && 0 == a.aux_valid) return false;   // neither the image nor the per-nonzero words: the CUDA-core kernels multiply these slices
   const void* kern = image ? (const void*)spmdm_compute_tc_kernel<16, false, true>
                    : (sparse_variant ? (const void*)spmdm_compute_tc_kernel<8, true, false> : (const void*)spmdm_compute_tc_kernel<16, false, false>);

@@ -2,8 +2,8 @@
 //
 //   C[256 rows, 256 cols] = beta*C + sum_kb densify(slices(kb, rows))[256 x 128] * B[kb*128 .. +128, 256 cols]
 //
-// What bounded the single-CTA kernel (K4h, spmdm_compute_tc16.cu; measured with its stages switched off one at
-// a time): B travels L2 -> SM once per 128 output rows (1.07 GB for 4096^3, 8.4 TB/s at the 128 us the bare
+// What bounded the single-CTA kernel this one replaced (K4h, 164 us for 4096^3 against 93 us here; measured with its
+// stages switched off one at a time): B travels L2 -> SM once per 128 output rows (1.07 GB for 4096^3, 8.4 TB/s at the 128 us the bare
 // MMA + TMA pipeline needs), the zero-fill of the A tile competes with the operand reads for shared memory, and
 // the epilogue of a tile is not overlapped with anything.  This kernel changes all three:
 //   * two CTAs of one TPC share every MMA (M = 256: 128 rows each, N = 256: each CTA stages 128 columns of B).
@@ -16,7 +16,8 @@
 //     instead of 32 KiB of zero-fill.
 // Roles per CTA (14 warps): warp 0 TMA producer, warp 1 MMA issuer (leader CTA only) and TMEM owner, warps 2-9
 // densify (two groups taking k-blocks in turn, thread = row), warps 10-13 epilogue (warp % 4 = TMEM lane quarter).
-// Like K4h this kernel keeps the 1e-2 contract of the bf16 path, not the reference's rounding sequence.
+// Like the fp32 branch this kernel keeps the 1e-2 contract of the bf16 path, not the reference's rounding sequence;
+// LIBXSMM_B200_SPMDM_TC=0 selects the order-preserving CUDA-core kernels.
 #include "common.cuh"
 #include "tc_common.cuh"
 #include <cstdlib>
@@ -367,7 +368,7 @@ spmdm_compute_tc16p_kernel(const __grid_constant__ CUtensorMap tmB, const Comput
 bool make_tensor_map_2d_sw128(CUtensorMap* map, const void* base, int elem_bytes, unsigned long long cols, unsigned long long rows,
                               unsigned long long row_pitch_bytes, unsigned box_cols, unsigned box_rows, bool atom32);
 
-// returns false when the panel does not qualify (caller falls back to K4h / the CUDA-core kernels)
+// returns false when the panel does not qualify (caller falls back to the CUDA-core kernels)
 bool launch_compute_tc16p(const ComputeArgs& a, cudaStream_t stream)
 {
   if (0 == a.aux_valid) return false;   // these kernels rebuild A from the packed per-nonzero words the slicing pass writes

@@ -556,7 +556,7 @@ bool launch_compute_tc16s(const ComputeArgs& a, cudaStream_t stream)
   // C leaves through TMA boxes of 32 x 32 when it is only written (beta = 0) and stored row-major
   CUtensorMap cmap = map;
   int c_tma = 0;
-  if (!a.transc && 0.f == a.beta && !(getenv("LIBXSMM_B200_K4S_TMA_C") && '0' == *getenv("LIBXSMM_B200_K4S_TMA_C"))) {
+  if (!a.transc && 0.f == a.beta) {
     const long long crows = (long long)a.g.m - a.row_origin;
     if (crows > 0 && make_tensor_map_2d_sw128(&cmap, a.c, 4, (unsigned long long)a.ncols, (unsigned long long)crows, (unsigned long long)a.ldc * 4, 32, 32, false)) c_tma = 1;
     else cmap = map;

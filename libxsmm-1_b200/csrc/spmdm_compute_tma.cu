@@ -17,7 +17,6 @@
 // else stays on the generic kernel in spmdm_kernels.cu.
 #include "common.cuh"
 #include "ptx.cuh"
-#include <cstdlib>
 #include <mutex>
 
 namespace xb {
@@ -364,30 +363,13 @@ bool launch_compute_tma(const ComputeArgs& a, bool partial, cudaStream_t stream)
 {
   if (a.transb || a.transc) return false;
   if (0 != ((uintptr_t)a.c & 15) || 0 != (a.ldc & 3)) return false;
-  static const int variant = [] { const char* e = getenv("LIBXSMM_B200_K2_VARIANT"); return (e && *e) ? atoi(e) : 0; }();
   if (partial) {   // at most bn - 1 columns: one narrow column tile, many short row tiles
     return a.is_bf16 ? launch_tma_variant<true, 4, 4, 8, 4, true>(a, stream) : launch_tma_variant<false, 2, 4, 8, 4, true>(a, stream);
   }
   if (a.ncols <= 32) {   // scalar tail of the narrow block: in-order chain, few columns
     return a.is_bf16 ? launch_tma_variant<true, 4, 4, 8, 4, false>(a, stream) : launch_tma_variant<false, 2, 4, 8, 4, false>(a, stream);
   }
-  if (a.is_bf16) {
-    switch (variant) {
-      case 1: return launch_tma_variant<true, 4, 16, 16, 4, false>(a, stream);
-      case 2: return launch_tma_variant<true, 4, 8, 16, 4, false>(a, stream);
-      case 3: return launch_tma_variant<true, 8, 16, 8, 3, false>(a, stream);
-      case 4: return launch_tma_variant<true, 8, 8, 8, 3, false>(a, stream);
-      case 5: return launch_tma_variant<true, 8, 4, 32, 3, false>(a, stream);
-      case 6: return launch_tma_variant<true, 8, 4, 24, 3, false>(a, stream);
-      default: return launch_tma_variant<true, 8, 8, 16, 3, false>(a, stream);
-    }
-  }
-  switch (variant) {
-    case 1: return launch_tma_variant<false, 4, 16, 16, 3, false>(a, stream);
-    case 3: return launch_tma_variant<false, 4, 16, 8, 3, false>(a, stream);
-    case 4: return launch_tma_variant<false, 4, 8, 8, 3, false>(a, stream);
-    default: return launch_tma_variant<false, 4, 8, 16, 3, false>(a, stream);
-  }
+  return a.is_bf16 ? launch_tma_variant<true, 8, 8, 16, 3, false>(a, stream) : launch_tma_variant<false, 4, 8, 16, 3, false>(a, stream);
 }
 
 }  // namespace xb

@@ -267,18 +267,13 @@ template <> struct K1Raw<true> {
   static __device__ __forceinline__ uint4 widen(raw_t r) { return make_uint4(r.x << 16, r.x & 0xFFFF0000u, r.y << 16, r.y & 0xFFFF0000u); }
 };
 
-// A slice may be split over P = 32 / CW CTAs of CW warps (part q owns the "virtual warps" q*CW .. q*CW+CW-1 of the
-// one-CTA form, i.e. a contiguous quarter of the slice's rows): several small CTAs per SM overlap their load, scan and store
-// phases, where one 1024-thread CTA per SM runs them back to back.  The running position across the parts of a slice is a
-// decoupled look-back: a part publishes {epoch, its count} and adds up the counts of the parts before it (lower block
-// indices: already dispatched), spinning on the few that are not there yet.  The epoch (one per launch, advanced by the
-// last CTA to finish) makes stale words of earlier launches -- including replays of a captured graph -- unreadable.
-struct K1Scan { uint32_t pos; uint32_t slice_total; };   // first output position of this warp's rows; the slice's total (valid in the last part)
+// Exclusive scan of the CW warp totals of a CTA on top of `base` (the kept elements of the rows before the CTA's): the first
+// output position of this warp's rows, and the running total after the CTA's rows.  wtot: CW words of shared memory.
+struct K1Scan { uint32_t pos; uint32_t slice_total; };
 
 template <int CW>
-__device__ __forceinline__ K1Scan k1_scan(const SliceArgs& p, int s, int part, uint32_t warp_total, uint32_t* wtot /* shared, CW + 1 words */, uint32_t epoch)
+__device__ __forceinline__ K1Scan k1_scan(uint32_t warp_total, uint32_t* wtot, uint32_t base)
 {
-  constexpr int P = 32 / CW;
   const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
   if (0 == lane) wtot[warp] = warp_total;
   __syncthreads();
@@ -290,41 +285,10 @@ __device__ __forceinline__ K1Scan k1_scan(const SliceArgs& p, int s, int part, u
     if (lane >= d) inc += u;
   }
   const uint32_t cta_total = __shfl_sync(0xffffffffu, inc, CW - 1);
-  uint32_t base = 0;
-  if (P > 1) {
-    if (0 == tid) {
-      unsigned long long* lb = p.out.lookback + (size_t)s * P;
-      const unsigned long long mine = ((unsigned long long)epoch << 32) | cta_total;
-      asm volatile("st.release.gpu.global.u64 [%0], %1;\n" ::"l"(lb + part), "l"(mine) : "memory");
-      uint32_t b = 0;
-      for (int j = part - 1; j >= 0; --j) {
-        unsigned long long v;
-        do { asm volatile("ld.acquire.gpu.global.u64 %0, [%1];\n" : "=l"(v) : "l"(lb + j) : "memory"); } while ((uint32_t)(v >> 32) != epoch);
-        b += (uint32_t)v;
-      }
-      wtot[CW] = b;
-    }
-    __syncthreads();
-    base = wtot[CW];
-  }
   K1Scan r;
   r.pos = base + __shfl_sync(0xffffffffu, inc - t, warp);
   r.slice_total = base + cta_total;
   return r;
-}
-
-__device__ __forceinline__ uint32_t k1_epoch(const SliceArgs& p) { return p.out.epoch ? (*(volatile uint32_t*)p.out.epoch + 1u) : 1u; }
-
-// last CTA of the launch to get here advances the epoch (all CTAs have read it long before)
-__device__ __forceinline__ void k1_finish(const SliceArgs& p, uint32_t epoch)
-{
-  if (0 == p.out.epoch) return;
-  __syncthreads();
-  if (0 == threadIdx.x) {
-    __threadfence();
-    const uint32_t done = atomicAdd(p.out.epoch + 1, 1u);
-    if (done + 1u == gridDim.x) { p.out.epoch[1] = 0u; __threadfence(); *(volatile uint32_t*)p.out.epoch = epoch; }
-  }
 }
 
 // keep-mask of the lane's four elements.  FULL = complete 128-column block whose columns are all inside the
@@ -345,21 +309,19 @@ __device__ __forceinline__ uint32_t k1n_mask(uint4 w, int lane, int ncols, int v
   return m;
 }
 
-// ROWS = rows a warp handles (>= rows per warp); KEEP = rows stay in registers between the two phases,
-// otherwise phase 2 re-reads them (fp32 slices of 512 rows do not fit the register file).
-template <bool BF16, bool FULL, int ROWS, bool KEEP, int CW>
-__global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 3) spmdm_slice_n_kernel(const SliceArgs p)
+// ROWS = rows a warp handles (>= rows per warp).  KEEP: the rows stay in registers between the two phases; at 16 rows
+// phase 2 re-reads them (fp32 slices of 512 rows do not fit the register file).
+template <bool BF16, bool FULL, int ROWS>
+__global__ void __launch_bounds__(K1N_THREADS, 1) spmdm_slice_n_kernel(const SliceArgs p)
 {
   typedef K1Raw<BF16> Raw;
   typedef typename Raw::raw_t raw_t;
-  constexpr int P = 32 / CW;
-  __shared__ uint32_t wtot[CW + 1];
+  constexpr bool KEEP = ROWS <= 8;
+  __shared__ uint32_t wtot[K1N_WARPS];
   pdl_wait();          // launch_pdl: the slices may still be read by the multiply in front of this kernel in the stream
   pdl_trigger();       // ... and the multiply behind it may be scheduled (it waits in turn)
   const Geom& g = p.g;
-  const uint32_t epoch = (P > 1) ? k1_epoch(p) : 0u;
-  const int part = (int)blockIdx.x % P;
-  const int s = p.slice0 + ((int)blockIdx.x / P) * p.slice_step;
+  const int s = p.slice0 + (int)blockIdx.x * p.slice_step;
   const int kb = s / g.mb, mbi = s - kb * g.mb;
   const int nrows = min(g.bm, g.m - mbi * g.bm);
   const int ncols = min(g.bk, g.k - kb * g.bk);
@@ -367,7 +329,7 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 3) spmdm_slice_n_ker
   if (p.simd_w <= 1) vec_end = 0;
   const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int rpw = (g.bm + K1N_WARPS - 1) / K1N_WARPS;      // rows per warp (<= 16 because bm <= 512)
-  const int row_lo = (part * CW + warp) * rpw, row_hi = min(nrows, row_lo + rpw);
+  const int row_lo = warp * rpw, row_hi = min(nrows, row_lo + rpw);
   const size_t esz = BF16 ? 2 : 4;
   const long long origin = p.origin_is_block ? 0ll : ((long long)mbi * g.bm * p.lda + (long long)kb * g.bk);
   const char* A = (const char*)p.a + origin * (long long)esz;
@@ -392,12 +354,11 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 3) spmdm_slice_n_ker
   for (int j = 0; j < (ROWS + 7) / 8; ++j) mine += __popc(masks[j]);
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
-  const K1Scan sc = k1_scan<CW>(p, s, part, mine, wtot, epoch);
+  const K1Scan sc = k1_scan<K1N_WARPS>(mine, wtot, 0u);
   uint32_t pos = sc.pos;   // first output position of this warp's rows
-  // completely full 512 x 128 slice: the reference's u16 counter wraps and its multiply sees the last row as empty.  Known
-  // here only to the last part -- which is the one that owns row 511
-  const bool wrapped = (P - 1 == part) && sc.slice_total >= 65536u;
-  if (P - 1 == part && 0 == tid) {
+  // completely full 512 x 128 slice: the reference's u16 counter wraps and its multiply sees the last row as empty
+  const bool wrapped = sc.slice_total >= 65536u;
+  if (0 == tid) {
     p.out.rowidx[(size_t)s * (g.bm + 1) + nrows] = (uint16_t)sc.slice_total;   // u16 like the reference's counter
     p.out.slice_nnz[s] = sc.slice_total;
     xb_publish_nnz(p, sc.slice_total);
@@ -451,14 +412,14 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 3) spmdm_slice_n_ker
       pos += __popc(b0) + 2 * __popc(b1) + 4 * __popc(b2);
     }
   }
-  if (P > 1) k1_finish(p, epoch);
 }
 
 // -------------------------------------------------------------------------------------------------
-// K1 wide variant for bf16, transa = 'N', complete 128-column blocks: a lane holds EIGHT consecutive elements
-// (one 16-byte load), so a row is half a warp and a warp works on two rows at a time; the keep test runs on
-// the packed bf16 pairs with carry arithmetic (no widening, no per-element compare).  Same two phases, same
-// outputs, about a third of the instructions of the generic kernel (which is instruction-issue bound).
+// K1x: bf16, transa = 'N', complete 128-column blocks with 16-byte aligned rows.  A lane holds SIXTEEN consecutive elements
+// (two 16-byte loads), so a row is a quarter of a warp and one iteration of the positioning phase covers four rows; the keep
+// test runs on the packed bf16 pairs with carry arithmetic (no widening, no per-element compare).  Same two phases and the same
+// outputs as the generic kernel, bit for bit, at about a third of its instructions (it is instruction-issue bound).  Measured on
+// C2: one 16-byte word per lane 25.1 us, two 23.2 us, four 23.1 us.
 // -------------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t k1w_mask8(uint4 w)
 {
@@ -482,141 +443,34 @@ __device__ __forceinline__ uint32_t k1w_mask8(uint4 w)
   return lo | (hi << 4);
 }
 
-template <int ROWS>
-__global__ void __launch_bounds__(K1N_THREADS, 1) spmdm_slice_bf16w_kernel(const SliceArgs p)
+// CW < 32: one CTA of CW warps walks the 32 / CW parts of its slice one after the other (the running total is the next part's
+// base), so that two 16-warp CTAs fit an SM and one's loads overlap the other's arithmetic.
+template <int ROWS, int CW>
+__global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x_kernel(const SliceArgs p)
 {
-  __shared__ uint32_t wtot[K1N_WARPS];
-  const Geom& g = p.g;
-  const int s = p.slice0 + (int)blockIdx.x * p.slice_step;
-  const int kb = s / g.mb, mbi = s - kb * g.mb;
-  const int nrows = min(g.bm, g.m - mbi * g.bm);
-  const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  const int half = lane >> 4, hl = lane & 15;
-  const int rpw = (g.bm + K1N_WARPS - 1) / K1N_WARPS;
-  const int row_lo = warp * rpw, row_hi = min(nrows, row_lo + rpw);
-  const long long origin = p.origin_is_block ? 0ll : ((long long)mbi * g.bm * p.lda + (long long)kb * g.bk);
-  const uint16_t* A = (const uint16_t*)p.a + origin + hl * 8;
-
-  // ---- phase 1: load, test, count ---------------------------------------------------------------------
-  uint4 w[ROWS / 2];
-  uint32_t masks[(ROWS / 2 + 3) / 4];      // 8 bits per iteration
-#pragma unroll
-  for (int j = 0; j < (ROWS / 2 + 3) / 4; ++j) masks[j] = 0;
-#pragma unroll
-  for (int it = 0; it < ROWS / 2; ++it) {
-    const int r = row_lo + 2 * it + half;
-    w[it] = (r < row_hi) ? __ldg((const uint4*)(A + (long long)r * p.lda)) : make_uint4(0, 0, 0, 0);
-  }
-#pragma unroll
-  for (int it = 0; it < ROWS / 2; ++it) masks[it / 4] |= k1w_mask8(w[it]) << (8 * (it % 4));
-  uint32_t mine = 0;
-#pragma unroll
-  for (int j = 0; j < (ROWS / 2 + 3) / 4; ++j) mine += __popc(masks[j]);
-#pragma unroll
-  for (int d = 16; d > 0; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
-  if (0 == lane) wtot[warp] = mine;
-  __syncthreads();
-  uint32_t pos;
-  {
-    const uint32_t t = wtot[lane];
-    uint32_t inc = t;
-#pragma unroll
-    for (int d = 1; d < 32; d <<= 1) {
-      const uint32_t u = __shfl_up_sync(0xffffffffu, inc, d);
-      if (lane >= d) inc += u;
-    }
-    pos = __shfl_sync(0xffffffffu, inc - t, warp);
-    const uint32_t total = __shfl_sync(0xffffffffu, inc, 31);
-    if (0 == tid) {
-      p.out.rowidx[(size_t)s * (g.bm + 1) + nrows] = (uint16_t)total;   // u16 like the reference's counter
-      p.out.slice_nnz[s] = total;
-      xb_publish_nnz(p, total);
-    }
-  }
-
-  // ---- phase 2: positions and stores -----------------------------------------------------------------------
-  uint16_t* ro = p.out.rowidx + (size_t)s * (g.bm + 1);
-  uint16_t* co = p.out.colidx + (size_t)s * g.bm * g.bk;
-  float* va = p.out.values + (size_t)s * g.bm * g.bk;
-  uint32_t* rk = p.out.tcpk + (size_t)s * g.bm * g.bk;
-  const uint32_t lt = (1u << lane) - 1u;
-  const uint32_t mymask = half ? 0xFFFF0000u : 0x0000FFFFu;
-  const bool aux = (0 != p.write_aux);
-#pragma unroll
-  for (int it = 0; it < ROWS / 2; ++it) {
-    if (row_lo + 2 * it < row_hi) {      // warp-uniform
-      const uint32_t m = (masks[it / 4] >> (8 * (it % 4))) & 255u;
-      const uint32_t nm = __popc(m);      // 0..8
-      const uint32_t b0 = __ballot_sync(0xffffffffu, nm & 1u), b1 = __ballot_sync(0xffffffffu, nm & 2u);
-      uint32_t lo_tot = __popc(b0 & 0xFFFFu) + 2 * __popc(b1 & 0xFFFFu);
-      uint32_t hi_tot = __popc(b0 >> 16) + 2 * __popc(b1 >> 16);
-      // a lane keeping four or more of its eight elements is rare below ~20 % density: the two upper count bits are
-      // voted on only then (warp-uniform branch)
-      const bool big = 0 != __any_sync(0xffffffffu, nm >= 4u);
-      uint32_t b2 = 0, b3 = 0;
-      if (big) {
-        b2 = __ballot_sync(0xffffffffu, nm & 4u); b3 = __ballot_sync(0xffffffffu, nm & 8u);
-        lo_tot += 4 * __popc(b2 & 0xFFFFu) + 8 * __popc(b3 & 0xFFFFu);
-        hi_tot += 4 * __popc(b2 >> 16) + 8 * __popc(b3 >> 16);
-      }
-      const uint32_t rowpos = pos + (half ? lo_tot : 0u);
-      const int r = row_lo + 2 * it + half;
-      if (0 == hl && r < row_hi) ro[r] = (uint16_t)rowpos;
-      if (m) {   // few lanes hold nonzeros in the sparse regime
-        const uint32_t pm = lt & mymask;
-        uint32_t q = rowpos + __popc(b0 & pm) + 2 * __popc(b1 & pm);
-        if (big) q += 4 * __popc(b2 & pm) + 8 * __popc(b3 & pm);
-        const uint32_t v[4] = { w[it].x, w[it].y, w[it].z, w[it].w };
-        // xb_tc16_pack(r, hl * 8 + e, value) = value | (base16 + e): everything but e is fixed for this lane and row
-        const uint32_t rowm = (uint32_t)r & 127u;
-        const uint32_t base16 = ((uint32_t)(hl >> 3) << 15) | ((rowm >> 3) * 512u + (rowm & 7u) * 64u + ((((uint32_t)hl ^ rowm) & 7u) << 3));
-        // one trip per kept element of the fullest lane (1-2 in the sparse regime) instead of eight predicated slots
-        for (uint32_t mm = m; mm; mm &= mm - 1u, ++q) {
-          const int e = __ffs((int)mm) - 1;
-          const uint32_t pr = (e & 4) ? ((e & 2) ? v[3] : v[2]) : ((e & 2) ? v[1] : v[0]);
-          const uint32_t vb = (e & 1) ? (pr & 0xFFFF0000u) : (pr << 16);
-          co[q] = (uint16_t)(hl * 8 + e);
-          va[q] = __uint_as_float(vb);
-          if (aux) rk[q] = vb | (base16 + (uint32_t)e);
-        }
-      }
-      pos += lo_tot + hi_tot;
-    }
-  }
-}
-
-// K1x: the same with NW 16-byte words (8 * NW elements) per lane: a row is 16 / NW lanes and one iteration of the
-// positioning phase covers 2 * NW rows, which divides the number of ballot rounds per slice by NW (the kernel is
-// instruction-issue bound).  Same outputs, bit for bit.  Measured on C2: NW = 1 (K1w) 25.1 us, NW = 2 23.2 us, NW = 4 23.1 us (not instantiated).
-// SEQ > 1: one CTA of CW warps walks the 32 / CW parts of its slice one after the other (the running total is the next part's
-// base: no look-back between CTAs), so that two 16-warp CTAs fit an SM and one's loads overlap the other's arithmetic.
-template <int ROWS, int NW, int CW, int SEQ = 1>
-__global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : ((SEQ > 1) ? 2 : 3)) spmdm_slice_bf16x_kernel(const SliceArgs p)
-{
+  constexpr int NW = 2;                      // 16-byte words per lane
+  constexpr int SEQ = 32 / CW;               // parts of the slice walked by the CTA in turn
   constexpr int LPR = 16 / NW;               // lanes per row
   constexpr int RPI = 32 / LPR;              // rows per iteration
   constexpr int ITS = (ROWS + RPI - 1) / RPI;
-  constexpr int P = (SEQ > 1) ? 1 : 32 / CW; // CTAs per slice (k1_scan)
-  __shared__ uint32_t wtot[CW + 1];
-  constexpr int SCAP = 64;                                // records per warp: all 16 rows of a warp at once up to 3 % density
-  __shared__ uint2 stage[(2 == NW) ? CW : 1][SCAP];      // per warp: the records of its outputs (stage and spread, phase 2)
+  __shared__ uint32_t wtot[CW];
+  constexpr int SCAP = 64;                   // records per warp: all 16 rows of a warp at once up to 3 % density
+  __shared__ uint2 stage[CW][SCAP];          // per warp: the records of its outputs (stage and spread, phase 2)
   // programmatic dependent launch (launch_slices): the slices this kernel overwrites may still be read by the multiply in front of
   // it in the stream -- wait for it before anything else; the multiply behind it may be scheduled from now on (it waits in turn)
   pdl_wait();
   pdl_trigger();
   const Geom& g = p.g;
-  const uint32_t epoch = (P > 1) ? k1_epoch(p) : 0u;
-  const int s = p.slice0 + ((int)blockIdx.x / P) * p.slice_step;
+  const int s = p.slice0 + (int)blockIdx.x * p.slice_step;
   const int kb = s / g.mb, mbi = s - kb * g.mb;
   const int nrows = min(g.bm, g.m - mbi * g.bm);
   const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int qr = lane / LPR, hl = lane % LPR;       // row inside the group, segment of the row
   const int rpw = (g.bm + K1N_WARPS - 1) / K1N_WARPS;
-  uint32_t seq_base = 0;                     // SEQ > 1: kept elements of the parts already done
+  uint32_t seq_base = 0;                     // kept elements of the parts already done
 #pragma unroll 1
   for (int pass = 0; pass < SEQ; ++pass) {
-  const int part = (SEQ > 1) ? pass : (int)blockIdx.x % P;
-  const int row_lo = (part * CW + warp) * rpw, row_hi = min(nrows, row_lo + rpw);
+  const int row_lo = (pass * CW + warp) * rpw, row_hi = min(nrows, row_lo + rpw);
   const long long origin = p.origin_is_block ? 0ll : ((long long)mbi * g.bm * p.lda + (long long)kb * g.bk);
   const uint16_t* A = (const uint16_t*)p.a + origin + hl * (8 * NW);
 
@@ -642,25 +496,11 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : ((SEQ > 1) ? 2 : 3))
 #pragma unroll
   for (int d = 16; d > 0; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
   const uint32_t warp_total = mine;
-  if (2 == NW && 1 == P && 0 == pass && 0 == tid && p.write_sp && p.out.tcsp) p.out.slice_ovf[s] = 0;   // counted below, after the scan's barrier
-  K1Scan sc;
-  if (SEQ > 1) {      // this CTA's parts in sequence: scan of the CW warp totals on top of the running total
-    if (0 == lane) wtot[warp] = mine;
-    __syncthreads();
-    const uint32_t t = (lane < CW) ? wtot[lane] : 0u;
-    uint32_t inc = t;
-#pragma unroll
-    for (int d = 1; d < CW; d <<= 1) {
-      const uint32_t u = __shfl_up_sync(0xffffffffu, inc, d);
-      if (lane >= d) inc += u;
-    }
-    sc.pos = seq_base + __shfl_sync(0xffffffffu, inc - t, warp);
-    sc.slice_total = seq_base + __shfl_sync(0xffffffffu, inc, CW - 1);
-    seq_base = sc.slice_total;
-  }
-  else sc = k1_scan<CW>(p, s, part, mine, wtot, epoch);
+  if (0 == pass && 0 == tid && p.write_sp && p.out.tcsp) p.out.slice_ovf[s] = 0;   // counted below, after the scan's barrier
+  const K1Scan sc = k1_scan<CW>(mine, wtot, seq_base);
+  seq_base = sc.slice_total;
   uint32_t pos = sc.pos;
-  if (((SEQ > 1) ? (SEQ - 1 == pass) : (P - 1 == part)) && 0 == tid) {
+  if (SEQ - 1 == pass && 0 == tid) {
     p.out.rowidx[(size_t)s * (g.bm + 1) + nrows] = (uint16_t)sc.slice_total;   // u16 like the reference's counter
     p.out.slice_nnz[s] = sc.slice_total;
     xb_publish_nnz(p, sc.slice_total);
@@ -672,13 +512,12 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : ((SEQ > 1) ? 2 : 3))
   float* va = p.out.values + (size_t)s * g.bm * g.bk;
   uint32_t* rk = p.out.tcpk + (size_t)s * g.bm * g.bk;
   const uint32_t lt = (1u << lane) - 1u;
-  uint2* stg = stage[(2 == NW) ? warp : 0];
-  const uint32_t rowmask = ((1u << LPR) - 1u) << (LPR * qr);   // the lanes of this lane's row
+  uint2* stg = stage[warp];
   const uint32_t before = (1u << (LPR * qr)) - 1u;             // the lanes of the rows above it in the group
   const bool aux = (0 != p.write_aux);
   // word per nonzero for the structured-sparse tensor-core kernel: a lane's 16 elements are exactly the four groups of four
   // whose nibbles make one 16-bit metadata word of the row, so everything is known to the lane (common.cuh: xb_sp_*)
-  const bool spw = (2 == NW) && (0 != p.write_sp) && (0 != p.out.tcsp);
+  const bool spw = (0 != p.write_sp) && (0 != p.out.tcsp);
   uint32_t* sp = p.out.tcsp + (size_t)s * g.bm * g.bk;
   uint32_t wdone = 0;                      // outputs of this warp's earlier iterations
   const uint32_t pos0 = pos;               // first output of this warp
@@ -722,102 +561,67 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : ((SEQ > 1) ? 2 : 3))
       const uint32_t rowpos = pos + kept(before);
       const int r = row_lo + RPI * it + qr;
       if (0 == hl && r < row_hi) ro[r] = (uint16_t)rowpos;
-      if (2 == NW) {
-        // Stage and spread.  In the sparse regime a handful of the 32 lanes hold a nonzero or two, and everything a nonzero costs
-        // (four stores, the positions in the tensor-core tiles, the metadata word) would run once per loop trip of the fullest
-        // lane with one to three lanes active.  Instead every lane drops its kept elements as 8-byte records {value | its 16-bit
-        // mask, element | lane << 4 | iteration << 9} at their output index into the warp's shared-memory stage (a short
-        // divergent loop), and lane t then does all the work for output t.  When the warp's 16 rows hold at most SCAP nonzeros
-        // (always below 3 % density) all four iterations are staged first and spread in one pass after the loop.
-        const uint32_t tot = kept(0xFFFFFFFFu);
-        if (tot) {                                        // warp-uniform
-          const uint32_t ex = kept(lt);                   // this lane's first output of the iteration (lane order = (row, column) order)
-          const bool all_at_once = warp_total <= (uint32_t)SCAP;
-          for (uint32_t c0 = 0; c0 < tot; c0 += 32u) {    // one chunk below ~6 % density
-            if (m) {
-              uint32_t i = all_at_once ? (wdone + ex) : (ex - c0);
+      // Stage and spread.  In the sparse regime a handful of the 32 lanes hold a nonzero or two, and everything a nonzero costs
+      // (four stores, the positions in the tensor-core tiles, the metadata word) would run once per loop trip of the fullest
+      // lane with one to three lanes active.  Instead every lane drops its kept elements as 8-byte records {value | its 16-bit
+      // mask, element | lane << 4 | iteration << 9} at their output index into the warp's shared-memory stage (a short
+      // divergent loop), and lane t then does all the work for output t.  When the warp's 16 rows hold at most SCAP nonzeros
+      // (always below 3 % density) all four iterations are staged first and spread in one pass after the loop.
+      const uint32_t tot = kept(0xFFFFFFFFu);
+      if (tot) {                                        // warp-uniform
+        const uint32_t ex = kept(lt);                   // this lane's first output of the iteration (lane order = (row, column) order)
+        const bool all_at_once = warp_total <= (uint32_t)SCAP;
+        for (uint32_t c0 = 0; c0 < tot; c0 += 32u) {    // one chunk below ~6 % density
+          if (m) {
+            uint32_t i = all_at_once ? (wdone + ex) : (ex - c0);
 #pragma unroll
-              for (int j = 0; j < NW; ++j) {
-                const uint32_t v[4] = { w[it][j].x, w[it][j].y, w[it][j].z, w[it][j].w };
-                for (uint32_t mm = (m >> (8 * j)) & 0xFFu; mm; mm &= mm - 1u, ++i) {
-                  if (all_at_once || i < 32u) {           // unsigned: outputs before this chunk wrap around
-                    const int e = __ffs((int)mm) - 1;
-                    const uint32_t pr = (e & 4) ? ((e & 2) ? v[3] : v[2]) : ((e & 2) ? v[1] : v[0]);
-                    const uint32_t vb = (e & 1) ? (pr & 0xFFFF0000u) : (pr << 16);
-                    stg[i] = make_uint2(vb | m, (uint32_t)(8 * j + e) | ((uint32_t)lane << 4) | ((uint32_t)it << 9));
-                  }
+            for (int j = 0; j < NW; ++j) {
+              const uint32_t v[4] = { w[it][j].x, w[it][j].y, w[it][j].z, w[it][j].w };
+              for (uint32_t mm = (m >> (8 * j)) & 0xFFu; mm; mm &= mm - 1u, ++i) {
+                if (all_at_once || i < 32u) {           // unsigned: outputs before this chunk wrap around
+                  const int e = __ffs((int)mm) - 1;
+                  const uint32_t pr = (e & 4) ? ((e & 2) ? v[3] : v[2]) : ((e & 2) ? v[1] : v[0]);
+                  const uint32_t vb = (e & 1) ? (pr & 0xFFFF0000u) : (pr << 16);
+                  stg[i] = make_uint2(vb | m, (uint32_t)(8 * j + e) | ((uint32_t)lane << 4) | ((uint32_t)it << 9));
                 }
               }
             }
-            if (all_at_once) break;
-            __syncwarp();
-            if (c0 + (uint32_t)lane < tot) spread(stg[lane], pos + c0 + (uint32_t)lane);
-            __syncwarp();                                 // the stage is rewritten by the next chunk / iteration
           }
-        }
-        pos += tot; wdone += tot;
-        continue;
-      }
-      if (m) {   // few lanes hold nonzeros in the sparse regime
-        uint32_t q = rowpos + kept(lt & rowmask);
-        const uint32_t rowm = (uint32_t)r & 127u;
-        const uint32_t k0 = (uint32_t)hl * (8u * NW);                  // first column of this lane
-        const uint32_t rbase = ((k0 >> 6) << 15) | ((rowm >> 3) * 512u + (rowm & 7u) * 64u);
-#pragma unroll
-        for (int j = 0; j < NW; ++j) {             // the lane's 16-byte words: k = k0 + 8 * j + e
-          const uint32_t v[4] = { w[it][j].x, w[it][j].y, w[it][j].z, w[it][j].w };
-          // xb_tc16_pack(r, k, value) = value | (base16 + e): everything but e is fixed for this lane, row and word
-          const uint32_t base16 = rbase | (((((k0 >> 3) + (uint32_t)j) ^ rowm) & 7u) << 3);
-          for (uint32_t mm = (m >> (8 * j)) & 0xFFu; mm; mm &= mm - 1u, ++q) {
-            const int e = __ffs((int)mm) - 1;
-            const uint32_t pr = (e & 4) ? ((e & 2) ? v[3] : v[2]) : ((e & 2) ? v[1] : v[0]);
-            const uint32_t vb = (e & 1) ? (pr & 0xFFFF0000u) : (pr << 16);
-            co[q] = (uint16_t)(k0 + 8u * j + (uint32_t)e);
-            va[q] = __uint_as_float(vb);
-            if (aux) rk[q] = vb | (base16 + (uint32_t)e);
-          }
+          if (all_at_once) break;
+          __syncwarp();
+          if (c0 + (uint32_t)lane < tot) spread(stg[lane], pos + c0 + (uint32_t)lane);
+          __syncwarp();                                 // the stage is rewritten by the next chunk / iteration
         }
       }
-      pos += kept(0xFFFFFFFFu);
+      pos += tot; wdone += tot;
     }
   }
-  if (2 == NW && warp_total <= (uint32_t)SCAP && warp_total > 0) {     // all iterations staged: one spread pass
+  if (warp_total <= (uint32_t)SCAP && warp_total > 0) {     // all iterations staged: one spread pass
     __syncwarp();
     for (uint32_t c0 = 0; c0 < warp_total; c0 += 32u)
       if (c0 + (uint32_t)lane < warp_total) spread(stg[c0 + lane], pos0 + c0 + (uint32_t)lane);
   }
   if (SEQ > 1) __syncthreads();             // wtot and the stages are reused by the next part
   }
-  if (P > 1) k1_finish(p, epoch);
 }
 
-// split: the slices of a whole pass are cut into four 8-warp CTAs each (k1_scan); a lone slice (legacy per-block calls, which
-// may run concurrently on several streams of one handle) keeps the one-CTA form, which shares no state between launches
-template <bool BF16, int ROWS, bool KEEP>
-static void launch_slice_n(const SliceArgs& args, int nslices, bool full, bool split, cudaStream_t stream)
+// K1x takes a slicing pass over bf16 A (transa = 'N') whose blocks are all complete 128-column blocks inside the reference's
+// vector loops and whose rows are 16-byte aligned.  It is the only slicing kernel that writes SliceArena::tcsp.
+static bool k1x_takes(const SliceArgs& a)
 {
-  if (split) {
-    if (full) spmdm_slice_n_kernel<BF16, true, ROWS, KEEP, 8><<<(unsigned)nslices * 4, 256, 0, stream>>>(args);
-    else spmdm_slice_n_kernel<BF16, false, ROWS, KEEP, 8><<<(unsigned)nslices * 4, 256, 0, stream>>>(args);
-  }
-  else if (full) XB_CUDA(launch_pdl(spmdm_slice_n_kernel<BF16, true, ROWS, KEEP, 32>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
-  else XB_CUDA(launch_pdl(spmdm_slice_n_kernel<BF16, false, ROWS, KEEP, 32>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
+  return !a.transa && a.is_bf16 && !a.origin_is_block && 0 == (a.g.k % 128) && a.simd_w > 1 && 0 == (a.lda & 7) && 0 == ((uintptr_t)a.a & 15);
 }
 
-// the wide bf16 kernel with two words per lane, one CTA per slice, is the only slicing kernel that writes SliceArena::tcsp
-static bool k1_split_env()
-{
-  static const bool split_env = [] { const char* e = getenv("LIBXSMM_B200_K1_SPLIT"); return e && '1' == *e; }();
-  return split_env;
-}
 bool slices_get_sp_words(const SliceArgs& args)
 {
-  if (args.transa || !args.is_bf16 || args.origin_is_block || 0 == args.write_sp || 0 == args.out.tcsp) return false;
-  const bool full = (0 == (args.g.k % 128)) && (args.simd_w > 1);
-  if (!(full && 0 == (args.lda & 7) && 0 == ((uintptr_t)args.a & 15) && 0 == (args.g.k & 7))) return false;
-  const char* wenv = getenv("LIBXSMM_B200_K1_WIDE");
-  const int wide = (wenv && *wenv >= '0' && *wenv <= '2') ? (*wenv - '0') : 2;
-  return wide >= 2 && !k1_split_env();
+  return k1x_takes(args) && 0 != args.write_sp && 0 != args.out.tcsp;
+}
+
+template <bool BF16, int ROWS>
+static void launch_slice_n(const SliceArgs& args, int nslices, bool full, cudaStream_t stream)
+{
+  if (full) XB_CUDA(launch_pdl(spmdm_slice_n_kernel<BF16, true, ROWS>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
+  else XB_CUDA(launch_pdl(spmdm_slice_n_kernel<BF16, false, ROWS>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
 }
 
 void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream)
@@ -825,51 +629,25 @@ void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream)
   if (nslices <= 0) return;
   if (!args.transa) {
     count_launch(1);
-    // FULL: every slice is a complete 128-column block inside the reference's vector loops (k % 128 == 0
-    // makes the NaN rule of the scalar remainder unreachable)
-    const bool full = (0 == (args.g.k % 128)) && (args.simd_w > 1);
     const int rpw = (args.g.bm + K1N_WARPS - 1) / K1N_WARPS;
-    // LIBXSMM_B200_K1_SPLIT=1: four 8-warp CTAs per slice chained by a decoupled look-back (k1_scan).  Measured on B200 it is
-    // SLOWER than one 32-warp CTA per slice (4096^2 bf16: 32.7 vs 23.3 us; 2048^2 fp32: 29.2 vs 19.0 us): the three hops
-    // of the look-back cost more than the overlap of the parts' phases gains.  Kept as an experiment, off by default.
-    const bool split = k1_split_env() && nslices > 1 && !args.origin_is_block && 0 != args.out.lookback && 0 != args.out.epoch;
-    if (args.is_bf16 && full && !args.origin_is_block && 0 == (args.lda & 7) && 0 == ((uintptr_t)args.a & 15) && 0 == (args.g.k & 7)) {
-      // complete 128-column blocks, 16-byte aligned rows: the wide kernel (a lane holds 8 elements)
-      const char* wenv = getenv("LIBXSMM_B200_K1_WIDE");      // developer switch, read per call (tests flip it)
-      const int wide = (wenv && *wenv >= '0' && *wenv <= '2') ? (*wenv - '0') : 2;
-      if (wide >= 2) {      // two 16-byte words per lane (default; LIBXSMM_B200_K1_WIDE=1: one word, =0: the generic kernel)
-        if (split) {
-          if (rpw <= 8) spmdm_slice_bf16x_kernel<8, 2, 8><<<(unsigned)nslices * 4, 256, 0, stream>>>(args);
-          else spmdm_slice_bf16x_kernel<16, 2, 8><<<(unsigned)nslices * 4, 256, 0, stream>>>(args);
-        }
-        else {
-          // 512-row slices: one 16-warp CTA that does the two halves of its slice one after the other, two such CTAs per SM (all
-          // 256 slices of a 4096^2 matrix resident at once instead of 1.73 waves of 32-warp CTAs).  Same time for the kernel alone
-          // (18.3 us), 1.1 us less per C2 step.  LIBXSMM_B200_K1_SEQ=1 (developer switch, read per call): one 32-warp CTA per slice.
-          const char* seq = getenv("LIBXSMM_B200_K1_SEQ");
-          if (rpw <= 8) XB_CUDA(launch_pdl(spmdm_slice_bf16x_kernel<8, 2, 32>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
-          else if (!(seq && '1' == *seq)) XB_CUDA(launch_pdl(spmdm_slice_bf16x_kernel<16, 2, 16, 2>, dim3((unsigned)nslices), dim3(512), 0, stream, args));
-          else XB_CUDA(launch_pdl(spmdm_slice_bf16x_kernel<16, 2, 32>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
-        }
-        XB_CUDA(cudaGetLastError());
-        return;
-      }
-      if (wide) {
-        if (rpw <= 8) spmdm_slice_bf16w_kernel<8><<<(unsigned)nslices, K1N_THREADS, 0, stream>>>(args);
-        else spmdm_slice_bf16w_kernel<16><<<(unsigned)nslices, K1N_THREADS, 0, stream>>>(args);
-        XB_CUDA(cudaGetLastError());
-        return;
-      }
-    }
-    if (args.is_bf16) {
-      static const int keep16 = [] { const char* e = getenv("LIBXSMM_B200_K1_KEEP"); return (e && '1' == *e) ? 1 : 0; }();
-      if (rpw <= 8) launch_slice_n<true, 8, true>(args, nslices, full, split, stream);
-      else if (keep16) launch_slice_n<true, 16, true>(args, nslices, full, split, stream);
-      else launch_slice_n<true, 16, false>(args, nslices, full, split, stream);
+    if (k1x_takes(args)) {
+      // 512-row slices: one 16-warp CTA that does the two halves of its slice one after the other, two such CTAs per SM (all
+      // 256 slices of a 4096^2 matrix resident at once instead of 1.73 waves of 32-warp CTAs): 1.1 us less per C2 step
+      if (rpw <= 8) XB_CUDA(launch_pdl(spmdm_slice_bf16x_kernel<8, 32>, dim3((unsigned)nslices), dim3(K1N_THREADS), 0, stream, args));
+      else XB_CUDA(launch_pdl(spmdm_slice_bf16x_kernel<16, 16>, dim3((unsigned)nslices), dim3(512), 0, stream, args));
     }
     else {
-      if (rpw <= 8) launch_slice_n<false, 8, true>(args, nslices, full, split, stream);
-      else launch_slice_n<false, 16, false>(args, nslices, full, split, stream);
+      // FULL: every slice is a complete 128-column block inside the reference's vector loops (k % 128 == 0
+      // makes the NaN rule of the scalar remainder unreachable)
+      const bool full = (0 == (args.g.k % 128)) && (args.simd_w > 1);
+      if (args.is_bf16) {
+        if (rpw <= 8) launch_slice_n<true, 8>(args, nslices, full, stream);
+        else launch_slice_n<true, 16>(args, nslices, full, stream);
+      }
+      else {
+        if (rpw <= 8) launch_slice_n<false, 8>(args, nslices, full, stream);
+        else launch_slice_n<false, 16>(args, nslices, full, stream);
+      }
     }
     XB_CUDA(cudaGetLastError());
     return;
@@ -1205,10 +983,9 @@ static int tc_mode()
   return ('0' == *e) ? 0 : (('1' == *e) ? 1 : 2);
 }
 
-// bf16 tensor-core branch: the CTA-pair kernel (K4p), the single-CTA kernel (K4h) when LIBXSMM_B200_TC16_PAIR=0
+// bf16 tensor-core branch: the 2:4 structured-sparse kernel (K4s) when it qualifies, else the CTA-pair kernel (K4p)
 static bool launch_tc_bf16(const ComputeArgs& a, cudaStream_t stream)
 {
-  const char* e = getenv("LIBXSMM_B200_TC16_PAIR");
   if (launch_compute_tc16s(a, stream)) {                 // 2:4 structured-sparse form (low density, slices from the wide kernel)
     const char* fe = getenv("LIBXSMM_B200_TC16_SPARSE");
     if (a.sp_guard && !(fe && '1' == *fe)) {             // the estimate is fresh or has just moved: the dense kernel stands by (ComputeArgs::sp_guard)
@@ -1218,23 +995,19 @@ static bool launch_tc_bf16(const ComputeArgs& a, cudaStream_t stream)
     }
     return true;
   }
-  if (!(e && '0' == *e) && launch_compute_tc16p(a, stream)) return true;
-  return launch_compute_tc16(a, stream);
+  return launch_compute_tc16p(a, stream);
 }
 
-// fp32 tensor-core branch: the CTA-pair kernel when the slices carry their dense image (LIBXSMM_B200_TCQ=0: never),
-// else the single-CTA kernel
+// fp32 tensor-core branch: the CTA-pair kernel (K4q) when the slices carry their dense image, else the single-CTA kernel (K4)
 static bool launch_tc_f32(const ComputeArgs& a, cudaStream_t stream)
 {
-  const char* e = getenv("LIBXSMM_B200_TCQ");
-  if (!(e && '0' == *e) && launch_compute_tcq(a, stream)) return true;
-  return launch_compute_tc(a, stream);
+  return launch_compute_tcq(a, stream) || launch_compute_tc(a, stream);
 }
 
 static void launch_part(const ComputeArgs& a, bool partial, cudaStream_t stream)
 {
-  if (!partial && launch_compute_sp(a, stream)) return;  // K2s: cluster-multicast TMA kernel (spmdm_compute_sp.cu)
-  if (launch_compute_tma(a, partial, stream)) return;   // K2: narrow-block parts and LIBXSMM_B200_K2S=0 (spmdm_compute_tma.cu)
+  if (!partial && launch_compute_sp(a, stream)) return;  // K2s: TMA ring, list-driven row walk (spmdm_compute_sp.cu)
+  if (launch_compute_tma(a, partial, stream)) return;   // K2: the narrow-block parts and what K2s refuses (spmdm_compute_tma.cu)
   if (a.is_bf16) {
     if (partial) launch_compute_variant<true, true, 4>(a, stream);
     else launch_compute_variant<true, false, 8>(a, stream);

@@ -45,15 +45,19 @@ def valid_slices_equal(g, got, want):
     return int(cnt.sum())
 
 
-def gpu_spmdm(xs, A, B, C0, M, N, K, transa="N", transb="N", transc="N", beta=0.0, bf16=False, max_threads=1):
-    """slice + compute on device buffers through the stream entries; returns (geometry, slices, C)."""
+def gpu_spmdm(xs, A, B, C0, M, N, K, transa="N", transb="N", transc="N", beta=0.0, bf16=False, max_threads=1, a_offset=0):
+    """slice + compute on device buffers through the stream entries; returns (geometry, slices, C).
+    a_offset: A is placed that many bytes past the start of its (256-byte aligned) device buffer."""
     import pyoracle
     p = xs.Spmdm(M, N, K, max_threads)
     try:
-        dA = xs.DeviceBuffer.from_numpy(A)
+        A = np.ascontiguousarray(A)
+        dA = xs.DeviceBuffer(max(A.nbytes + a_offset, 1))
+        if A.nbytes:
+            dA.upload(A, a_offset)
         dB = xs.DeviceBuffer.from_numpy(B)
         dC = xs.DeviceBuffer.from_numpy(C0)
-        p.create_slices(dA, transa, bf16)
+        p.create_slices(dA.ptr + a_offset, transa, bf16)
         p.compute(dB, dC, transb, transc, beta, bf16)
         xs.synchronize()
         sl = p.read_slices()
@@ -171,14 +175,13 @@ def test_special_values_in_a(gpu, oracle):
     np.testing.assert_array_equal(C[ok].view(np.uint32), OC[ok].view(np.uint32))
 
 
-@pytest.mark.parametrize("wide", ["2", "2-one-cta", "1", "0"])
-def test_special_values_bf16_wide_slicing(gpu, oracle, monkeypatch, wide):
-    """bf16 bit patterns through the slicing kernels for complete, aligned blocks (two / one 16-byte word per lane,
-    generic): +-0, NaN with either sign, +-Inf, denormals, the largest finite value, dense and empty lanes and rows --
-    kept iff ordered-nonzero like the reference's vector loops (quirk Q3).  Slices bit for bit against the oracle."""
-    monkeypatch.setenv("LIBXSMM_B200_K1_WIDE", wide[0])
-    if wide.endswith("one-cta"):     # the two-word kernel as one 32-warp CTA per slice instead of a 16-warp CTA doing both halves in turn
-        monkeypatch.setenv("LIBXSMM_B200_K1_SEQ", "1")
+@pytest.mark.parametrize("wide", ["2", "0"])
+def test_special_values_bf16_wide_slicing(gpu, oracle, wide):
+    """bf16 bit patterns through the slicing kernels for complete blocks: +-0, NaN with either sign, +-Inf, denormals,
+    the largest finite value, dense and empty lanes and rows -- kept iff ordered-nonzero like the reference's vector
+    loops (quirk Q3).  Slices bit for bit against the oracle.  wide = 16-byte words per lane of the kernel that slices A:
+    "2" = the wide kernel (16-byte aligned rows), "0" = the generic kernel, reached with A 8 bytes past a 16-byte
+    boundary (it still takes the complete-block form and 8-byte loads)."""
     M, N, K = 600, 48, 256           # two complete k-blocks, row pitch 512 B; two row blocks (512 + 88 rows)
     rng = np.random.default_rng(11)
     bits = np.where(rng.random((M, K)) < 0.05, rng.integers(1, 0x7F80, (M, K)), 0).astype(np.uint16)
@@ -193,7 +196,7 @@ def test_special_values_bf16_wide_slicing(gpu, oracle, monkeypatch, wide):
     A = np.ascontiguousarray(bits)
     B = gpu.workloads.to_bf16_bits(rng.random((K, N)).astype(np.float32))
     C0 = rng.random((M, N)).astype(np.float32)
-    g, sl, C = gpu_spmdm(gpu, A, B, C0, M, N, K, beta=0, bf16=True)
+    g, sl, C = gpu_spmdm(gpu, A, B, C0, M, N, K, beta=0, bf16=True, a_offset=0 if "2" == wide else 8)
     og, osl, OC = oracle_spmdm(oracle, g, A, B, C0, "N", "N", "N", 0.0)
     nnz = valid_slices_equal(og, sl, osl)
     keep = ((bits & 0x7FFF) >= 1) & ((bits & 0x7FFF) <= 0x7F80)

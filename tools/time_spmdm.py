@@ -1,6 +1,5 @@
 """Developer tool: times the slicing and compute kernels of one spmdm workload with CUDA events
-(ring of inputs larger than L2, like bench.py) and prints one line.  Kernel variants are selected by
-environment variables read by the library (LIBXSMM_B200_K2_VARIANT ...).
+(ring of inputs larger than L2, like bench.py) and prints one line.
 
     python tools/time_spmdm.py c2 [reps]
 """
@@ -26,8 +25,8 @@ def main():
     for _ in gen:
         pass
     p = r["parts"]
-    print("%s variant=%s: step %.1f us  slice %.1f us (%.0f GB/s)  compute %.1f us (%.0f GB/s, %.0f GFLOP/s)" % (
-        name, os.environ.get("LIBXSMM_B200_K2_VARIANT", "-"), r["total_ms"] / reps * 1e3, p["slice_ms"] * 1e3,
+    print("%s: step %.1f us  slice %.1f us (%.0f GB/s)  compute %.1f us (%.0f GB/s, %.0f GFLOP/s)" % (
+        name, r["total_ms"] / reps * 1e3, p["slice_ms"] * 1e3,
         p["slice_bytes"] / p["slice_ms"] / 1e6, p["compute_ms"] * 1e3, p["compute_bytes"] / p["compute_ms"] / 1e6,
         r["flops"] / p["compute_ms"] / 1e6))
 

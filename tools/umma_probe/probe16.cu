@@ -1,5 +1,5 @@
 // Developer probe: 128x128x64 BF16 tcgen05.mma chain; A K-major SWIZZLE_128B, B MN-major SWIZZLE_128B (the [k][n] tile a TMA
-// box of 64 columns lands), to pin LBO / SBO / k-step for spmdm_compute_tc16.cu.
+// box of 64 columns lands), to pin LBO / SBO / k-step for the bf16 tensor-core kernels (spmdm_compute_tc16p.cu).
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
 #include <cstdio>
