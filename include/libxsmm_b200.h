@@ -159,6 +159,32 @@ LIBXSMM_API void libxsmm_b200_csr_soa_execute(const libxsmm_b200_csr_soa* handle
 LIBXSMM_API int libxsmm_b200_csr_soa_is_baked(const libxsmm_b200_csr_soa* handle);
 LIBXSMM_API void libxsmm_b200_csr_soa_destroy(libxsmm_b200_csr_soa* handle);
 
+/* Dense x SoA kernels: the GPU counterparts of
+ *     kernel = libxsmm_create_rm_ac_soa(descriptor(m, n, k, lda, ldb, ldc, alpha = 1, beta))   or   libxsmm_create_rm_bc_soa(...)
+ *     kernel(a, b, c)                                        once per mesh element
+ * (reference src/libxsmm_main.c:2477,2500).  Layout as for the csr_soa entries: an SoA operand with R rows and pitch ld is
+ * [R][ld][soa_width], a plain operand is row-major with pitch ld, strides count scalars.
+ *   ac form  A [M][lda][soa_width], b K x N (pitch ldb), C [M][ldc][soa_width]:
+ *            C[m][n][s] = chain over k = 0 .. K-1 ascending of acc = fma(A[m][k][s], b[k][n], acc);
+ *   bc form  a M x K (pitch lda), B [K][ldb][soa_width], C [M][ldc][soa_width]:
+ *            C[m][n][s] = chain over k = 0 .. K-1 ascending of acc = fma(a[m][k], B[k][n][s], acc);
+ * acc starts from C[m][n][s] for beta = 1 and from +0 for beta = 0 (C is then never read).  One rounding per k; zeros are not
+ * skipped (0 * Inf gives NaN).  Exactly the columns 0 .. N-1 of every C row are written.  alpha is 1; beta must be 0 or 1.
+ * Create is host only (no CUDA call) and returns NULL with the sticky error set for an empty shape (-80), a pitch smaller than
+ * its extent (lda < K, ldb < N, ldc < N: -81) or another beta (-82).  Execute is BATCHED and asynchronous on `stream`: element e
+ * has its operands at d_a + e * stride_a, d_b + e * stride_b and d_c + e * stride_c (DEVICE pointers, strides in scalars).  An
+ * input stride of 0 shares that operand among all elements.  n_elements = 0 does nothing; a negative count or stride, or
+ * n_elements > 1 with stride_c below one element's C extent ((M-1) * ldc + N) * soa_width, sets error -83 and launches nothing.
+ * All operands are read at call time. */
+typedef struct libxsmm_b200_rm_soa libxsmm_b200_rm_soa;
+LIBXSMM_API libxsmm_b200_rm_soa* libxsmm_b200_drm_ac_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, double beta);
+LIBXSMM_API libxsmm_b200_rm_soa* libxsmm_b200_srm_ac_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, float beta);
+LIBXSMM_API libxsmm_b200_rm_soa* libxsmm_b200_drm_bc_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, double beta);
+LIBXSMM_API libxsmm_b200_rm_soa* libxsmm_b200_srm_bc_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, float beta);
+LIBXSMM_API void libxsmm_b200_rm_soa_execute(const libxsmm_b200_rm_soa* handle, const void* d_a, const void* d_b, void* d_c,
+  long long n_elements, long long stride_a, long long stride_b, long long stride_c, void* stream);
+LIBXSMM_API void libxsmm_b200_rm_soa_destroy(libxsmm_b200_rm_soa* handle);
+
 /* Dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3): the GPU counterpart of
  *     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, flags, prefetch)
  *     for (i = 0; i < N; i += nblock) kernel(B_panel + i, A_op, C_panel + i)

@@ -54,6 +54,8 @@ ADDED_SYMBOLS = [
     "libxsmm_b200_dcsr_soa_create", "libxsmm_b200_scsr_soa_create", "libxsmm_b200_csr_soa_execute", "libxsmm_b200_csr_soa_is_baked",
     "libxsmm_b200_csr_soa_destroy", "libxsmm_b200_dcsc_soa_create", "libxsmm_b200_scsc_soa_create",
     "libxsmm_b200_dmmdispatch", "libxsmm_b200_smmdispatch", "libxsmm_b200_mm_execute", "libxsmm_b200_mm_kernel", "libxsmm_b200_mm_release",
+    "libxsmm_b200_drm_ac_soa_create", "libxsmm_b200_srm_ac_soa_create", "libxsmm_b200_drm_bc_soa_create", "libxsmm_b200_srm_bc_soa_create",
+    "libxsmm_b200_rm_soa_execute", "libxsmm_b200_rm_soa_destroy",
 ]
 
 
@@ -717,6 +719,68 @@ class CsrSoa:
             L.libxsmm_b200_csr_soa_destroy.argtypes = [ctypes.c_void_p]
             L.libxsmm_b200_csr_soa_destroy(self.handle)
             self.handle = None
+
+
+class RmSoa:
+    """Dense operand applied to [element][row][column][soa] tensors (libxsmm_b200_[sd]rm_{ac,bc}_soa_*; the batched GPU counterpart of
+    libxsmm_create_rm_ac_soa / libxsmm_create_rm_bc_soa).  form="ac": A [M][lda][soa] and C [M][ldc][soa] are SoA, b is K x N
+    row-major; form="bc": B [K][ldb][soa] and C are SoA, a is M x K row-major.  Pitches default to the dense extents."""
+
+    def __init__(self, form, M, N, K, soa, dtype, lda=None, ldb=None, ldc=None, beta=0.0):
+        assert form in ("ac", "bc")
+        self.double = np.dtype(dtype) == np.float64
+        assert self.double or np.dtype(dtype) == np.float32
+        self.form, self.M, self.N, self.K, self.soa = form, M, N, K, soa
+        self.lda = K if lda is None else lda
+        self.ldb = N if ldb is None else ldb
+        self.ldc = N if ldc is None else ldc
+        self.handle = rm_soa_create(form, self.double, M, N, K, self.lda, self.ldb, self.ldc, soa, beta)
+        if not self.handle:
+            code, msg = last_error()
+            clear_error()
+            raise ValueError("rm_soa_create failed (%d): %s" % (code, msg))
+
+    @property
+    def extents(self):
+        """scalars of one element's (first operand, second operand, C) as they lie in memory"""
+        a = ((self.M - 1) * self.lda + self.K) * (self.soa if self.form == "ac" else 1)
+        b = ((self.K - 1) * self.ldb + self.N) * (self.soa if self.form == "bc" else 1)
+        return a, b, ((self.M - 1) * self.ldc + self.N) * self.soa
+
+    def execute(self, d_a, d_b, d_c, n_elements, stride_a=None, stride_b=None, stride_c=None, stream=None):
+        """stride None: the dense extent of one element (M lda, K ldb or M ldc rows, times soa for an SoA operand)"""
+        sa = self.M * self.lda * (self.soa if self.form == "ac" else 1) if stride_a is None else stride_a
+        sb = self.K * self.ldb * (self.soa if self.form == "bc" else 1) if stride_b is None else stride_b
+        sc = self.M * self.ldc * self.soa if stride_c is None else stride_c
+        rm_soa_execute(self.handle, d_a, d_b, d_c, n_elements, sa, sb, sc, stream)
+
+    def destroy(self):
+        if self.handle:
+            rm_soa_destroy(self.handle)
+            self.handle = None
+
+
+def rm_soa_create(form, double, M, N, K, lda, ldb, ldc, soa, beta):
+    """the raw create entry (host only): the handle or None"""
+    L = load()
+    f = getattr(L, "libxsmm_b200_%srm_%s_soa_create" % ("d" if double else "s", form))
+    f.restype = ctypes.c_void_p
+    f.argtypes = [ctypes.c_int] * 7 + [ctypes.c_double if double else ctypes.c_float]
+    return f(M, N, K, lda, ldb, ldc, soa, float(beta))
+
+
+def rm_soa_execute(handle, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, stream=None):
+    L = load()
+    L.libxsmm_b200_rm_soa_execute.restype = None
+    L.libxsmm_b200_rm_soa_execute.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_longlong] * 4 + [ctypes.c_void_p]
+    L.libxsmm_b200_rm_soa_execute(handle, _addr(d_a), _addr(d_b), _addr(d_c), n_elements, stride_a, stride_b, stride_c, _sptr(stream))
+
+
+def rm_soa_destroy(handle):
+    L = load()
+    L.libxsmm_b200_rm_soa_destroy.restype = None
+    L.libxsmm_b200_rm_soa_destroy.argtypes = [ctypes.c_void_p]
+    L.libxsmm_b200_rm_soa_destroy(handle)
 
 
 # ---- host-only planning (works without a GPU) ----------------------------------------------------------

@@ -888,6 +888,50 @@ void libxsmm_b200_csr_soa_execute(const libxsmm_b200_csr_soa* handle, const void
 int libxsmm_b200_csr_soa_is_baked(const libxsmm_b200_csr_soa* handle) { return fs_is_baked((const FsOperator*)handle); }
 void libxsmm_b200_csr_soa_destroy(libxsmm_b200_csr_soa* handle) { fs_destroy((FsOperator*)handle); }
 
+// ---- dense SoA kernels (rm_soa.cu) ---------------------------------------------------------------------------------------------
+// GPU counterparts of libxsmm_create_rm_ac_soa / libxsmm_create_rm_bc_soa (reference src/libxsmm_main.c:2477,2500), batched over
+// mesh elements like csr_soa_execute.  Create only checks the descriptor (host only, no CUDA call); execute reads all three
+// operands at call time.
+struct libxsmm_b200_rm_soa;
+static libxsmm_b200_rm_soa* rm_soa_create(int is_double, int form, int M, int N, int K, int lda, int ldb, int ldc, int soa, double beta)
+{
+  static const char* const nm[2] = {"rm_ac_soa_create", "rm_bc_soa_create"};
+  if (M < 1 || N < 1 || K < 1 || soa < 1) { set_error(-80, "%s: empty shape (M=%d N=%d K=%d soa_width=%d)", nm[form], M, N, K, soa); return 0; }
+  if (lda < K || ldb < N || ldc < N) { set_error(-81, "%s: pitch smaller than its extent (lda=%d >= K=%d, ldb=%d >= N=%d, ldc=%d >= N)", nm[form], lda, K, ldb, N, ldc); return 0; }
+  if (!(0.0 == beta || 1.0 == beta)) { set_error(-82, "%s: beta=%g; it must be 0 or 1 like the reference's JIT", nm[form], beta); return 0; }
+  RmSoa* h = new RmSoa();
+  h->is_double = is_double; h->form = form; h->M = M; h->N = N; h->K = K; h->lda = lda; h->ldb = ldb; h->ldc = ldc; h->soa = soa;
+  h->beta_one = 1.0 == beta;
+  return (libxsmm_b200_rm_soa*)h;
+}
+libxsmm_b200_rm_soa* libxsmm_b200_drm_ac_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, double beta)
+{ return rm_soa_create(1, 0, M, N, K, lda, ldb, ldc, soa_width, beta); }
+libxsmm_b200_rm_soa* libxsmm_b200_srm_ac_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, float beta)
+{ return rm_soa_create(0, 0, M, N, K, lda, ldb, ldc, soa_width, (double)beta); }
+libxsmm_b200_rm_soa* libxsmm_b200_drm_bc_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, double beta)
+{ return rm_soa_create(1, 1, M, N, K, lda, ldb, ldc, soa_width, beta); }
+libxsmm_b200_rm_soa* libxsmm_b200_srm_bc_soa_create(int M, int N, int K, int lda, int ldb, int ldc, int soa_width, float beta)
+{ return rm_soa_create(0, 1, M, N, K, lda, ldb, ldc, soa_width, (double)beta); }
+void libxsmm_b200_rm_soa_execute(const libxsmm_b200_rm_soa* handle, const void* d_a, const void* d_b, void* d_c, long long n_elements,
+  long long stride_a, long long stride_b, long long stride_c, void* stream)
+{
+  const RmSoa* h = (const RmSoa*)handle;
+  if (0 == h) { set_error(-83, "rm_soa_execute: NULL handle"); return; }
+  if (n_elements < 0 || stride_a < 0 || stride_b < 0 || stride_c < 0) {
+    set_error(-83, "rm_soa_execute: negative count or stride (n_elements=%lld stride_a=%lld stride_b=%lld stride_c=%lld)", n_elements, stride_a, stride_b, stride_c);
+    return;
+  }
+  if (0 == n_elements) return;
+  const long long c_extent = ((long long)(h->M - 1) * h->ldc + h->N) * h->soa;
+  if (n_elements > 1 && stride_c < c_extent) {
+    set_error(-83, "rm_soa_execute: stride_c=%lld is smaller than one element's C (%lld scalars): elements would overlap", stride_c, c_extent);
+    return;
+  }
+  if (0 == d_a || 0 == d_b || 0 == d_c) { set_error(-83, "rm_soa_execute: NULL operand"); return; }
+  rm_soa_execute(*h, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, (cudaStream_t)stream);
+}
+void libxsmm_b200_rm_soa_destroy(libxsmm_b200_rm_soa* handle) { delete (RmSoa*)handle; }
+
 // ---- dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3) ---------------------------
 // The reference's callers apply a DENSE fixed operator to a row-major panel with the column-major SMM kernel
 //     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, ...)

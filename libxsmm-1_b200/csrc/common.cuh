@@ -258,4 +258,10 @@ int fs_is_double(const FsOperator* o);
 void fs_shape(const FsOperator* o, int* M, int* N, int* K, int* ldb, int* ldc, int* beta_one);
 void fs_destroy(FsOperator* op);
 
+// ---- dense SoA kernels (rm_soa.cu) ----------------------------------------------------------
+// form 0: ac (A and C are [row][ld][soa], b is plain row-major), 1: bc (B and C are SoA, a is plain)
+struct RmSoa { int is_double, form, M, N, K, lda, ldb, ldc, soa, beta_one; };
+void rm_soa_execute(const RmSoa& h, const void* d_a, const void* d_b, void* d_c, long long n_elem, long long stride_a,
+                    long long stride_b, long long stride_c, cudaStream_t stream);
+
 }  // namespace xb
