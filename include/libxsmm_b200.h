@@ -18,6 +18,18 @@ LIBXSMM_API void libxsmm_spmdm_createSparseSlice_fp32_stream(const libxsmm_spmdm
 LIBXSMM_API void libxsmm_spmdm_createSparseSlice_bfloat16_stream(const libxsmm_spmdm_handle* handle, char transa,
   const libxsmm_bfloat16* d_a, libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
 
+/* A (M x K, the handle's shape) in CSR form: row_ptr[M + 1], col_idx[nnz], values[nnz], all DEVICE pointers, 0-based,
+ * column indices strictly ascending within each row.  Fills the handle's slices exactly as createSparseSlice_*_stream would
+ * for the dense matrix holding these entries (transa = 'N'); asynchronous on stream.  The compute entries then take the
+ * slices unchanged.  Errors (sticky, nothing launched): -90 NULL row_ptr, or NULL col_idx / values with nnz > 0;
+ * -91 nnz < 0 or nnz > 2^32 - 1.  Malformed arrays on the device give unspecified slices, never writes outside them. */
+LIBXSMM_API void libxsmm_spmdm_createSparseSlice_csr_fp32_stream(const libxsmm_spmdm_handle* handle,
+  const unsigned int* d_row_ptr, const unsigned int* d_col_idx, const float* d_values, long long nnz,
+  libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
+LIBXSMM_API void libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(const libxsmm_spmdm_handle* handle,
+  const unsigned int* d_row_ptr, const unsigned int* d_col_idx, const libxsmm_bfloat16* d_values, long long nnz,
+  libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
+
 /* All block ids of reference samples/spmdm/spmdm.c:106-110 in one launch.  d_b, d_c are DEVICE pointers;
  * alpha and beta are HOST pointers read at call time (alpha is ignored like in the reference). */
 LIBXSMM_API void libxsmm_spmdm_compute_fp32_stream(const libxsmm_spmdm_handle* handle, char transa, char transb,

@@ -31,6 +31,7 @@ REFERENCE_SYMBOLS = [
 ]
 ADDED_SYMBOLS = [
     "libxsmm_spmdm_createSparseSlice_fp32_stream", "libxsmm_spmdm_createSparseSlice_bfloat16_stream",
+    "libxsmm_spmdm_createSparseSlice_csr_fp32_stream", "libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream",
     "libxsmm_spmdm_compute_fp32_stream", "libxsmm_spmdm_compute_bfloat16_stream",
     "libxsmm_spmdm_exec_host", "libxsmm_spmdm_exec_stream",
     "libxsmm_dfsspmdm_execute_stream", "libxsmm_sfsspmdm_execute_stream",
@@ -108,6 +109,9 @@ def load():
         f.restype = None
         f = getattr(L, "libxsmm_spmdm_compute_%s_stream" % nm)
         f.argtypes = [H, cc, cc, vp, S, vp, cc, vp, vp, vp]
+        f.restype = None
+        f = getattr(L, "libxsmm_spmdm_createSparseSlice_csr_%s_stream" % nm)
+        f.argtypes = [H, vp, vp, vp, ctypes.c_longlong, S, vp]
         f.restype = None
     L.libxsmm_spmdm_exec_host.argtypes = [H, S, ci, cc, cc, cc, vp, vp, vp, vp]
     L.libxsmm_spmdm_exec_host.restype = None
@@ -395,6 +399,16 @@ def libxsmm_spmdm_createSparseSlice_bfloat16_stream(handle, transa, d_a, slices,
     load().libxsmm_spmdm_createSparseSlice_bfloat16_stream(ctypes.byref(handle), _c(transa), _addr(d_a), slices, _sptr(stream))
 
 
+def libxsmm_spmdm_createSparseSlice_csr_fp32_stream(handle, d_row_ptr, d_col_idx, d_values, nnz, slices, stream=None):
+    load().libxsmm_spmdm_createSparseSlice_csr_fp32_stream(ctypes.byref(handle), _addr(d_row_ptr), _addr(d_col_idx), _addr(d_values),
+                                                           int(nnz), slices, _sptr(stream))
+
+
+def libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(handle, d_row_ptr, d_col_idx, d_values, nnz, slices, stream=None):
+    load().libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(ctypes.byref(handle), _addr(d_row_ptr), _addr(d_col_idx), _addr(d_values),
+                                                               int(nnz), slices, _sptr(stream))
+
+
 def libxsmm_spmdm_compute_fp32_stream(handle, transa, transb, alpha, slices, d_b, transc, beta, d_c, stream=None):
     al = ctypes.c_float(alpha)
     be = ctypes.c_float(beta)
@@ -528,6 +542,12 @@ class Spmdm:
     def create_slices(self, d_a, transa="N", bf16=False, stream=None):
         f = libxsmm_spmdm_createSparseSlice_bfloat16_stream if bf16 else libxsmm_spmdm_createSparseSlice_fp32_stream
         f(self.handle, transa, d_a, self.slices, stream)
+
+    def create_slices_csr(self, d_row_ptr, d_col_idx, d_values, nnz, bf16=False, stream=None):
+        """A in CSR form: device arrays row_ptr[M + 1], col_idx[nnz] (uint32, 0-based, ascending within a row) and values[nnz]
+        (float32, or bf16 bit patterns as uint16); the same slices as create_slices() on the dense matrix (transa 'N')."""
+        f = libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream if bf16 else libxsmm_spmdm_createSparseSlice_csr_fp32_stream
+        f(self.handle, d_row_ptr, d_col_idx, d_values, nnz, self.slices, stream)
 
     def compute(self, d_b, d_c, transb="N", transc="N", beta=0.0, bf16=False, stream=None, transa="N"):
         if bf16:

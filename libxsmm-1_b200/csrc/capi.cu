@@ -140,7 +140,9 @@ static bool stream_is_capturing(cudaStream_t stream)
   return cudaStreamCaptureStatusNone != st;
 }
 
-static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cudaStream_t stream)
+// dense_image = false: the slicing kernel cannot write the dense tile image (A in CSR form); an image left by an earlier pass is
+// then stale and marked so.
+static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cudaStream_t stream, bool dense_image = true)
 {
   a->acc = c->d_acc; a->host_total = c->d_nnz; a->total_slices = c->g.mb * c->g.kb;
   a->write_dense = 0; a->write_sp = 0;
@@ -167,7 +169,7 @@ static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cud
   // orientation of B and C.  Costs ~4 us of extra stores per 2048^2 and takes 50-90 us off the multiply.  Allocated and
   // zeroed on first use (rows and columns of partial tiles are never written and stay zero).
   // (A stored k x m goes through the strip kernel, which writes the image from its shared-memory tile: no alignment rule)
-  if (!is_bf16 && 0 == (c->g.k % 128) && c->simd_w > 1 && (a->transa || (0 == (a->lda & 3) && 0 == ((uintptr_t)a->a & 15)))) {
+  if (dense_image && !is_bf16 && 0 == (c->g.k % 128) && c->simd_w > 1 && (a->transa || (0 == (a->lda & 3) && 0 == ((uintptr_t)a->a & 15)))) {
     const float d = density_estimate(c);
     if (capturing || d < 0.f || d >= 0.01f) {
       if (0 == c->arena.dense && !capturing) {
@@ -195,7 +197,7 @@ static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cud
     a->out.tcsp = c->arena.tcsp; a->out.ovf_list = c->arena.ovf_list;
     a->write_sp = c->arena.tcsp ? 1 : 0;
   }
-  c->sp_written = slices_get_sp_words(*a);
+  c->sp_written = dense_image ? slices_get_sp_words(*a) : slices_csr_get_sp_words(*a);
 }
 
 static int compute_policy(const SpmdmCtx* c, int is_bf16, bool transb, bool transc)
@@ -279,6 +281,24 @@ static void slices_whole(const libxsmm_spmdm_handle* handle, char transa, const 
   a.origin_is_block = 0; a.slice0 = 0; a.slice_step = 1; a.simd_w = c->simd_w; a.g = c->g; a.out = c->arena;
   slice_policy(c, &a, is_bf16, true, stream);
   launch_slices(a, c->g.mb * c->g.kb, stream);
+}
+
+// A in CSR form (device arrays): the same slices as slices_whole() for the dense matrix holding these entries, transa = 'N'
+static void slices_csr(const libxsmm_spmdm_handle* handle, const unsigned int* d_row_ptr, const unsigned int* d_col_idx,
+                       const void* d_values, long long nnz, int is_bf16, cudaStream_t stream)
+{
+  SpmdmCtx* c = find_ctx(handle);
+  if (0 == c) return;
+  if (0 == d_row_ptr) { set_error(-90, "createSparseSlice_csr: NULL row_ptr"); return; }
+  if (nnz < 0 || nnz > 0xFFFFFFFFll) { set_error(-91, "createSparseSlice_csr: nnz=%lld outside [0, 2^32 - 1]", nnz); return; }
+  if (nnz > 0 && (0 == d_col_idx || 0 == d_values)) { set_error(-90, "createSparseSlice_csr: NULL col_idx or values with nnz=%lld", nnz); return; }
+  SliceArgs a;
+  a.a = 0; a.transa = 0; a.lda = c->g.k; a.is_bf16 = is_bf16;
+  a.origin_is_block = 0; a.slice0 = 0; a.slice_step = 1; a.simd_w = c->simd_w; a.g = c->g; a.out = c->arena;
+  slice_policy(c, &a, is_bf16, true, stream, false);
+  CsrArgs csr;
+  csr.row_ptr = d_row_ptr; csr.col_idx = d_col_idx; csr.values = d_values; csr.nnz = (uint32_t)nnz;
+  launch_slices_csr(a, csr, stream);
 }
 
 static void compute_whole(const libxsmm_spmdm_handle* handle, char transb, char transc, float beta,
@@ -551,6 +571,21 @@ void libxsmm_spmdm_createSparseSlice_bfloat16_stream(const libxsmm_spmdm_handle*
 {
   (void)libxsmm_output_csr_a;
   slices_whole(handle, transa, d_a, 1, (cudaStream_t)stream);
+}
+
+void libxsmm_spmdm_createSparseSlice_csr_fp32_stream(const libxsmm_spmdm_handle* handle, const unsigned int* d_row_ptr,
+  const unsigned int* d_col_idx, const float* d_values, long long nnz, libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream)
+{
+  (void)libxsmm_output_csr_a;
+  slices_csr(handle, d_row_ptr, d_col_idx, d_values, nnz, 0, (cudaStream_t)stream);
+}
+
+void libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(const libxsmm_spmdm_handle* handle, const unsigned int* d_row_ptr,
+  const unsigned int* d_col_idx, const libxsmm_bfloat16* d_values, long long nnz, libxsmm_CSR_sparseslice* libxsmm_output_csr_a,
+  void* stream)
+{
+  (void)libxsmm_output_csr_a;
+  slices_csr(handle, d_row_ptr, d_col_idx, d_values, nnz, 1, (cudaStream_t)stream);
 }
 
 void libxsmm_spmdm_compute_fp32_stream(const libxsmm_spmdm_handle* handle, char transa, char transb, const float* alpha,

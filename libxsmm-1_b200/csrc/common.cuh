@@ -229,6 +229,12 @@ inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, s
 #endif
 
 void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream);
+// A in CSR form (device arrays, 0-based, columns ascending within a row): row_ptr[m + 1], col_idx[nnz], values[nnz] (float or
+// bf16 bits).  launch_slices_csr writes every slice of args.g exactly as launch_slices would for the dense matrix holding these
+// entries (transa = 'N'), except the dense tile image; args.write_sp is honoured only for bf16 with k % 128 == 0 and simd_w > 1.
+struct CsrArgs { const unsigned int* row_ptr; const unsigned int* col_idx; const void* values; uint32_t nnz; };
+void launch_slices_csr(const SliceArgs& args, const CsrArgs& csr, cudaStream_t stream);
+bool slices_csr_get_sp_words(const SliceArgs& args);                     // would launch_slices_csr() write tcsp for these arguments?
 void launch_compute(const ComputeArgs& args, cudaStream_t stream);
 bool launch_compute_tma(const ComputeArgs& args, bool partial, cudaStream_t stream);
 bool launch_compute_sp(const ComputeArgs& args, cudaStream_t stream);    // K2s: order-preserving TMA-ring kernel (spmdm_compute_sp.cu)

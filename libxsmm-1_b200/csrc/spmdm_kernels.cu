@@ -669,6 +669,183 @@ void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream)
   XB_CUDA(cudaLaunchKernelEx(&cfg, spmdm_slice_kernel, args));
 }
 
+// -------------------------------------------------------------------------------------------------
+// K1c: A given in CSR form (transa = 'N') -> the same slices as K1n / K1x write for the dense matrix holding these entries.
+// One CTA per slice, one thread per row of it.  With sorted columns the slice's entries of a row are one contiguous range of
+// col_idx, found by two binary searches; the CTA then walks the concatenation of its rows' ranges ("candidates", already in
+// output order) 512 at a time, one candidate per thread, and a block scan of the keep verdicts gives each kept entry its
+// output index.  Row pointers come from per-row kept counts.  Malformed input (row_ptr not monotone or past nnz, columns
+// unsorted, duplicated or >= K) gives unspecified slices but stays inside the arrays: every row range is clamped to
+// [0, nnz] and to at most ncols candidates, and a candidate is kept only if its column lies in the slice.
+// -------------------------------------------------------------------------------------------------
+constexpr int K1C_THREADS = 512;      // >= bm: one row per thread
+constexpr int K1C_WARPS = K1C_THREADS / 32;
+
+// first index in [lo, hi) whose column is >= c (hi if none); on unsorted columns some index in [lo, hi]
+__device__ __forceinline__ uint32_t k1c_lower_bound(const unsigned int* col, uint32_t lo, uint32_t hi, uint32_t c)
+{
+  while (lo < hi) {
+    const uint32_t mid = lo + ((hi - lo) >> 1);
+    if (__ldg(col + mid) < c) lo = mid + 1; else hi = mid;
+  }
+  return lo;
+}
+
+// block-wide exclusive scan of one value per thread; returns the thread's prefix, *total the sum.  wtot: K1C_WARPS words.
+__device__ __forceinline__ uint32_t k1c_scan(uint32_t v, uint32_t* wtot, uint32_t* total)
+{
+  const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
+  uint32_t inc = v;
+#pragma unroll
+  for (int d = 1; d < 32; d <<= 1) {
+    const uint32_t u = __shfl_up_sync(0xffffffffu, inc, d);
+    if (lane >= d) inc += u;
+  }
+  __syncthreads();                       // wtot may still be read by the previous scan
+  if (31 == lane) wtot[warp] = inc;
+  __syncthreads();
+  uint32_t base = 0, sum = 0;
+#pragma unroll
+  for (int w = 0; w < K1C_WARPS; ++w) { const uint32_t t = wtot[w]; base += (w < warp) ? t : 0u; sum += t; }
+  *total = sum;
+  return base + inc - v;
+}
+
+template <bool BF16>
+__device__ __forceinline__ uint32_t k1c_bits(const void* values, uint32_t j)
+{
+  if (BF16) return (uint32_t)__ldg((const uint16_t*)values + j) << 16;
+  return __float_as_uint(__ldg((const float*)values + j));
+}
+
+template <bool BF16>
+__global__ void __launch_bounds__(K1C_THREADS, 2) spmdm_slice_csr_kernel(const SliceArgs p, const CsrArgs a)
+{
+  __shared__ uint32_t cbeg[K1C_THREADS];       // first candidate of the row in col_idx
+  __shared__ uint32_t coff[K1C_THREADS + 1];   // exclusive scan of the rows' candidate counts
+  __shared__ uint32_t kcnt[K1C_THREADS];       // kept entries of the row
+  __shared__ uint32_t wtot[K1C_WARPS];
+  pdl_wait();          // launch_pdl: the slices may still be read by the multiply in front of this kernel in the stream
+  pdl_trigger();       // ... and the multiply behind it may be scheduled (it waits in turn)
+  const Geom& g = p.g;
+  const int s = (int)blockIdx.x;
+  const int kb = s / g.mb, mbi = s - kb * g.mb;
+  const int nrows = min(g.bm, g.m - mbi * g.bm);
+  const int ncols = min(g.bk, g.k - kb * g.bk);
+  int vec_end = BF16 ? (ncols / (4 * p.simd_w)) * (4 * p.simd_w) : (ncols / p.simd_w) * p.simd_w;
+  if (p.simd_w <= 1) vec_end = 0;
+  const uint32_t c0 = (uint32_t)kb * (uint32_t)g.bk, c1 = c0 + (uint32_t)ncols;
+  const int tid = (int)threadIdx.x, lane = tid & 31;
+  const bool spw = BF16 && (0 != p.write_sp) && (0 != p.out.tcsp) && 0 == (g.k % 128) && p.simd_w > 1;
+  if (spw && 0 == tid) p.out.slice_ovf[s] = 0;     // counted below, after the first barrier
+
+  // ---- the row's candidate range --------------------------------------------------------------------------
+  uint32_t n = 0;
+  if (tid < nrows) {
+    const int gr = mbi * g.bm + tid;
+    const uint32_t lo = min(__ldg(a.row_ptr + gr), a.nnz);
+    const uint32_t hi = max(lo, min(__ldg(a.row_ptr + gr + 1), a.nnz));
+    const uint32_t b = k1c_lower_bound(a.col_idx, lo, hi, c0);
+    const uint32_t e = k1c_lower_bound(a.col_idx, b, (hi - b > (uint32_t)ncols) ? b + (uint32_t)ncols : hi, c1);
+    cbeg[tid] = b;
+    n = e - b;
+  }
+  kcnt[tid] = 0;
+  uint32_t ncand;
+  coff[tid] = k1c_scan(n, wtot, &ncand);
+  if (0 == tid) coff[K1C_THREADS] = ncand;
+  __syncthreads();
+
+  // ---- walk the candidates in output order ------------------------------------------------------------------
+  uint16_t* co = p.out.colidx + (size_t)s * g.bm * g.bk;
+  float* va = p.out.values + (size_t)s * g.bm * g.bk;
+  uint16_t* ri = p.out.tcoff + (size_t)s * g.bm * g.bk;
+  uint32_t* rk = p.out.tcpk + (size_t)s * g.bm * g.bk;
+  uint32_t* sp = p.out.tcsp + (size_t)s * g.bm * g.bk;
+  const bool aux = (0 != p.write_aux);
+  uint32_t base = 0;
+  for (uint32_t i0 = 0; i0 < ncand; i0 += K1C_THREADS) {      // block-uniform
+    const uint32_t i = i0 + (uint32_t)tid;
+    bool keep = false;
+    int r = 0;
+    uint32_t j = 0, k = 0, vb = 0;
+    if (i < ncand) {
+      int lo = 0, hi = nrows - 1;                  // last row whose first candidate is <= i (it owns i: empty rows are skipped)
+      while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (coff[mid] <= i) lo = mid; else hi = mid - 1; }
+      r = lo;
+      j = cbeg[r] + (i - coff[r]);
+      const uint32_t col = __ldg(a.col_idx + j);
+      vb = k1c_bits<BF16>(a.values, j);
+      k = col - c0;
+      keep = (col >= c0) && (col < c1) && k1_keep(__uint_as_float(vb), (int)k, vec_end);
+    }
+    uint32_t nkept;
+    const uint32_t q = base + k1c_scan(keep ? 1u : 0u, wtot, &nkept);
+    base += nkept;
+    // per-row kept counts: one shared-memory add per row and warp
+    const unsigned same = __match_any_sync(0xffffffffu, keep ? r : -1);
+    const unsigned kept_lanes = __ballot_sync(0xffffffffu, keep) & same;
+    if (keep && lane == __ffs((int)kept_lanes) - 1) atomicAdd(&kcnt[r], (uint32_t)__popc(kept_lanes));
+    if (keep) {
+      co[q] = (uint16_t)k;
+      va[q] = __uint_as_float(vb);
+      if (aux) { if (BF16) rk[q] = xb_tc16_pack(r, (int)k, vb); else ri[q] = xb_tc_pack(r, (int)k); }
+      if (BF16 && spw) {
+        // the kept-mask of the row's 16-k span holding k (K1x: one lane's 16 elements), from the entry's neighbours in the row
+        const uint32_t span = k & ~15u, rb = cbeg[r], re = cbeg[r] + (coff[r + 1] - coff[r]);
+        uint32_t ms = 1u << (k & 15u);
+        for (uint32_t t = j; t > rb; --t) {
+          const uint32_t cn = __ldg(a.col_idx + t - 1);
+          if (cn < c0 + span || cn >= c0 + span + 16u) break;
+          if (k1_keep(__uint_as_float(k1c_bits<BF16>(a.values, t - 1)), 0, vec_end)) ms |= 1u << ((cn - c0) & 15u);
+        }
+        for (uint32_t t = j + 1; t < re; ++t) {
+          const uint32_t cn = __ldg(a.col_idx + t);
+          if (cn < c0 + span || cn >= c0 + span + 16u) break;
+          if (k1_keep(__uint_as_float(k1c_bits<BF16>(a.values, t)), 0, vec_end)) ms |= 1u << ((cn - c0) & 15u);
+        }
+        const uint32_t e16 = k & 15u, hs = k >> 4, rowm = (uint32_t)r & 127u;
+        uint32_t meta16 = 0;
+#pragma unroll
+        for (int gi = 0; gi < 4; ++gi) meta16 |= xb_sp_nibble((ms >> (4 * gi)) & 15u) << (16 + 4 * gi);
+        const uint32_t gi = e16 >> 2, slot = xb_sp_slot((ms >> (4u * gi)) & 15u, e16 & 3u);
+        sp[q] = meta16 | ((slot & 2u) << 14) | xb_sp_pos(rowm, hs * 8u + 2u * gi + (slot & 1u));
+        if (slot & 2u) {     // third / fourth nonzero of its group of four: counted per slice, the first kSpOvfCap listed
+          const uint32_t idx = atomicAdd(p.out.slice_ovf + s, 1u);
+          if (idx < (uint32_t)kSpOvfCap) p.out.ovf_list[(size_t)s * kSpOvfCap + idx] = make_uint2((uint32_t)r | (k << 16), vb);
+        }
+      }
+    }
+  }
+
+  // ---- row pointers (u16 like the reference's counter), the slice's count, density feedback -------------------------
+  __syncthreads();
+  uint32_t total;
+  const uint32_t rp = k1c_scan(tid < nrows ? kcnt[tid] : 0u, wtot, &total);
+  uint16_t* ro = p.out.rowidx + (size_t)s * (g.bm + 1);
+  if (tid < nrows) ro[tid] = (uint16_t)rp;
+  if (0 == tid) {
+    ro[nrows] = (uint16_t)total;
+    p.out.slice_nnz[s] = total;
+    xb_publish_nnz(p, total);
+  }
+}
+
+// K1x's geometric condition: complete 128-column blocks inside the reference's vector loops
+bool slices_csr_get_sp_words(const SliceArgs& args)
+{
+  return args.is_bf16 && 0 == (args.g.k % 128) && args.simd_w > 1 && 0 != args.write_sp && 0 != args.out.tcsp;
+}
+
+void launch_slices_csr(const SliceArgs& args, const CsrArgs& csr, cudaStream_t stream)
+{
+  const int nslices = args.g.mb * args.g.kb;
+  if (nslices <= 0) return;
+  count_launch(1);
+  if (args.is_bf16) XB_CUDA(launch_pdl(spmdm_slice_csr_kernel<true>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csr));
+  else XB_CUDA(launch_pdl(spmdm_slice_csr_kernel<false>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csr));
+}
+
 // =================================================================================================
 // K2: sliced SpMM.
 // CTA = 16 warps x RPW rows of one row block (mb) x BN = 32*VEC columns.  Per k-block the
