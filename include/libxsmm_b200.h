@@ -30,6 +30,20 @@ LIBXSMM_API void libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(const libxs
   const unsigned int* d_row_ptr, const unsigned int* d_col_idx, const libxsmm_bfloat16* d_values, long long nnz,
   libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
 
+/* A (M x K, the handle's shape) in CSC form: col_ptr[K + 1], row_idx[nnz], values[nnz], all DEVICE pointers, 0-based, row
+ * indices strictly ascending within each column.  These are also the CSR arrays of A stored K x M (a kernel kept as
+ * in x out and multiplied with transpose_a).  Fills the handle's slices exactly as createSparseSlice_*_stream would with
+ * transa = 'T' for the K x M array holding these entries, and as the CSR entry would for A's CSR arrays; asynchronous on
+ * stream.  The compute entries then take the slices unchanged.  Errors (sticky, nothing launched): -90 NULL col_ptr, or NULL
+ * row_idx / values with nnz > 0; -91 nnz < 0 or nnz > 2^32 - 1.  Malformed arrays on the device give unspecified slices,
+ * never writes outside them. */
+LIBXSMM_API void libxsmm_spmdm_createSparseSlice_csc_fp32_stream(const libxsmm_spmdm_handle* handle,
+  const unsigned int* d_col_ptr, const unsigned int* d_row_idx, const float* d_values, long long nnz,
+  libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
+LIBXSMM_API void libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream(const libxsmm_spmdm_handle* handle,
+  const unsigned int* d_col_ptr, const unsigned int* d_row_idx, const libxsmm_bfloat16* d_values, long long nnz,
+  libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream);
+
 /* All block ids of reference samples/spmdm/spmdm.c:106-110 in one launch.  d_b, d_c are DEVICE pointers;
  * alpha and beta are HOST pointers read at call time (alpha is ignored like in the reference). */
 LIBXSMM_API void libxsmm_spmdm_compute_fp32_stream(const libxsmm_spmdm_handle* handle, char transa, char transb,

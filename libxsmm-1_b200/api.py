@@ -32,6 +32,7 @@ REFERENCE_SYMBOLS = [
 ADDED_SYMBOLS = [
     "libxsmm_spmdm_createSparseSlice_fp32_stream", "libxsmm_spmdm_createSparseSlice_bfloat16_stream",
     "libxsmm_spmdm_createSparseSlice_csr_fp32_stream", "libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream",
+    "libxsmm_spmdm_createSparseSlice_csc_fp32_stream", "libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream",
     "libxsmm_spmdm_compute_fp32_stream", "libxsmm_spmdm_compute_bfloat16_stream",
     "libxsmm_spmdm_exec_host", "libxsmm_spmdm_exec_stream",
     "libxsmm_dfsspmdm_execute_stream", "libxsmm_sfsspmdm_execute_stream",
@@ -110,9 +111,10 @@ def load():
         f = getattr(L, "libxsmm_spmdm_compute_%s_stream" % nm)
         f.argtypes = [H, cc, cc, vp, S, vp, cc, vp, vp, vp]
         f.restype = None
-        f = getattr(L, "libxsmm_spmdm_createSparseSlice_csr_%s_stream" % nm)
-        f.argtypes = [H, vp, vp, vp, ctypes.c_longlong, S, vp]
-        f.restype = None
+        for form in ("csr", "csc"):
+            f = getattr(L, "libxsmm_spmdm_createSparseSlice_%s_%s_stream" % (form, nm))
+            f.argtypes = [H, vp, vp, vp, ctypes.c_longlong, S, vp]
+            f.restype = None
     L.libxsmm_spmdm_exec_host.argtypes = [H, S, ci, cc, cc, cc, vp, vp, vp, vp]
     L.libxsmm_spmdm_exec_host.restype = None
     L.libxsmm_spmdm_exec_stream.argtypes = [H, S, ci, cc, cc, cc, vp, vp, vp, vp, vp]
@@ -409,6 +411,16 @@ def libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(handle, d_row_ptr, d_col
                                                                int(nnz), slices, _sptr(stream))
 
 
+def libxsmm_spmdm_createSparseSlice_csc_fp32_stream(handle, d_col_ptr, d_row_idx, d_values, nnz, slices, stream=None):
+    load().libxsmm_spmdm_createSparseSlice_csc_fp32_stream(ctypes.byref(handle), _addr(d_col_ptr), _addr(d_row_idx), _addr(d_values),
+                                                           int(nnz), slices, _sptr(stream))
+
+
+def libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream(handle, d_col_ptr, d_row_idx, d_values, nnz, slices, stream=None):
+    load().libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream(ctypes.byref(handle), _addr(d_col_ptr), _addr(d_row_idx), _addr(d_values),
+                                                               int(nnz), slices, _sptr(stream))
+
+
 def libxsmm_spmdm_compute_fp32_stream(handle, transa, transb, alpha, slices, d_b, transc, beta, d_c, stream=None):
     al = ctypes.c_float(alpha)
     be = ctypes.c_float(beta)
@@ -548,6 +560,12 @@ class Spmdm:
         (float32, or bf16 bit patterns as uint16); the same slices as create_slices() on the dense matrix (transa 'N')."""
         f = libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream if bf16 else libxsmm_spmdm_createSparseSlice_csr_fp32_stream
         f(self.handle, d_row_ptr, d_col_idx, d_values, nnz, self.slices, stream)
+
+    def create_slices_csc(self, d_col_ptr, d_row_idx, d_values, nnz, bf16=False, stream=None):
+        """A in CSC form (equally: the CSR arrays of A stored K x M): device arrays col_ptr[K + 1], row_idx[nnz] (uint32, 0-based,
+        ascending within a column) and values[nnz]; the same slices as create_slices() on the K x M array with transa 'T'."""
+        f = libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream if bf16 else libxsmm_spmdm_createSparseSlice_csc_fp32_stream
+        f(self.handle, d_col_ptr, d_row_idx, d_values, nnz, self.slices, stream)
 
     def compute(self, d_b, d_c, transb="N", transc="N", beta=0.0, bf16=False, stream=None, transa="N"):
         if bf16:

@@ -140,8 +140,8 @@ static bool stream_is_capturing(cudaStream_t stream)
   return cudaStreamCaptureStatusNone != st;
 }
 
-// dense_image = false: the slicing kernel cannot write the dense tile image (A in CSR form); an image left by an earlier pass is
-// then stale and marked so.
+// dense_image = false: the slicing kernel cannot write the dense tile image (A in CSR or CSC form); an image left by an earlier
+// pass is then stale and marked so.
 static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cudaStream_t stream, bool dense_image = true)
 {
   a->acc = c->d_acc; a->host_total = c->d_nnz; a->total_slices = c->g.mb * c->g.kb;
@@ -197,7 +197,7 @@ static void slice_policy(SpmdmCtx* c, SliceArgs* a, int is_bf16, bool whole, cud
     a->out.tcsp = c->arena.tcsp; a->out.ovf_list = c->arena.ovf_list;
     a->write_sp = c->arena.tcsp ? 1 : 0;
   }
-  c->sp_written = dense_image ? slices_get_sp_words(*a) : slices_csr_get_sp_words(*a);
+  c->sp_written = dense_image ? slices_get_sp_words(*a) : slices_sparse_get_sp_words(*a);
 }
 
 static int compute_policy(const SpmdmCtx* c, int is_bf16, bool transb, bool transc)
@@ -283,22 +283,47 @@ static void slices_whole(const libxsmm_spmdm_handle* handle, char transa, const 
   launch_slices(a, c->g.mb * c->g.kb, stream);
 }
 
+// A in CSR or CSC form (device arrays): the argument checks and the slicing policy of both routes.  Returns false, after setting
+// the error, when nothing may be launched.
+static bool sparse_slices_setup(const libxsmm_spmdm_handle* handle, bool csc, const unsigned int* d_ptr, const unsigned int* d_idx,
+                                const void* d_values, long long nnz, int is_bf16, cudaStream_t stream, SliceArgs* a)
+{
+  SpmdmCtx* c = find_ctx(handle);
+  if (0 == c) return false;
+  const char* form = csc ? "csc" : "csr";
+  if (0 == d_ptr) { set_error(-90, "createSparseSlice_%s: NULL %s", form, csc ? "col_ptr" : "row_ptr"); return false; }
+  if (nnz < 0 || nnz > 0xFFFFFFFFll) { set_error(-91, "createSparseSlice_%s: nnz=%lld outside [0, 2^32 - 1]", form, nnz); return false; }
+  if (nnz > 0 && (0 == d_idx || 0 == d_values)) {
+    set_error(-90, "createSparseSlice_%s: NULL %s or values with nnz=%lld", form, csc ? "row_idx" : "col_idx", nnz);
+    return false;
+  }
+  a->a = 0; a->transa = csc ? 1 : 0; a->lda = csc ? c->g.m : c->g.k; a->is_bf16 = is_bf16;
+  a->origin_is_block = 0; a->slice0 = 0; a->slice_step = 1; a->simd_w = c->simd_w; a->g = c->g; a->out = c->arena;
+  slice_policy(c, a, is_bf16, true, stream, false);
+  return true;
+}
+
 // A in CSR form (device arrays): the same slices as slices_whole() for the dense matrix holding these entries, transa = 'N'
 static void slices_csr(const libxsmm_spmdm_handle* handle, const unsigned int* d_row_ptr, const unsigned int* d_col_idx,
                        const void* d_values, long long nnz, int is_bf16, cudaStream_t stream)
 {
-  SpmdmCtx* c = find_ctx(handle);
-  if (0 == c) return;
-  if (0 == d_row_ptr) { set_error(-90, "createSparseSlice_csr: NULL row_ptr"); return; }
-  if (nnz < 0 || nnz > 0xFFFFFFFFll) { set_error(-91, "createSparseSlice_csr: nnz=%lld outside [0, 2^32 - 1]", nnz); return; }
-  if (nnz > 0 && (0 == d_col_idx || 0 == d_values)) { set_error(-90, "createSparseSlice_csr: NULL col_idx or values with nnz=%lld", nnz); return; }
   SliceArgs a;
-  a.a = 0; a.transa = 0; a.lda = c->g.k; a.is_bf16 = is_bf16;
-  a.origin_is_block = 0; a.slice0 = 0; a.slice_step = 1; a.simd_w = c->simd_w; a.g = c->g; a.out = c->arena;
-  slice_policy(c, &a, is_bf16, true, stream, false);
+  if (!sparse_slices_setup(handle, false, d_row_ptr, d_col_idx, d_values, nnz, is_bf16, stream, &a)) return;
   CsrArgs csr;
   csr.row_ptr = d_row_ptr; csr.col_idx = d_col_idx; csr.values = d_values; csr.nnz = (uint32_t)nnz;
   launch_slices_csr(a, csr, stream);
+}
+
+// A in CSC form (device arrays; equally the CSR arrays of A stored k x m): the same slices as slices_whole() with transa = 'T' for
+// the k x m array holding these entries, and as slices_csr() for A's CSR arrays
+static void slices_csc(const libxsmm_spmdm_handle* handle, const unsigned int* d_col_ptr, const unsigned int* d_row_idx,
+                       const void* d_values, long long nnz, int is_bf16, cudaStream_t stream)
+{
+  SliceArgs a;
+  if (!sparse_slices_setup(handle, true, d_col_ptr, d_row_idx, d_values, nnz, is_bf16, stream, &a)) return;
+  CscArgs csc;
+  csc.col_ptr = d_col_ptr; csc.row_idx = d_row_idx; csc.values = d_values; csc.nnz = (uint32_t)nnz;
+  launch_slices_csc(a, csc, stream);
 }
 
 static void compute_whole(const libxsmm_spmdm_handle* handle, char transb, char transc, float beta,
@@ -586,6 +611,21 @@ void libxsmm_spmdm_createSparseSlice_csr_bfloat16_stream(const libxsmm_spmdm_han
 {
   (void)libxsmm_output_csr_a;
   slices_csr(handle, d_row_ptr, d_col_idx, d_values, nnz, 1, (cudaStream_t)stream);
+}
+
+void libxsmm_spmdm_createSparseSlice_csc_fp32_stream(const libxsmm_spmdm_handle* handle, const unsigned int* d_col_ptr,
+  const unsigned int* d_row_idx, const float* d_values, long long nnz, libxsmm_CSR_sparseslice* libxsmm_output_csr_a, void* stream)
+{
+  (void)libxsmm_output_csr_a;
+  slices_csc(handle, d_col_ptr, d_row_idx, d_values, nnz, 0, (cudaStream_t)stream);
+}
+
+void libxsmm_spmdm_createSparseSlice_csc_bfloat16_stream(const libxsmm_spmdm_handle* handle, const unsigned int* d_col_ptr,
+  const unsigned int* d_row_idx, const libxsmm_bfloat16* d_values, long long nnz, libxsmm_CSR_sparseslice* libxsmm_output_csr_a,
+  void* stream)
+{
+  (void)libxsmm_output_csr_a;
+  slices_csc(handle, d_col_ptr, d_row_idx, d_values, nnz, 1, (cudaStream_t)stream);
 }
 
 void libxsmm_spmdm_compute_fp32_stream(const libxsmm_spmdm_handle* handle, char transa, char transb, const float* alpha,

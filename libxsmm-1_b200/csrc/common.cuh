@@ -234,7 +234,12 @@ void launch_slices(const SliceArgs& args, int nslices, cudaStream_t stream);
 // entries (transa = 'N'), except the dense tile image; args.write_sp is honoured only for bf16 with k % 128 == 0 and simd_w > 1.
 struct CsrArgs { const unsigned int* row_ptr; const unsigned int* col_idx; const void* values; uint32_t nnz; };
 void launch_slices_csr(const SliceArgs& args, const CsrArgs& csr, cudaStream_t stream);
-bool slices_csr_get_sp_words(const SliceArgs& args);                     // would launch_slices_csr() write tcsp for these arguments?
+// A in CSC form (device arrays, 0-based, rows ascending within a column): col_ptr[k + 1], row_idx[nnz], values[nnz].
+// launch_slices_csc writes what launch_slices_csr writes for the same A, and launch_slices for the k x m array holding these
+// entries with transa = 'T', except the dense tile image.
+struct CscArgs { const unsigned int* col_ptr; const unsigned int* row_idx; const void* values; uint32_t nnz; };
+void launch_slices_csc(const SliceArgs& args, const CscArgs& csc, cudaStream_t stream);
+bool slices_sparse_get_sp_words(const SliceArgs& args);                  // would launch_slices_csr() / _csc() write tcsp for these arguments?
 void launch_compute(const ComputeArgs& args, cudaStream_t stream);
 bool launch_compute_tma(const ComputeArgs& args, bool partial, cudaStream_t stream);
 bool launch_compute_sp(const ComputeArgs& args, cudaStream_t stream);    // K2s: order-preserving TMA-ring kernel (spmdm_compute_sp.cu)

@@ -831,8 +831,131 @@ __global__ void __launch_bounds__(K1C_THREADS, 2) spmdm_slice_csr_kernel(const S
   }
 }
 
-// K1x's geometric condition: complete 128-column blocks inside the reference's vector loops
-bool slices_csr_get_sp_words(const SliceArgs& args)
+// -------------------------------------------------------------------------------------------------
+// K1t: A given in CSC form (col_ptr[k + 1], row_idx[nnz]; also the CSR arrays of A stored k x m) -> the same slices as the dense
+// slicer writes for transa = 'T' on the k x m array holding these entries, and as K1c writes for the CSR arrays of A.  One CTA
+// of K1c's shape per slice.  A column lists its rows in ascending order, a slice lists each row's columns in ascending order; the
+// transpose goes through a shared bitmask of the slice's kept entries (bm x 128 bits) instead of a sort or scratch memory:
+//   1. thread t < ncols finds column c0 + t's entries in the slice's rows (two binary searches, at most nrows candidates); a
+//      block scan lays the columns' ranges end to end;
+//   2. the CTA walks the candidates 512 at a time, tests each and sets its bit in its row's mask (shared atomicOr);
+//   3. thread r scans the popcount of row r's mask into the row pointers;
+//   4. a second walk writes every kept entry (r, k) at rowstart[r] + the kept bits of row r below k.
+// Placement depends only on the mask: the output is deterministic, and for any input an entry's index is below its row's end,
+// at most bm * bk.  Malformed input (col_ptr not monotone or past nnz, rows unsorted, duplicated or >= M) gives unspecified
+// slices but stays inside the arrays: column ranges are clamped to [0, nnz] and to nrows candidates, a candidate is kept only if
+// its row lies in the slice, and the duplicates of an entry set one bit and write one slot.
+// -------------------------------------------------------------------------------------------------
+template <bool BF16>
+__global__ void __launch_bounds__(K1C_THREADS, 2) spmdm_slice_csc_kernel(const SliceArgs p, const CscArgs a)
+{
+  __shared__ __align__(16) uint32_t kmask[K1C_THREADS][4];   // kept columns of each row of the slice
+  __shared__ uint32_t rstart[K1C_THREADS];                   // first output of each row
+  __shared__ uint32_t cbeg[128];                             // first candidate of the column in row_idx
+  __shared__ uint32_t coff[128];                             // exclusive scan of the columns' candidate counts
+  __shared__ uint32_t wtot[K1C_WARPS];
+  pdl_wait();          // launch_pdl: the slices may still be read by the multiply in front of this kernel in the stream
+  pdl_trigger();       // ... and the multiply behind it may be scheduled (it waits in turn)
+  const Geom& g = p.g;
+  const int s = (int)blockIdx.x;
+  const int kb = s / g.mb, mbi = s - kb * g.mb;
+  const int nrows = min(g.bm, g.m - mbi * g.bm);
+  const int ncols = min(g.bk, g.k - kb * g.bk);
+  int vec_end = BF16 ? (ncols / (4 * p.simd_w)) * (4 * p.simd_w) : (ncols / p.simd_w) * p.simd_w;
+  if (p.simd_w <= 1) vec_end = 0;
+  const uint32_t c0 = (uint32_t)kb * (uint32_t)g.bk;
+  const uint32_t r0 = (uint32_t)mbi * (uint32_t)g.bm, r1 = r0 + (uint32_t)nrows;
+  const int tid = (int)threadIdx.x;
+  const bool spw = BF16 && (0 != p.write_sp) && (0 != p.out.tcsp) && 0 == (g.k % 128) && p.simd_w > 1;
+  if (spw && 0 == tid) p.out.slice_ovf[s] = 0;     // counted in step 4, after the first barrier
+
+  // ---- 1. the column's candidate range ------------------------------------------------------------------------
+  uint32_t n = 0;
+  if (tid < ncols) {
+    const uint32_t gc = c0 + (uint32_t)tid;
+    const uint32_t lo = min(__ldg(a.col_ptr + gc), a.nnz);
+    const uint32_t hi = max(lo, min(__ldg(a.col_ptr + gc + 1), a.nnz));
+    const uint32_t b = k1c_lower_bound(a.row_idx, lo, hi, r0);
+    const uint32_t e = k1c_lower_bound(a.row_idx, b, (hi - b > (uint32_t)nrows) ? b + (uint32_t)nrows : hi, r1);
+    cbeg[tid] = b;
+    n = e - b;
+  }
+  *(uint4*)kmask[tid] = make_uint4(0, 0, 0, 0);
+  uint32_t ncand;
+  const uint32_t off = k1c_scan(n, wtot, &ncand);
+  if (tid < ncols) coff[tid] = off;
+  __syncthreads();
+
+  // the candidate i < ncand: its column (the last one whose first candidate is <= i: empty columns are skipped), row and value
+  auto candidate = [&](uint32_t i, int* c, uint32_t* r, uint32_t* vb) {
+    int lo = 0, hi = ncols - 1;
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (coff[mid] <= i) lo = mid; else hi = mid - 1; }
+    const uint32_t j = cbeg[lo] + (i - coff[lo]);
+    *c = lo;
+    *r = __ldg(a.row_idx + j) - r0;              // rows outside the slice wrap to >= nrows
+    *vb = k1c_bits<BF16>(a.values, j);
+    return *r < (uint32_t)nrows && k1_keep(__uint_as_float(*vb), lo, vec_end);
+  };
+
+  // ---- 2. the kept-mask of every row -----------------------------------------------------------------------------
+  for (uint32_t i = (uint32_t)tid; i < ncand; i += K1C_THREADS) {
+    int c;
+    uint32_t r, vb;
+    if (candidate(i, &c, &r, &vb)) atomicOr(&kmask[r][c >> 5], 1u << (c & 31));
+  }
+  __syncthreads();
+
+  // ---- 3. row pointers (u16 like the reference's counter), the slice's count, density feedback -------------------------
+  uint32_t cnt = 0;
+  if (tid < nrows) { const uint4 m = *(const uint4*)kmask[tid]; cnt = __popc(m.x) + __popc(m.y) + __popc(m.z) + __popc(m.w); }
+  uint32_t total;
+  const uint32_t rp = k1c_scan(cnt, wtot, &total);
+  rstart[tid] = rp;
+  uint16_t* ro = p.out.rowidx + (size_t)s * (g.bm + 1);
+  if (tid < nrows) ro[tid] = (uint16_t)rp;
+  if (0 == tid) {
+    ro[nrows] = (uint16_t)total;
+    p.out.slice_nnz[s] = total;
+    xb_publish_nnz(p, total);
+  }
+  __syncthreads();
+
+  // ---- 4. place the kept entries -----------------------------------------------------------------------------------
+  uint16_t* co = p.out.colidx + (size_t)s * g.bm * g.bk;
+  float* va = p.out.values + (size_t)s * g.bm * g.bk;
+  uint16_t* ri = p.out.tcoff + (size_t)s * g.bm * g.bk;
+  uint32_t* rk = p.out.tcpk + (size_t)s * g.bm * g.bk;
+  uint32_t* sp = p.out.tcsp + (size_t)s * g.bm * g.bk;
+  const bool aux = (0 != p.write_aux);
+  for (uint32_t i = (uint32_t)tid; i < ncand; i += K1C_THREADS) {
+    int c;
+    uint32_t r, vb;
+    if (!candidate(i, &c, &r, &vb)) continue;
+    const uint4 m = *(const uint4*)kmask[r];
+    const uint32_t k = (uint32_t)c, w = k >> 5, mw = (w & 2) ? ((w & 1) ? m.w : m.z) : ((w & 1) ? m.y : m.x);
+    const uint32_t q = rstart[r] + __popc(mw & ((1u << (k & 31u)) - 1u))
+                     + (w > 0 ? __popc(m.x) : 0u) + (w > 1 ? __popc(m.y) : 0u) + (w > 2 ? __popc(m.z) : 0u);
+    co[q] = (uint16_t)k;
+    va[q] = __uint_as_float(vb);
+    if (aux) { if (BF16) rk[q] = xb_tc16_pack((int)r, (int)k, vb); else ri[q] = xb_tc_pack((int)r, (int)k); }
+    if (BF16 && spw) {
+      const uint32_t ms = (mw >> (k & 16u)) & 0xFFFFu;      // the kept-mask of the row's 16-k span holding k (K1x: one lane's 16 elements)
+      const uint32_t e16 = k & 15u, hs = k >> 4, rowm = r & 127u;
+      uint32_t meta16 = 0;
+#pragma unroll
+      for (int gi = 0; gi < 4; ++gi) meta16 |= xb_sp_nibble((ms >> (4 * gi)) & 15u) << (16 + 4 * gi);
+      const uint32_t gi = e16 >> 2, slot = xb_sp_slot((ms >> (4u * gi)) & 15u, e16 & 3u);
+      sp[q] = meta16 | ((slot & 2u) << 14) | xb_sp_pos(rowm, hs * 8u + 2u * gi + (slot & 1u));
+      if (slot & 2u) {     // third / fourth nonzero of its group of four: counted per slice, the first kSpOvfCap listed
+        const uint32_t idx = atomicAdd(p.out.slice_ovf + s, 1u);
+        if (idx < (uint32_t)kSpOvfCap) p.out.ovf_list[(size_t)s * kSpOvfCap + idx] = make_uint2(r | (k << 16), vb);
+      }
+    }
+  }
+}
+
+// K1c and K1t write tcsp under K1x's geometric condition: complete 128-column blocks inside the reference's vector loops
+bool slices_sparse_get_sp_words(const SliceArgs& args)
 {
   return args.is_bf16 && 0 == (args.g.k % 128) && args.simd_w > 1 && 0 != args.write_sp && 0 != args.out.tcsp;
 }
@@ -844,6 +967,15 @@ void launch_slices_csr(const SliceArgs& args, const CsrArgs& csr, cudaStream_t s
   count_launch(1);
   if (args.is_bf16) XB_CUDA(launch_pdl(spmdm_slice_csr_kernel<true>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csr));
   else XB_CUDA(launch_pdl(spmdm_slice_csr_kernel<false>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csr));
+}
+
+void launch_slices_csc(const SliceArgs& args, const CscArgs& csc, cudaStream_t stream)
+{
+  const int nslices = args.g.mb * args.g.kb;
+  if (nslices <= 0) return;
+  count_launch(1);
+  if (args.is_bf16) XB_CUDA(launch_pdl(spmdm_slice_csc_kernel<true>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csc));
+  else XB_CUDA(launch_pdl(spmdm_slice_csc_kernel<false>, dim3((unsigned)nslices), dim3(K1C_THREADS), 0, stream, args, csc));
 }
 
 // =================================================================================================
