@@ -445,6 +445,12 @@ __device__ __forceinline__ uint32_t k1w_mask8(uint4 w)
 
 // CW < 32: one CTA of CW warps walks the 32 / CW parts of its slice one after the other (the running total is the next part's
 // base), so that two 16-warp CTAs fit an SM and one's loads overlap the other's arithmetic.
+//
+// Sparse regime (at most 32 candidate lanes in a warp's rows, i.e. up to about 2 % density): a lane whose 16 elements are all
+// +-0 keeps nothing, and at 1 % density that is 85 % of the lanes.  One cheap test per lane (any half with a magnitude bit set)
+// and one ballot per iteration list the candidate lanes; in (iteration, lane) order they are exactly the output order.  The
+// candidates' 32 bytes are compacted through the warp's stage, lane t runs the exact keep test on candidate t, and a warp scan of
+// the counts gives every output index and every row pointer.  Denser warps take the per-lane path (warp-uniform branch).
 template <int ROWS, int CW>
 __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x_kernel(const SliceArgs p)
 {
@@ -454,8 +460,10 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
   constexpr int RPI = 32 / LPR;              // rows per iteration
   constexpr int ITS = (ROWS + RPI - 1) / RPI;
   __shared__ uint32_t wtot[CW];
-  constexpr int SCAP = 64;                   // records per warp: all 16 rows of a warp at once up to 3 % density
-  __shared__ uint2 stage[CW][SCAP];          // per warp: the records of its outputs (stage and spread, phase 2)
+  constexpr int SCAP = 64;                   // records per warp of the per-lane path: all 16 rows of a warp at once up to 3 % density
+  constexpr int CCAP = 128;                  // records per warp of the compacted path (the candidates' words take the same 1 KiB first)
+  __shared__ uint4 stage_mem[CW][2 * 32];    // per warp: 32 candidates x 32 bytes, then the records of its outputs (stage and spread)
+  __shared__ uint32_t csrc_mem[CW][32];      // per warp: where candidate t came from, as record bits: lane << 4 | iteration << 9
   // programmatic dependent launch (launch_slices): the slices this kernel overwrites may still be read by the multiply in front of
   // it in the stream -- wait for it before anything else; the multiply behind it may be scheduled from now on (it waits in turn)
   pdl_wait();
@@ -467,6 +475,8 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
   const int tid = (int)threadIdx.x, warp = tid >> 5, lane = tid & 31;
   const int qr = lane / LPR, hl = lane % LPR;       // row inside the group, segment of the row
   const int rpw = (g.bm + K1N_WARPS - 1) / K1N_WARPS;
+  const uint32_t lt = (1u << lane) - 1u;
+  uint2* stg = (uint2*)stage_mem[warp];
   uint32_t seq_base = 0;                     // kept elements of the parts already done
 #pragma unroll 1
   for (int pass = 0; pass < SEQ; ++pass) {
@@ -476,7 +486,6 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
 
   // ---- phase 1: load, test, count ---------------------------------------------------------------------
   uint4 w[ITS][NW];
-  uint32_t masks[ITS];
 #pragma unroll
   for (int it = 0; it < ITS; ++it) {
     const int r = row_lo + RPI * it + qr;
@@ -484,17 +493,70 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
 #pragma unroll
     for (int j = 0; j < NW; ++j) w[it][j] = (r < row_hi) ? __ldg(src + j) : make_uint4(0, 0, 0, 0);
   }
-  uint32_t mine = 0;
+  // candidate lanes: some half has a magnitude bit set.  The others hold only +-0, which the keep rule drops.
+  uint32_t cb[ITS], cb0[ITS], ncand = 0;
 #pragma unroll
   for (int it = 0; it < ITS; ++it) {
-    uint32_t m = 0;
+    uint32_t o = 0;
 #pragma unroll
-    for (int j = 0; j < NW; ++j) m |= k1w_mask8(w[it][j]) << (8 * j);
-    masks[it] = m;
-    mine += __popc(m);
+    for (int j = 0; j < NW; ++j) o |= w[it][j].x | w[it][j].y | w[it][j].z | w[it][j].w;
+    cb[it] = __ballot_sync(0xffffffffu, 0 != (o & 0x7FFF7FFFu));
+    cb0[it] = ncand;
+    ncand += __popc(cb[it]);
   }
+  const bool compact = ncand <= 32u;         // warp-uniform
+  uint32_t masks[ITS];
+  // compacted: lane t's candidate: its keep mask, origin, first output in the warp, and its words in w[0] (the two paths share
+  // the registers that stay live across the scan)
+  uint32_t cm = 0, csrc = 0, cex = 0;
+  uint4 (&cw)[NW] = w[0];
+  // ... and for the warp's row i = RPI * it + qr held by lane i: the index of its first candidate, or ncand when none follows
+  uint32_t rci = 0;
+  uint32_t mine = 0;
+  if (compact) {
+    const int itr = lane / RPI;
+    const uint32_t above = (1u << (LPR * (lane % RPI))) - 1u;      // the lanes of the rows above it in its group
 #pragma unroll
-  for (int d = 16; d > 0; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
+    for (int it = 0; it < ITS; ++it) rci += __popc(cb[it] & ((it < itr) ? 0xFFFFFFFFu : ((it == itr) ? above : 0u)));
+#pragma unroll
+    for (int it = 0; it < ITS; ++it) {
+      if ((cb[it] >> lane) & 1u) {
+        const uint32_t t = cb0[it] + __popc(cb[it] & lt);
+#pragma unroll
+        for (int j = 0; j < NW; ++j) stage_mem[warp][NW * t + j] = w[it][j];
+        csrc_mem[warp][t] = ((uint32_t)lane << 4) | ((uint32_t)it << 9);
+      }
+    }
+    __syncwarp();
+#pragma unroll
+    for (int j = 0; j < NW; ++j) cw[j] = make_uint4(0, 0, 0, 0);
+    if ((uint32_t)lane < ncand) {
+#pragma unroll
+      for (int j = 0; j < NW; ++j) { cw[j] = stage_mem[warp][NW * lane + j]; cm |= k1w_mask8(cw[j]) << (8 * j); }
+      csrc = csrc_mem[warp][lane];
+    }
+    const uint32_t cnt = __popc(cm);
+    uint32_t inc = cnt;
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const uint32_t u = __shfl_up_sync(0xffffffffu, inc, d);
+      if (lane >= d) inc += u;
+    }
+    cex = inc - cnt;                         // lanes past the candidates: the warp's total
+    mine = __shfl_sync(0xffffffffu, inc, 31);
+  }
+  else {
+#pragma unroll
+    for (int it = 0; it < ITS; ++it) {
+      uint32_t m = 0;
+#pragma unroll
+      for (int j = 0; j < NW; ++j) m |= k1w_mask8(w[it][j]) << (8 * j);
+      masks[it] = m;
+      mine += __popc(m);
+    }
+#pragma unroll
+    for (int d = 16; d > 0; d >>= 1) mine += __shfl_xor_sync(0xffffffffu, mine, d);
+  }
   const uint32_t warp_total = mine;
   if (0 == pass && 0 == tid && p.write_sp && p.out.tcsp) p.out.slice_ovf[s] = 0;   // counted below, after the scan's barrier
   const K1Scan sc = k1_scan<CW>(mine, wtot, seq_base);
@@ -511,16 +573,11 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
   uint16_t* co = p.out.colidx + (size_t)s * g.bm * g.bk;
   float* va = p.out.values + (size_t)s * g.bm * g.bk;
   uint32_t* rk = p.out.tcpk + (size_t)s * g.bm * g.bk;
-  const uint32_t lt = (1u << lane) - 1u;
-  uint2* stg = stage[warp];
-  const uint32_t before = (1u << (LPR * qr)) - 1u;             // the lanes of the rows above it in the group
   const bool aux = (0 != p.write_aux);
   // word per nonzero for the structured-sparse tensor-core kernel: a lane's 16 elements are exactly the four groups of four
   // whose nibbles make one 16-bit metadata word of the row, so everything is known to the lane (common.cuh: xb_sp_*)
   const bool spw = (0 != p.write_sp) && (0 != p.out.tcsp);
   uint32_t* sp = p.out.tcsp + (size_t)s * g.bm * g.bk;
-  uint32_t wdone = 0;                      // outputs of this warp's earlier iterations
-  const uint32_t pos0 = pos;               // first output of this warp
   auto spread = [&](const uint2 rec, const uint32_t q) {      // everything one output costs, by whichever lane gets it
     const uint32_t vb = rec.x & 0xFFFF0000u, ms = rec.x & 0xFFFFu, e16 = rec.y & 15u, sl = (rec.y >> 4) & 31u, its = rec.y >> 9;
     const uint32_t rs = (uint32_t)row_lo + (uint32_t)RPI * its + sl / LPR, hs = sl % LPR, rowm = rs & 127u, k = hs * 16u + e16;
@@ -539,6 +596,36 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
       }
     }
   };
+  if (compact) {
+    // row pointers: lane i takes the warp's row i, whose first output is that of its first candidate (or the warp's total when
+    // no candidate follows it)
+    const uint32_t off = __shfl_sync(0xffffffffu, cex, rci & 31u);
+    if (lane < ROWS && row_lo + lane < row_hi) ro[row_lo + lane] = (uint16_t)(pos + (rci < 32u ? off : warp_total));
+    // stage and spread: lane t drops its candidate's kept elements as 8-byte records {value | the lane's 16-bit mask,
+    // element | lane << 4 | iteration << 9} at their output index, then lane t does all the work for output t
+    for (uint32_t c0 = 0; c0 < warp_total; c0 += (uint32_t)CCAP) {      // one round below ~6 % density
+      if (cm) {
+        uint32_t i = cex - c0;                  // unsigned: outputs before this round wrap around
+        for (uint32_t mm = cm; mm; mm &= mm - 1u, ++i) {
+          if (i < (uint32_t)CCAP) {
+            const int e = __ffs((int)mm) - 1;
+            const uint4 v = (e & 8) ? cw[NW - 1] : cw[0];
+            const uint32_t pr = (e & 4) ? ((e & 2) ? v.w : v.z) : ((e & 2) ? v.y : v.x);
+            const uint32_t vb = (e & 1) ? (pr & 0xFFFF0000u) : (pr << 16);
+            stg[i] = make_uint2(vb | cm, (uint32_t)e | csrc);
+          }
+        }
+      }
+      __syncwarp();
+      const uint32_t nc = min((uint32_t)CCAP, warp_total - c0);
+      for (uint32_t t = (uint32_t)lane; t < nc; t += 32u) spread(stg[t], pos + c0 + t);
+      __syncwarp();                             // the stage is rewritten by the next round
+    }
+  }
+  else {
+  const uint32_t before = (1u << (LPR * qr)) - 1u;             // the lanes of the rows above it in the group
+  uint32_t wdone = 0;                      // outputs of this warp's earlier iterations
+  const uint32_t pos0 = pos;               // first output of this warp
 #pragma unroll
   for (int it = 0; it < ITS; ++it) {
     if (row_lo + RPI * it < row_hi) {      // warp-uniform
@@ -561,12 +648,9 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
       const uint32_t rowpos = pos + kept(before);
       const int r = row_lo + RPI * it + qr;
       if (0 == hl && r < row_hi) ro[r] = (uint16_t)rowpos;
-      // Stage and spread.  In the sparse regime a handful of the 32 lanes hold a nonzero or two, and everything a nonzero costs
-      // (four stores, the positions in the tensor-core tiles, the metadata word) would run once per loop trip of the fullest
-      // lane with one to three lanes active.  Instead every lane drops its kept elements as 8-byte records {value | its 16-bit
-      // mask, element | lane << 4 | iteration << 9} at their output index into the warp's shared-memory stage (a short
-      // divergent loop), and lane t then does all the work for output t.  When the warp's 16 rows hold at most SCAP nonzeros
-      // (always below 3 % density) all four iterations are staged first and spread in one pass after the loop.
+      // Stage and spread as in the compacted path, one iteration at a time, without the compaction.  When the warp's 16 rows
+      // hold at most SCAP nonzeros (always below 3 % density) all four iterations are staged first and spread in one pass after
+      // the loop.
       const uint32_t tot = kept(0xFFFFFFFFu);
       if (tot) {                                        // warp-uniform
         const uint32_t ex = kept(lt);                   // this lane's first output of the iteration (lane order = (row, column) order)
@@ -600,6 +684,7 @@ __global__ void __launch_bounds__(CW * 32, (32 == CW) ? 1 : 2) spmdm_slice_bf16x
     __syncwarp();
     for (uint32_t c0 = 0; c0 < warp_total; c0 += 32u)
       if (c0 + (uint32_t)lane < warp_total) spread(stg[c0 + lane], pos0 + c0 + (uint32_t)lane);
+  }
   }
   if (SEQ > 1) __syncthreads();             // wtot and the stages are reused by the next part
   }
