@@ -211,6 +211,28 @@ LIBXSMM_API void libxsmm_b200_rm_soa_execute(const libxsmm_b200_rm_soa* handle, 
   long long n_elements, long long stride_a, long long stride_b, long long stride_c, void* stream);
 LIBXSMM_API void libxsmm_b200_rm_soa_destroy(libxsmm_b200_rm_soa* handle);
 
+/* Indexed execution of the batched SoA entries: per-element slots, so that neighbour (flux) terms and element subsets need no
+ * gather copy.  Define slot_x(e) = d_x_index ? d_x_index[e] : e, and the same for every operand.  Element e (0 <= e < n_elements)
+ * computes exactly what the strided entry computes for one element whose operands sit at base + slot(e) * stride: the same chain
+ * of fused multiply-adds, the same bits.
+ *   - A NULL index is the identity.  A stride of 0 still shares that operand among all elements, with or without an index.
+ *   - An element whose index in some operand is at or past that operand's *_slots is skipped on the device: nothing of it is
+ *     read, its C slot is untouched.  Input indices may repeat.  If C indices repeat, the C of those slots is unspecified;
+ *     nothing is written outside slots 0 .. c_slots - 1 (0 .. n_elements - 1 without a C index).
+ *   - Index arrays are DEVICE arrays of n_elements entries, read at execute time on `stream` (a graph replay reads their
+ *     current contents).
+ *   - One call is one launch; n_elements = 0 does nothing.  Rejected on the host, before any CUDA call, with error -84 and
+ *     nothing launched: a NULL handle, a negative count or stride, a non-NULL index with *_slots < 1 or > 2^32, a NULL operand
+ *     (n_elements > 0), and C slots that overlap: stride_c below one element's C extent with a C index and c_slots > 1, or
+ *     without a C index and n_elements > 1. */
+LIBXSMM_API void libxsmm_b200_csr_soa_execute_indexed(const libxsmm_b200_csr_soa* handle, const void* d_X, void* d_C,
+  long long n_elements, long long stride_x, long long stride_c,
+  const unsigned int* d_x_index, long long x_slots, const unsigned int* d_c_index, long long c_slots, void* stream);
+LIBXSMM_API void libxsmm_b200_rm_soa_execute_indexed(const libxsmm_b200_rm_soa* handle, const void* d_a, const void* d_b, void* d_c,
+  long long n_elements, long long stride_a, long long stride_b, long long stride_c,
+  const unsigned int* d_a_index, long long a_slots, const unsigned int* d_b_index, long long b_slots,
+  const unsigned int* d_c_index, long long c_slots, void* stream);
+
 /* Dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3): the GPU counterpart of
  *     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, flags, prefetch)
  *     for (i = 0; i < N; i += nblock) kernel(B_panel + i, A_op, C_panel + i)

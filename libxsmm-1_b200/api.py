@@ -58,6 +58,7 @@ ADDED_SYMBOLS = [
     "libxsmm_b200_dmmdispatch", "libxsmm_b200_smmdispatch", "libxsmm_b200_mm_execute", "libxsmm_b200_mm_kernel", "libxsmm_b200_mm_release",
     "libxsmm_b200_drm_ac_soa_create", "libxsmm_b200_srm_ac_soa_create", "libxsmm_b200_drm_bc_soa_create", "libxsmm_b200_srm_bc_soa_create",
     "libxsmm_b200_rm_soa_execute", "libxsmm_b200_rm_soa_destroy",
+    "libxsmm_b200_csr_soa_execute_indexed", "libxsmm_b200_rm_soa_execute_indexed",
 ]
 
 
@@ -751,6 +752,14 @@ class CsrSoa:
         sc = self.M * self.ldc * self.soa if stride_c is None else stride_c
         L.libxsmm_b200_csr_soa_execute(self.handle, _addr(d_X), _addr(d_C), n_elements, sx, sc, _sptr(stream))
 
+    def execute_indexed(self, d_X, d_C, n_elements, x_index=None, x_slots=0, c_index=None, c_slots=0, stride_x=None, stride_c=None, stream=None):
+        """element e reads its dense operand at slot x_index[e] and writes its C at slot c_index[e] (DEVICE uint32 arrays; None:
+        slot e); an element with a slot at or past x_slots / c_slots is skipped.  Strides as for execute()."""
+        dense = self.K * self.ldb if self.sparse == "A" else self.M * self.lda
+        sx = dense * self.soa if stride_x is None else stride_x
+        sc = self.M * self.ldc * self.soa if stride_c is None else stride_c
+        csr_soa_execute_indexed(self.handle, d_X, d_C, n_elements, sx, sc, x_index, x_slots, c_index, c_slots, stream)
+
     def destroy(self):
         if self.handle:
             L = load()
@@ -792,6 +801,15 @@ class RmSoa:
         sc = self.M * self.ldc * self.soa if stride_c is None else stride_c
         rm_soa_execute(self.handle, d_a, d_b, d_c, n_elements, sa, sb, sc, stream)
 
+    def execute_indexed(self, d_a, d_b, d_c, n_elements, a_index=None, a_slots=0, b_index=None, b_slots=0, c_index=None, c_slots=0,
+                        stride_a=None, stride_b=None, stride_c=None, stream=None):
+        """element e reads a, b and writes C at slots a_index[e], b_index[e], c_index[e] (DEVICE uint32 arrays; None: slot e); an
+        element with a slot at or past that operand's *_slots is skipped.  Strides as for execute()."""
+        sa = self.M * self.lda * (self.soa if self.form == "ac" else 1) if stride_a is None else stride_a
+        sb = self.K * self.ldb * (self.soa if self.form == "bc" else 1) if stride_b is None else stride_b
+        sc = self.M * self.ldc * self.soa if stride_c is None else stride_c
+        rm_soa_execute_indexed(self.handle, d_a, d_b, d_c, n_elements, sa, sb, sc, a_index, a_slots, b_index, b_slots, c_index, c_slots, stream)
+
     def destroy(self):
         if self.handle:
             rm_soa_destroy(self.handle)
@@ -812,6 +830,26 @@ def rm_soa_execute(handle, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride
     L.libxsmm_b200_rm_soa_execute.restype = None
     L.libxsmm_b200_rm_soa_execute.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_longlong] * 4 + [ctypes.c_void_p]
     L.libxsmm_b200_rm_soa_execute(handle, _addr(d_a), _addr(d_b), _addr(d_c), n_elements, stride_a, stride_b, stride_c, _sptr(stream))
+
+
+def rm_soa_execute_indexed(handle, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, a_index, a_slots, b_index, b_slots,
+                           c_index, c_slots, stream=None):
+    """the raw indexed entry: every pointer may be a DeviceBuffer, an address or None (checked by the library, error -84)"""
+    L = load()
+    f = L.libxsmm_b200_rm_soa_execute_indexed
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p] * 4 + [ctypes.c_longlong] * 4 + [ctypes.c_void_p, ctypes.c_longlong] * 3 + [ctypes.c_void_p]
+    f(handle, _addr(d_a), _addr(d_b), _addr(d_c), n_elements, stride_a, stride_b, stride_c,
+      _addr(a_index), a_slots, _addr(b_index), b_slots, _addr(c_index), c_slots, _sptr(stream))
+
+
+def csr_soa_execute_indexed(handle, d_X, d_C, n_elements, stride_x, stride_c, x_index, x_slots, c_index, c_slots, stream=None):
+    """the raw indexed entry of a csr_soa handle (see rm_soa_execute_indexed)"""
+    L = load()
+    f = L.libxsmm_b200_csr_soa_execute_indexed
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p] * 3 + [ctypes.c_longlong] * 3 + [ctypes.c_void_p, ctypes.c_longlong] * 2 + [ctypes.c_void_p]
+    f(handle, _addr(d_X), _addr(d_C), n_elements, stride_x, stride_c, _addr(x_index), x_slots, _addr(c_index), c_slots, _sptr(stream))
 
 
 def rm_soa_destroy(handle):

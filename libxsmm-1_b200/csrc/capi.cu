@@ -958,7 +958,8 @@ void libxsmm_b200_csr_soa_execute(const libxsmm_b200_csr_soa* handle, const void
   long long stride_b, long long stride_c, void* stream)
 {
   if (0 == handle) { set_error(-63, "csr_soa_execute: NULL handle"); return; }
-  fs_execute_batched((const FsOperator*)handle, d_B, d_C, n_elements, stride_b, stride_c, (cudaStream_t)stream);
+  const ElemIndex none = {0, 0};
+  fs_execute_batched((const FsOperator*)handle, d_B, d_C, n_elements, stride_b, stride_c, none, none, (cudaStream_t)stream);
 }
 int libxsmm_b200_csr_soa_is_baked(const libxsmm_b200_csr_soa* handle) { return fs_is_baked((const FsOperator*)handle); }
 void libxsmm_b200_csr_soa_destroy(libxsmm_b200_csr_soa* handle) { fs_destroy((FsOperator*)handle); }
@@ -1003,9 +1004,67 @@ void libxsmm_b200_rm_soa_execute(const libxsmm_b200_rm_soa* handle, const void* 
     return;
   }
   if (0 == d_a || 0 == d_b || 0 == d_c) { set_error(-83, "rm_soa_execute: NULL operand"); return; }
-  rm_soa_execute(*h, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, (cudaStream_t)stream);
+  const ElemIndex none = {0, 0};
+  rm_soa_execute(*h, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, none, none, none, (cudaStream_t)stream);
 }
 void libxsmm_b200_rm_soa_destroy(libxsmm_b200_rm_soa* handle) { delete (RmSoa*)handle; }
+
+// ---- indexed execution of the batched SoA entries ------------------------------------------------------------------------------
+// Element e reads operand X at d_X + slot * stride_x with slot = d_x_index[e] (DEVICE array, read at execute time on the stream) or
+// e for a NULL index, and writes its C likewise.  An element whose slot in some operand is at or past that operand's slot count is
+// skipped on the device.  The host checks below run before any CUDA call; every rejection sets -84 and launches nothing.
+static bool soa_index_ok(const char* who, const char* name, const unsigned int* idx, long long slots)
+{
+  if (0 != idx && (slots < 1 || slots > (1ll << 32))) { set_error(-84, "%s: %s_slots=%lld outside [1, 2^32] for a non-NULL index", who, name, slots); return false; }
+  return true;
+}
+// C slots must not overlap: with a C index whenever more than one slot may be written, without one (slot = element) when more than
+// one element runs -- the strided entries' rule
+static bool soa_c_disjoint(const char* who, long long n_elements, long long stride_c, long long c_extent, const unsigned int* d_c_index, long long c_slots)
+{
+  if ((d_c_index ? c_slots > 1 : n_elements > 1) && stride_c < c_extent) {
+    set_error(-84, "%s: stride_c=%lld is smaller than one C slot (%lld scalars): slots would overlap", who, stride_c, c_extent);
+    return false;
+  }
+  return true;
+}
+void libxsmm_b200_csr_soa_execute_indexed(const libxsmm_b200_csr_soa* handle, const void* d_X, void* d_C, long long n_elements,
+  long long stride_x, long long stride_c, const unsigned int* d_x_index, long long x_slots, const unsigned int* d_c_index, long long c_slots, void* stream)
+{
+  static const char* const who = "csr_soa_execute_indexed";
+  const FsOperator* o = (const FsOperator*)handle;
+  if (0 == o) { set_error(-84, "%s: NULL handle", who); return; }
+  if (n_elements < 0 || stride_x < 0 || stride_c < 0) {
+    set_error(-84, "%s: negative count or stride (n_elements=%lld stride_x=%lld stride_c=%lld)", who, n_elements, stride_x, stride_c);
+    return;
+  }
+  if (!soa_index_ok(who, "x", d_x_index, x_slots) || !soa_index_ok(who, "c", d_c_index, c_slots)) return;
+  if (0 == n_elements) return;
+  if (0 == d_X || 0 == d_C) { set_error(-84, "%s: NULL operand", who); return; }
+  if (!soa_c_disjoint(who, n_elements, stride_c, fs_soa_c_extent(o), d_c_index, c_slots)) return;
+  const ElemIndex ix = {d_x_index, x_slots}, ic = {d_c_index, c_slots};
+  fs_execute_batched(o, d_X, d_C, n_elements, stride_x, stride_c, ix, ic, (cudaStream_t)stream);
+}
+void libxsmm_b200_rm_soa_execute_indexed(const libxsmm_b200_rm_soa* handle, const void* d_a, const void* d_b, void* d_c,
+  long long n_elements, long long stride_a, long long stride_b, long long stride_c,
+  const unsigned int* d_a_index, long long a_slots, const unsigned int* d_b_index, long long b_slots,
+  const unsigned int* d_c_index, long long c_slots, void* stream)
+{
+  static const char* const who = "rm_soa_execute_indexed";
+  const RmSoa* h = (const RmSoa*)handle;
+  if (0 == h) { set_error(-84, "%s: NULL handle", who); return; }
+  if (n_elements < 0 || stride_a < 0 || stride_b < 0 || stride_c < 0) {
+    set_error(-84, "%s: negative count or stride (n_elements=%lld stride_a=%lld stride_b=%lld stride_c=%lld)", who, n_elements, stride_a, stride_b, stride_c);
+    return;
+  }
+  if (!soa_index_ok(who, "a", d_a_index, a_slots) || !soa_index_ok(who, "b", d_b_index, b_slots) || !soa_index_ok(who, "c", d_c_index, c_slots)) return;
+  if (0 == n_elements) return;
+  if (0 == d_a || 0 == d_b || 0 == d_c) { set_error(-84, "%s: NULL operand", who); return; }
+  const long long c_extent = ((long long)(h->M - 1) * h->ldc + h->N) * h->soa;
+  if (!soa_c_disjoint(who, n_elements, stride_c, c_extent, d_c_index, c_slots)) return;
+  const ElemIndex ia = {d_a_index, a_slots}, ib = {d_b_index, b_slots}, ic = {d_c_index, c_slots};
+  rm_soa_execute(*h, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, ia, ib, ic, (cudaStream_t)stream);
+}
 
 // ---- dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3) ---------------------------
 // The reference's callers apply a DENSE fixed operator to a row-major panel with the column-major SMM kernel

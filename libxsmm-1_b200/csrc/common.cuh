@@ -259,13 +259,18 @@ FsOperator* fs_create_csr(int is_double, int M, int N, int K, int lda, int ldb, 
                           const unsigned int* rowptr, const unsigned int* colidx, const void* values);
 FsOperator* fs_create_csc(int is_double, int M, int N, int K, int lda, int ldc, int soa, double beta,
                           const unsigned int* colptr, const unsigned int* rowidx, const void* values);
-void fs_execute_batched(const FsOperator* o, const void* dB, void* dC, long long n_elem, long long stride_b, long long stride_c, cudaStream_t stream);
+// the slot of every element in one operand of the batched SoA entries: idx[e] (a DEVICE array) or, for idx = NULL, e itself;
+// an element with a slot at or past `slots` is skipped
+struct ElemIndex { const unsigned int* idx; long long slots; };
+void fs_execute_batched(const FsOperator* o, const void* dB, void* dC, long long n_elem, long long stride_b, long long stride_c,
+                        ElemIndex ib, ElemIndex ic, cudaStream_t stream);
 void fs_execute(const FsOperator* op, const void* dB, void* dC, long long ncols, long long ldb, long long ldc, cudaStream_t stream);
 int fs_is_sparse_branch(const FsOperator* o);
 int fs_is_baked(const FsOperator* o);
 int fs_is_tensor_core(const FsOperator* o);
 int fs_needs_c_input(const FsOperator* o);
 int fs_is_double(const FsOperator* o);
+long long fs_soa_c_extent(const FsOperator* o);   // scalars from the first to past the last C entry one element of a csr_soa handle writes
 void fs_shape(const FsOperator* o, int* M, int* N, int* K, int* ldb, int* ldc, int* beta_one);
 void fs_destroy(FsOperator* op);
 
@@ -273,6 +278,6 @@ void fs_destroy(FsOperator* op);
 // form 0: ac (A and C are [row][ld][soa], b is plain row-major), 1: bc (B and C are SoA, a is plain)
 struct RmSoa { int is_double, form, M, N, K, lda, ldb, ldc, soa, beta_one; };
 void rm_soa_execute(const RmSoa& h, const void* d_a, const void* d_b, void* d_c, long long n_elem, long long stride_a,
-                    long long stride_b, long long stride_c, cudaStream_t stream);
+                    long long stride_b, long long stride_c, ElemIndex ia, ElemIndex ib, ElemIndex ic, cudaStream_t stream);
 
 }  // namespace xb

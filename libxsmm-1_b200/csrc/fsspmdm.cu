@@ -77,6 +77,7 @@ struct FsDev {
   long long ldb, ldc;
   long long J, sb, sc;   // batched form (CSR x SoA): columns per item and element strides; J = 0: plain column panel
   long long ipe, ib, ic; // items per element and item strides
+  ElemIndex xb, xc;      // batched form: slots of B and C per element (fs_execute_batched)
   const int* rowptr;
   const int* col;
   const void* val;
@@ -91,7 +92,9 @@ __global__ void __launch_bounds__(256) fs_generic_kernel(const FsDev p, const T*
   long long nb = n, nc = n;
   if (p.J > 0) {   // (element, item, column) form: VEC == 1
     const long long item = n / p.J, j = n - item * p.J, e = item / p.ipe, i = item - e * p.ipe;
-    nb = e * p.sb + i * p.ib + j; nc = e * p.sc + i * p.ic + j;
+    const long long sb = p.xb.idx ? (long long)p.xb.idx[e] : e, sc = p.xc.idx ? (long long)p.xc.idx[e] : e;
+    if (sb >= p.xb.slots || sc >= p.xc.slots) return;
+    nb = sb * p.sb + i * p.ib + j; nc = sc * p.sc + i * p.ic + j;
   }
   const T* Bn = B + nb;
   for (int m = 0; m < p.M; ++m) {
@@ -286,6 +289,7 @@ void fs_execute(const FsOperator* o, const void* dB, void* dC, long long ncols, 
   d.M = o->M; d.beta_one = o->beta_one; d.skip_empty = o->sparse_branch;
   d.ldb = ldb; d.ldc = ldc; d.rowptr = o->d_rowptr; d.col = o->d_col; d.val = o->d_val;
   d.J = 0; d.sb = 0; d.sc = 0; d.ipe = 1; d.ib = 0; d.ic = 0;
+  d.xb.idx = 0; d.xb.slots = 0; d.xc.idx = 0; d.xc.slots = 0;
   const int threads = 256;
   if (o->is_double) {
     const bool v2 = (0 == (ldb & 1)) && (0 == (ldc & 1)) && (0 == (((uintptr_t)dB | (uintptr_t)dC) & 15));
@@ -436,16 +440,22 @@ FsOperator* fs_create_csc(int is_double, int M, int N, int K, int lda, int ldc, 
   return fs_finish_soa(o);
 }
 
-void fs_execute_batched(const FsOperator* o, const void* dB, void* dC, long long n_elem, long long stride_b, long long stride_c, cudaStream_t stream)
+// ib / ic: the slot of every element's B and C (no index: the element itself, never skipped)
+void fs_execute_batched(const FsOperator* o, const void* dB, void* dC, long long n_elem, long long stride_b, long long stride_c,
+                        ElemIndex ib, ElemIndex ic, cudaStream_t stream)
 {
   if (0 == o || n_elem <= 0 || o->M <= 0) return;   // B sparse without a single nonzero: the reference's kernel touches nothing
+  if (0 == ib.idx) ib.slots = n_elem;
+  if (0 == ic.idx) ic.slots = n_elem;
   count_launch(1);
-  if (o->jit && fs_jit_launch_batched(o->jit, dB, dC, n_elem, o->items, o->item_cols, o->ldb, o->ldc, stride_b, stride_c, o->item_b, o->item_c, stream)) { note_compute_kernel("fs_baked (batched)"); return; }
+  if (o->jit && fs_jit_launch_batched(o->jit, dB, dC, n_elem, o->items, o->item_cols, o->ldb, o->ldc, stride_b, stride_c, o->item_b, o->item_c,
+                                      ib.idx, ib.slots, ic.idx, ic.slots, stream)) { note_compute_kernel("fs_baked (batched)"); return; }
   note_compute_kernel("fs_generic_kernel (batched)");
   FsDev d;
   d.M = o->M; d.beta_one = o->beta_one; d.skip_empty = o->sparse_branch;
   d.ldb = o->ldb; d.ldc = o->ldc; d.rowptr = o->d_rowptr; d.col = o->d_col; d.val = o->d_val;
   d.J = o->item_cols; d.sb = stride_b; d.sc = stride_c; d.ipe = o->items; d.ib = o->item_b; d.ic = o->item_c;
+  d.xb = ib; d.xc = ic;
   const int threads = 256;
   const long long total = n_elem * o->items * o->item_cols, blocks = (total + threads - 1) / threads;
   if (o->is_double) fs_generic_kernel<double, 1><<<(unsigned)blocks, threads, 0, stream>>>(d, (const double*)dB, (double*)dC, total);
@@ -476,6 +486,11 @@ int fs_needs_c_input(const FsOperator* o)
   return 0;
 }
 int fs_is_double(const FsOperator* o) { return o ? o->is_double : 0; }
+long long fs_soa_c_extent(const FsOperator* o)
+{
+  if (o->M <= 0) return 0;     // B sparse without a nonzero: nothing is written
+  return (o->items - 1) * o->item_c + (long long)(o->M - 1) * o->ldc + o->item_cols;
+}
 void fs_plan_info(const FsOperator* o, long long* info)
 {
   info[0] = o->nnz; info[1] = o->n_unique; info[2] = o->sparse_branch; info[3] = o->x86_code_size; info[4] = o->N_chunksize;

@@ -177,7 +177,8 @@ static int fs_prefetch_groups()
 }
 
 // batched: the columns are (element, column-in-element) pairs -- thread n works on element n / J, column n % J, whose B / C
-// rows start at element * stride (the [element][row][column][soa] tensors of the CSR x SoA kernels, SURVEY.md section 8f-1)
+// rows start at slot * stride (the [element][row][column][soa] tensors of the CSR x SoA kernels, SURVEY.md section 8f-1); the
+// slot is the element itself, or its entry in a per-element index array (fs_jit_launch_batched)
 std::string emit_ptx(int is_double, int vec2, int M, int K, int beta_one, int skip_empty,
                      const int* rowptr, const int* col, const double* val, int batched = 0, int variant = 0)
 {
@@ -225,12 +226,13 @@ std::string emit_ptx(int is_double, int vec2, int M, int K, int beta_one, int sk
     for (size_t i = 0; i < ctab.size(); ++i) append(s, "%s0x%016llX", i ? ", " : "", ctab[i]);
     s += "};\n\n";
   }
-  if (batched) s += ".visible .entry fs_baked(.param .u64 pB, .param .u64 pC, .param .u64 pN, .param .u64 pLDB, .param .u64 pLDC, .param .u64 pJ, .param .u64 pSB, .param .u64 pSC, .param .u64 pIPE, .param .u64 pIB, .param .u64 pIC)\n";
+  if (batched) s += ".visible .entry fs_baked(.param .u64 pB, .param .u64 pC, .param .u64 pN, .param .u64 pLDB, .param .u64 pLDC, .param .u64 pJ, .param .u64 pSB, .param .u64 pSC, .param .u64 pIPE, .param .u64 pIB, .param .u64 pIC, .param .u64 pXI, .param .u64 pXS, .param .u64 pCI, .param .u64 pCS)\n";
   else s += ".visible .entry fs_baked(.param .u64 pB, .param .u64 pC, .param .u64 pN, .param .u64 pLDB, .param .u64 pLDC)\n";
   append(s, ".maxntid %d, 1, 1\n", kBlock);
   if (minctas >= 2) append(s, ".minnctapersm %d\n", minctas);
   s += "{\n";
   s += "  .reg .pred %p, %pf;\n  .reg .b32 %r<4>;\n  .reg .b64 %rd<28>;\n";
+  if (batched) s += "  .reg .b32 %ri;\n  .reg .b64 %rs<3>;\n";
   append(s, "  .reg .%s %%bx<%d>, %%by<%d>, %%cx<%d>, %%cy<%d>, %%ax, %%ay, %%ai<8>, %%aj<8>, %%kv;\n", ty, K, K, M, M);
   s += "  ld.param.u64 %rd0, [pB];\n  ld.param.u64 %rd1, [pC];\n  ld.param.u64 %rd2, [pN];\n  ld.param.u64 %rd3, [pLDB];\n  ld.param.u64 %rd4, [pLDC];\n";
   s += "  mov.u32 %r0, %ctaid.x;\n  mov.u32 %r1, %tid.x;\n";
@@ -242,8 +244,16 @@ std::string emit_ptx(int is_double, int vec2, int M, int K, int beta_one, int sk
     s += "  ld.param.u64 %rd20, [pIPE];\n  ld.param.u64 %rd21, [pIB];\n  ld.param.u64 %rd22, [pIC];\n";
     s += "  div.u64 %rd15, %rd5, %rd12;\n  mul.lo.s64 %rd16, %rd15, %rd12;\n  sub.s64 %rd16, %rd5, %rd16;\n";      // rd15 = item, rd16 = j
     s += "  div.u64 %rd23, %rd15, %rd20;\n  mul.lo.s64 %rd24, %rd23, %rd20;\n  sub.s64 %rd24, %rd15, %rd24;\n";    // rd23 = e, rd24 = i
-    s += "  mad.lo.s64 %rd17, %rd23, %rd13, %rd16;\n  mad.lo.s64 %rd17, %rd24, %rd21, %rd17;\n";
-    s += "  mad.lo.s64 %rd18, %rd23, %rd14, %rd16;\n  mad.lo.s64 %rd18, %rd24, %rd22, %rd18;\n";
+    // slots of B and C: e, or idx[e] where the index pointer is not NULL; a slot at or past its count ends the thread
+    const char* const pidx[2] = {"pXI", "pCI"};
+    const char* const pcnt[2] = {"pXS", "pCS"};
+    for (int t = 0; t < 2; ++t) {
+      append(s, "  mov.b64 %%rs%d, %%rd23;\n  ld.param.u64 %%rs2, [%s];\n  setp.eq.u64 %%p, %%rs2, 0;\n  @%%p bra SLOT%d;\n", t, pidx[t], t);
+      append(s, "  mad.lo.s64 %%rs2, %%rd23, 4, %%rs2;\n  ld.global.u32 %%ri, [%%rs2];\n  cvt.u64.u32 %%rs%d, %%ri;\n", t);
+      append(s, "  ld.param.u64 %%rs2, [%s];\n  setp.ge.u64 %%p, %%rs%d, %%rs2;\n  @%%p bra DONE;\nSLOT%d:\n", pcnt[t], t, t);
+    }
+    s += "  mad.lo.s64 %rd17, %rs0, %rd13, %rd16;\n  mad.lo.s64 %rd17, %rd24, %rd21, %rd17;\n";
+    s += "  mad.lo.s64 %rd18, %rs1, %rd14, %rd16;\n  mad.lo.s64 %rd18, %rd24, %rd22, %rd18;\n";
     append(s, "  mad.lo.s64 %%rd0, %%rd17, %d, %%rd0;\n  mad.lo.s64 %%rd1, %%rd18, %d, %%rd1;\n", esz, esz);
   }
   else
@@ -677,13 +687,14 @@ bool fs_jit_launch(const FsJit* j, const void* dB, void* dC, long long ncols, lo
 }
 
 bool fs_jit_launch_batched(const FsJit* j, const void* dB, void* dC, long long n_elem, long long items_per_elem, long long cols_per_item, long long ldb, long long ldc,
-                           long long stride_b, long long stride_c, long long item_b, long long item_c, cudaStream_t stream)
+                           long long stride_b, long long stride_c, long long item_b, long long item_c,
+                           const unsigned int* b_index, long long b_slots, const unsigned int* c_index, long long c_slots, cudaStream_t stream)
 {
   if (!j->batched) return false;
   long long total = n_elem * items_per_elem * cols_per_item;
   const long long blocks = (total + j->block - 1) / j->block;
   void* args[] = { (void*)&dB, (void*)&dC, (void*)&total, (void*)&ldb, (void*)&ldc, (void*)&cols_per_item, (void*)&stride_b, (void*)&stride_c,
-                   (void*)&items_per_elem, (void*)&item_b, (void*)&item_c };
+                   (void*)&items_per_elem, (void*)&item_b, (void*)&item_c, (void*)&b_index, (void*)&b_slots, (void*)&c_index, (void*)&c_slots };
   const cudaError_t e = cudaLaunchKernel((const void*)j->kern, dim3((unsigned)blocks, 1, 1), dim3((unsigned)j->block, 1, 1), args, 0, stream);
   if (cudaSuccess != e) { set_error((int)e, "csr_soa: baked kernel launch failed: %s", cudaGetErrorString(e)); (void)cudaGetLastError(); return false; }
   return true;
