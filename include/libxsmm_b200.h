@@ -233,6 +233,26 @@ LIBXSMM_API void libxsmm_b200_rm_soa_execute_indexed(const libxsmm_b200_rm_soa* 
   const unsigned int* d_a_index, long long a_slots, const unsigned int* d_b_index, long long b_slots,
   const unsigned int* d_c_index, long long c_slots, void* stream);
 
+/* A fixed 2:4-sparse bf16 operator (M x K, row-major, pitch lda; HOST or DEVICE pointer, read only during create).
+ * An element is kept iff it is an ordered nonzero (+-0 and NaN dropped, as the spmdm slicing kernels do).  Every aligned
+ * group of four along k (k = 4g .. 4g+3; the last group of a row may be partial) must keep at most two elements.
+ * create compresses A on the GPU into [M_pad][K_pad / 2] kept values plus the metadata image the sparse tensor-core
+ * instruction takes (M_pad, K_pad: multiples of 128, zero-padded), then synchronises once to read the 2:4 check.
+ * NULL + sticky error: -95 M < 1, K < 1, lda < K or NULL a (checked on the host, before any CUDA call);
+ *                      -96 A is not 2:4 (the message names the first offending row and group).
+ * execute: C = A . op(B) + beta . C, accumulated in fp32 on the tensor cores (same contract as the bf16 spmdm path).
+ *   transb 'N': B is K x N (d_b[k * ldb + n]);  'T': B is stored N x K (d_b[n * ldb + k]; y = x . W^T with x tokens x K)
+ *   transc 'N': C is M x N (d_c[m * ldc + n]);  'T': C is stored N x M (d_c[n * ldc + m])
+ *   beta = 0: C is not read.  Any other beta: C = fmaf(beta, C, acc).
+ *   One launch, asynchronous on stream, no allocation, no host synchronisation (graph-capturable); N = 0 does nothing.
+ *   -97 (nothing launched): NULL handle, a trans flag outside N/n/T/t, N < 0, ldb or ldc below its extent, NULL d_b / d_c
+ *   with N > 0, d_b not 16-byte aligned or ldb % 8 != 0 (B goes through TMA), a current device other than create's. */
+typedef struct libxsmm_b200_sp24 libxsmm_b200_sp24;
+LIBXSMM_API libxsmm_b200_sp24* libxsmm_b200_sp24_create_bfloat16(int M, int K, int lda, const libxsmm_bfloat16* a);
+LIBXSMM_API void libxsmm_b200_sp24_execute(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const libxsmm_bfloat16* d_b, int ldb, float beta, float* d_c, int ldc, void* stream);
+LIBXSMM_API void libxsmm_b200_sp24_destroy(libxsmm_b200_sp24* handle);
+
 /* Dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3): the GPU counterpart of
  *     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, flags, prefetch)
  *     for (i = 0; i < N; i += nblock) kernel(B_panel + i, A_op, C_panel + i)

@@ -59,6 +59,7 @@ ADDED_SYMBOLS = [
     "libxsmm_b200_drm_ac_soa_create", "libxsmm_b200_srm_ac_soa_create", "libxsmm_b200_drm_bc_soa_create", "libxsmm_b200_srm_bc_soa_create",
     "libxsmm_b200_rm_soa_execute", "libxsmm_b200_rm_soa_destroy",
     "libxsmm_b200_csr_soa_execute_indexed", "libxsmm_b200_rm_soa_execute_indexed",
+    "libxsmm_b200_sp24_create_bfloat16", "libxsmm_b200_sp24_execute", "libxsmm_b200_sp24_destroy",
 ]
 
 
@@ -857,6 +858,74 @@ def rm_soa_destroy(handle):
     L.libxsmm_b200_rm_soa_destroy.restype = None
     L.libxsmm_b200_rm_soa_destroy.argtypes = [ctypes.c_void_p]
     L.libxsmm_b200_rm_soa_destroy(handle)
+
+
+class Sp24:
+    """A fixed 2:4-sparse bf16 operator (libxsmm_b200_sp24_*): every aligned group of four along k keeps at most two ordered
+    nonzeros.  a: M x K bf16 -- a torch bfloat16 tensor (host or CUDA, rows with unit stride) or a numpy uint16 array of bf16
+    bit patterns; lda defaults to a's row stride.  Create compresses A on the GPU once; a matrix that is not 2:4 raises ValueError
+    naming the first offending row and group."""
+
+    def __init__(self, a, lda=None):
+        if hasattr(a, "data_ptr"):
+            assert a.dim() == 2 and a.element_size() == 2 and a.stride(1) == 1
+            self.M, self.K = int(a.shape[0]), int(a.shape[1])
+            self.lda = int(a.stride(0)) if lda is None else lda
+            ptr = a.data_ptr()
+        else:
+            assert isinstance(a, np.ndarray) and a.dtype == np.uint16 and a.ndim == 2 and a.strides[1] == 2
+            self.M, self.K = a.shape
+            self.lda = a.strides[0] // 2 if lda is None else lda
+            ptr = a.ctypes.data
+        self.handle = sp24_create_bfloat16(self.M, self.K, self.lda, ptr)
+        if not self.handle:
+            code, msg = last_error()
+            clear_error()
+            raise ValueError("sp24_create_bfloat16 failed (%d): %s" % (code, msg))
+
+    def execute(self, d_b, d_c, N, ldb=None, ldc=None, beta=0.0, transb="N", transc="N", stream=None):
+        """C = A . op(B) + beta C (fp32 C).  d_b, d_c: DEVICE memory (DeviceBuffer, torch CUDA tensor or address).  transb 'N': B is
+        K x N, 'T': B is stored N x K; transc 'N': C is M x N, 'T': C is stored N x M.  Pitches default to the dense extents."""
+        tb, tc = transb in ("T", "t"), transc in ("T", "t")
+        ldb = (self.K if tb else N) if ldb is None else ldb
+        ldc = (self.M if tc else N) if ldc is None else ldc
+        sp24_execute(self.handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream)
+
+    def destroy(self):
+        if self.handle:
+            sp24_destroy(self.handle)
+            self.handle = None
+
+
+def _dptr(x):
+    return x.data_ptr() if hasattr(x, "data_ptr") else _addr(x)
+
+
+def sp24_create_bfloat16(M, K, lda, a):
+    """the raw create entry: a is an address (host or device) or None; the handle or None"""
+    L = load()
+    f = L.libxsmm_b200_sp24_create_bfloat16
+    f.restype = ctypes.c_void_p
+    f.argtypes = [ctypes.c_int] * 3 + [ctypes.c_void_p]
+    return f(M, K, lda, _dptr(a))
+
+
+def sp24_execute(handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream=None):
+    """the raw execute entry (arguments checked by the library, error -97)"""
+    L = load()
+    f = L.libxsmm_b200_sp24_execute
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p, ctypes.c_char, ctypes.c_char, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_float,
+                  ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
+    s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
+    f(handle, _c(transb), _c(transc), N, _dptr(d_b), ldb, float(beta), _dptr(d_c), ldc, s)
+
+
+def sp24_destroy(handle):
+    L = load()
+    L.libxsmm_b200_sp24_destroy.restype = None
+    L.libxsmm_b200_sp24_destroy.argtypes = [ctypes.c_void_p]
+    L.libxsmm_b200_sp24_destroy(handle)
 
 
 # ---- host-only planning (works without a GPU) ----------------------------------------------------------

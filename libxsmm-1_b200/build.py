@@ -14,7 +14,7 @@ ROOT = os.path.dirname(HERE)
 CSRC = os.path.join(HERE, "csrc")
 LIBDIR = os.path.join(HERE, "lib")
 LIB = os.path.join(LIBDIR, "libxsmm_b200.so")
-SOURCES = ["capi.cu", "spmdm_kernels.cu", "spmdm_compute_tma.cu", "spmdm_compute_sp.cu", "spmdm_compute_tc.cu", "spmdm_compute_tcq.cu", "spmdm_compute_tc16p.cu", "spmdm_compute_tc16s.cu", "fsspmdm.cu", "fsspmdm_tc.cu", "fsspmdm_jit.cpp", "rm_soa.cu"]
+SOURCES = ["capi.cu", "spmdm_kernels.cu", "spmdm_compute_tma.cu", "spmdm_compute_sp.cu", "spmdm_compute_tc.cu", "spmdm_compute_tcq.cu", "spmdm_compute_tc16p.cu", "spmdm_compute_tc16s.cu", "fsspmdm.cu", "fsspmdm_tc.cu", "fsspmdm_jit.cpp", "rm_soa.cu", "sp24.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 FLAGS = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC,-fvisibility=hidden", "-I", os.path.join(ROOT, "include")]

@@ -104,6 +104,15 @@ __host__ __device__ __forceinline__ uint32_t xb_sp_slot(uint32_t gm, uint32_t p)
   if (0 == (gm & (gm - 1u))) return p & 1u;
   return rank >= 2u ? 3u : rank;
 }
+// Metadata image of a compressed tile (2 KiB, the operand of tcgen05.cp.128x128b: tensor-memory lane L at byte 16 L): byte
+// offset of the 16-bit metadata word of (row, 16-k span), from the position xb_sp_pos of any kept element of that span.
+// Lane = row % 8 + 8 * (span % 2) + 16 * (row / 16), column = span / 2, upper half word for rows 8..15 of 16.
+__host__ __device__ __forceinline__ uint32_t xb_sp_meta_off(uint32_t pos)
+{
+  const uint32_t r7 = (pos >> 6) & 7u, span = ((pos >> 3) & 7u) ^ r7;
+  const uint32_t tl = r7 + ((span & 1u) << 3) + ((pos >> 10) << 4);
+  return tl * 16u + (span >> 1) * 4u + ((pos >> 8) & 2u);
+}
 #endif
 
 constexpr int kSpOvfCap = 256;        // overflow entries listed per slice (SliceArena::ovf_list); a slice with more is walked by its row pointers instead
@@ -273,6 +282,15 @@ int fs_is_double(const FsOperator* o);
 long long fs_soa_c_extent(const FsOperator* o);   // scalars from the first to past the last C entry one element of a csr_soa handle writes
 void fs_shape(const FsOperator* o, int* M, int* N, int* K, int* ldb, int* ldc, int* beta_one);
 void fs_destroy(FsOperator* op);
+
+// ---- fixed 2:4-sparse bf16 operators (sp24.cu); arguments checked by capi.cu ---------------------------------------------
+struct Sp24Op;
+Sp24Op* sp24_create(int M, int K, int lda, const uint16_t* a, bool a_on_device);
+void sp24_execute(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, float beta, float* d_c, int ldc, cudaStream_t stream);
+int sp24_device(const Sp24Op* op);
+int sp24_rows(const Sp24Op* op);
+int sp24_cols(const Sp24Op* op);
+void sp24_destroy(Sp24Op* op);
 
 // ---- dense SoA kernels (rm_soa.cu) ----------------------------------------------------------
 // form 0: ac (A and C are [row][ld][soa], b is plain row-major), 1: bc (B and C are SoA, a is plain)

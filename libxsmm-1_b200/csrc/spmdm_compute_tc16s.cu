@@ -74,15 +74,6 @@ constexpr float kSpMaxDensity = 0.022f;         // measured crossover with K4p o
 
 struct SpTile { int mbi, ml0, rows, n0; };
 
-__device__ __forceinline__ void tc_mma_bf16_sp_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t tmem_e, uint32_t idesc, uint32_t accumulate)
-{
-  asm volatile(
-    "{\n\t.reg .pred p;\n\t"
-    "setp.ne.b32 p, %5, 0;\n\t"
-    "tcgen05.mma.sp.cta_group::2.kind::f16 [%0], %1, %2, [%3], %4, p;\n\t}\n"
-    ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accumulate) : "memory");
-}
-
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(S_THREADS, 1)
 spmdm_compute_tc16s_kernel(const __grid_constant__ CUtensorMap tmB, const __grid_constant__ CUtensorMap tmC, const int c_tma, const ComputeArgs p)
 {
@@ -217,13 +208,8 @@ spmdm_compute_tc16s_kernel(const __grid_constant__ CUtensorMap tmB, const __grid
     const int wt = (tid - 64) % S_GT;
     const size_t cap = (size_t)g.bm * g.bk;
     const uint32_t lead_ready0 = map_to_cta(&a_ready[0], 0);
-    // byte offset of the 16-bit metadata word of (row, 16-k span) inside the image, from the position of a kept element:
-    // tensor-memory lane = row % 8 + 8 * (span % 2) + 16 * (row / 16), column = span / 2, upper half word for rows 8..15 of 16
-    auto meta_off = [](uint32_t pos) -> uint32_t {
-      const uint32_t r7 = (pos >> 6) & 7u, span = ((pos >> 3) & 7u) ^ r7;
-      const uint32_t tl = r7 + ((span & 1u) << 3) + ((pos >> 10) << 4);
-      return tl * 16u + (span >> 1) * 4u + ((pos >> 8) & 2u);
-    };
+    // byte offset of the metadata word of (row, 16-k span) in the image (a lambda: calling the helper directly changes the SASS)
+    auto meta_off = [](uint32_t pos) -> uint32_t { return xb_sp_meta_off(pos); };
     int c_wi = 0, c_kb = grp, c_rows = 0, c_sidx = 0;
     const uint16_t* c_ro = p.sl.rowidx;
     auto seat = [&]() {

@@ -136,6 +136,16 @@ __device__ __forceinline__ void tc_commit_pair(uint64_t* bar)
                ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
 }
 
+// 2:4 structured-sparse A (compressed, common.cuh: xb_sp_*); tmem_e: the tensor-memory column holding the metadata
+__device__ __forceinline__ void tc_mma_bf16_sp_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t tmem_e, uint32_t idesc, uint32_t accumulate)
+{
+  asm volatile(
+    "{\n\t.reg .pred p;\n\t"
+    "setp.ne.b32 p, %5, 0;\n\t"
+    "tcgen05.mma.sp.cta_group::2.kind::f16 [%0], %1, %2, [%3], %4, p;\n\t}\n"
+    ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accumulate) : "memory");
+}
+
 __device__ __forceinline__ void tc_mma_tf32_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
 {
   asm volatile(
