@@ -251,7 +251,23 @@ typedef struct libxsmm_b200_sp24 libxsmm_b200_sp24;
 LIBXSMM_API libxsmm_b200_sp24* libxsmm_b200_sp24_create_bfloat16(int M, int K, int lda, const libxsmm_bfloat16* a);
 LIBXSMM_API void libxsmm_b200_sp24_execute(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
   const libxsmm_bfloat16* d_b, int ldb, float beta, float* d_c, int ldc, void* stream);
-LIBXSMM_API void libxsmm_b200_sp24_destroy(libxsmm_b200_sp24* handle);
+LIBXSMM_API void libxsmm_b200_sp24_destroy(libxsmm_b200_sp24* handle);   /* either kind; NULL does nothing */
+
+/* A fixed 2:4-sparse FP8 operator: A is M x K bytes, row-major, pitch lda, HOST or DEVICE pointer, in one format:
+ *   format 0 = e4m3 (OCP E4M3, "fn": no Inf, NaN = 0x7F / 0xFF), 1 = e5m2.
+ * Same keep rule as the bf16 operator: ordered nonzeros, so +-0 and NaN are dropped and e5m2 +-Inf is kept; a group of four
+ * keeping three or four elements is -96 (first row and group named), and a group of two values and two NaN is legal.
+ * The multiply runs on the 8-bit structured-sparse tensor-core instruction (twice the rate of the bf16 one).
+ * NULL + sticky error: -95 M < 1, K < 1, lda < K, NULL a or a format other than 0 / 1 (on the host, before any CUDA call).
+ * execute_fp8: C = alpha . (A . op(B)) + beta . C with fp32 C and fp32 accumulation, per element fmaf(beta, C, alpha * acc);
+ *   beta = 0: C is not read.  alpha carries the per-tensor scales (scale_a * scale_b).  b_format (0 / 1) may differ from A's.
+ *   transb / transc, launch behaviour and N = 0 as for execute.
+ *   -97 (nothing launched): NULL handle or a bf16 handle (and execute rejects an FP8 handle), a trans flag outside N/n/T/t,
+ *   b_format not 0 / 1, N < 0, ldb or ldc below its extent, NULL d_b / d_c with N > 0, d_b not 16-byte aligned or
+ *   ldb % 16 != 0 (B goes through TMA), a current device other than create's. */
+LIBXSMM_API libxsmm_b200_sp24* libxsmm_b200_sp24_create_fp8(int M, int K, int lda, const unsigned char* a, int format);
+LIBXSMM_API void libxsmm_b200_sp24_execute_fp8(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const unsigned char* d_b, int b_format, int ldb, float alpha, float beta, float* d_c, int ldc, void* stream);
 
 /* Dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3): the GPU counterpart of
  *     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, flags, prefetch)

@@ -60,6 +60,7 @@ ADDED_SYMBOLS = [
     "libxsmm_b200_rm_soa_execute", "libxsmm_b200_rm_soa_destroy",
     "libxsmm_b200_csr_soa_execute_indexed", "libxsmm_b200_rm_soa_execute_indexed",
     "libxsmm_b200_sp24_create_bfloat16", "libxsmm_b200_sp24_execute", "libxsmm_b200_sp24_destroy",
+    "libxsmm_b200_sp24_create_fp8", "libxsmm_b200_sp24_execute_fp8",
 ]
 
 
@@ -860,36 +861,71 @@ def rm_soa_destroy(handle):
     L.libxsmm_b200_rm_soa_destroy(handle)
 
 
-class Sp24:
-    """A fixed 2:4-sparse bf16 operator (libxsmm_b200_sp24_*): every aligned group of four along k keeps at most two ordered
-    nonzeros.  a: M x K bf16 -- a torch bfloat16 tensor (host or CUDA, rows with unit stride) or a numpy uint16 array of bf16
-    bit patterns; lda defaults to a's row stride.  Create compresses A on the GPU once; a matrix that is not 2:4 raises ValueError
-    naming the first offending row and group."""
+FP8_FORMATS = {"e4m3": 0, "e5m2": 1}
 
-    def __init__(self, a, lda=None):
+
+def _fp8_format(x, fmt):
+    """the library's format code (0 e4m3, 1 e5m2) of a torch float8 tensor, or of raw bytes given with fmt"""
+    name = str(getattr(x, "dtype", ""))
+    if name in ("torch.float8_e4m3fn", "torch.float8_e5m2"):
+        code = 0 if name == "torch.float8_e4m3fn" else 1
+        if fmt is not None and FP8_FORMATS.get(fmt) != code:
+            raise ValueError("fmt=%r does not match the tensor's %s" % (fmt, name))
+        return code
+    if fmt not in FP8_FORMATS:
+        raise ValueError("raw FP8 bytes need fmt='e4m3' or 'e5m2', got %r" % (fmt,))
+    return FP8_FORMATS[fmt]
+
+
+class Sp24:
+    """A fixed 2:4-sparse operator (libxsmm_b200_sp24_*): every aligned group of four along k keeps at most two ordered
+    nonzeros.  a: M x K, rows with unit stride, host or CUDA --
+      bf16: a torch bfloat16 tensor or a numpy uint16 array of bf16 bit patterns;
+      FP8:  a torch float8_e4m3fn / float8_e5m2 tensor, or a numpy uint8 array of FP8 bytes with fmt="e4m3" | "e5m2".
+    lda defaults to a's row stride.  Create compresses A on the GPU once; a matrix that is not 2:4 raises ValueError naming
+    the first offending row and group."""
+    fp8, format = False, None       # FP8 operators set both in __init__
+
+    def __init__(self, a, lda=None, fmt=None):
         if hasattr(a, "data_ptr"):
-            assert a.dim() == 2 and a.element_size() == 2 and a.stride(1) == 1
+            assert a.dim() == 2 and a.stride(1) == 1
+            esize = a.element_size()
             self.M, self.K = int(a.shape[0]), int(a.shape[1])
             self.lda = int(a.stride(0)) if lda is None else lda
             ptr = a.data_ptr()
         else:
-            assert isinstance(a, np.ndarray) and a.dtype == np.uint16 and a.ndim == 2 and a.strides[1] == 2
+            assert isinstance(a, np.ndarray) and a.dtype in (np.uint16, np.uint8) and a.ndim == 2 and a.strides[1] == a.itemsize
+            esize = a.itemsize
             self.M, self.K = a.shape
-            self.lda = a.strides[0] // 2 if lda is None else lda
+            self.lda = a.strides[0] // esize if lda is None else lda
             ptr = a.ctypes.data
-        self.handle = sp24_create_bfloat16(self.M, self.K, self.lda, ptr)
+        self.fp8 = esize == 1
+        assert esize in (1, 2)
+        if self.fp8:
+            self.format = _fp8_format(a, fmt)
+            self.handle = sp24_create_fp8(self.M, self.K, self.lda, ptr, self.format)
+        else:
+            assert fmt is None, "fmt names an FP8 format; a holds bf16"
+            self.format = None
+            self.handle = sp24_create_bfloat16(self.M, self.K, self.lda, ptr)
         if not self.handle:
             code, msg = last_error()
             clear_error()
-            raise ValueError("sp24_create_bfloat16 failed (%d): %s" % (code, msg))
+            raise ValueError("%s failed (%d): %s" % ("sp24_create_fp8" if self.fp8 else "sp24_create_bfloat16", code, msg))
 
-    def execute(self, d_b, d_c, N, ldb=None, ldc=None, beta=0.0, transb="N", transc="N", stream=None):
-        """C = A . op(B) + beta C (fp32 C).  d_b, d_c: DEVICE memory (DeviceBuffer, torch CUDA tensor or address).  transb 'N': B is
-        K x N, 'T': B is stored N x K; transc 'N': C is M x N, 'T': C is stored N x M.  Pitches default to the dense extents."""
+    def execute(self, d_b, d_c, N, ldb=None, ldc=None, beta=0.0, transb="N", transc="N", stream=None, alpha=1.0, b_fmt=None):
+        """C = alpha . (A . op(B)) + beta C (fp32 C; alpha only for FP8 operators, where it carries the per-tensor scales).
+        d_b, d_c: DEVICE memory (DeviceBuffer, torch CUDA tensor or address).  For an FP8 operator B is a torch float8 tensor,
+        or device bytes with b_fmt="e4m3" | "e5m2".  transb 'N': B is K x N, 'T': B is stored N x K; transc 'N': C is M x N,
+        'T': C is stored N x M.  Pitches default to the dense extents."""
         tb, tc = transb in ("T", "t"), transc in ("T", "t")
         ldb = (self.K if tb else N) if ldb is None else ldb
         ldc = (self.M if tc else N) if ldc is None else ldc
-        sp24_execute(self.handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream)
+        if self.fp8:
+            sp24_execute_fp8(self.handle, transb, transc, N, d_b, _fp8_format(d_b, b_fmt), ldb, alpha, beta, d_c, ldc, stream)
+        else:
+            assert alpha == 1.0 and b_fmt is None, "alpha and b_fmt belong to FP8 operators"
+            sp24_execute(self.handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream)
 
     def destroy(self):
         if self.handle:
@@ -919,6 +955,26 @@ def sp24_execute(handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream=Non
                   ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
     s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
     f(handle, _c(transb), _c(transc), N, _dptr(d_b), ldb, float(beta), _dptr(d_c), ldc, s)
+
+
+def sp24_create_fp8(M, K, lda, a, fmt):
+    """the raw FP8 create entry: a is an address (host or device) or None, fmt 0 (e4m3) / 1 (e5m2); the handle or None"""
+    L = load()
+    f = L.libxsmm_b200_sp24_create_fp8
+    f.restype = ctypes.c_void_p
+    f.argtypes = [ctypes.c_int] * 3 + [ctypes.c_void_p, ctypes.c_int]
+    return f(M, K, lda, _dptr(a), fmt)
+
+
+def sp24_execute_fp8(handle, transb, transc, N, d_b, b_fmt, ldb, alpha, beta, d_c, ldc, stream=None):
+    """the raw FP8 execute entry (arguments checked by the library, error -97); b_fmt 0 (e4m3) / 1 (e5m2)"""
+    L = load()
+    f = L.libxsmm_b200_sp24_execute_fp8
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p, ctypes.c_char, ctypes.c_char, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                  ctypes.c_float, ctypes.c_float, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
+    s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
+    f(handle, _c(transb), _c(transc), N, _dptr(d_b), b_fmt, ldb, float(alpha), float(beta), _dptr(d_c), ldc, s)
 
 
 def sp24_destroy(handle):

@@ -1066,7 +1066,7 @@ void libxsmm_b200_rm_soa_execute_indexed(const libxsmm_b200_rm_soa* handle, cons
   rm_soa_execute(*h, d_a, d_b, d_c, n_elements, stride_a, stride_b, stride_c, ia, ib, ic, (cudaStream_t)stream);
 }
 
-// ---- fixed 2:4-sparse bf16 operators (sp24.cu) ---------------------------------------------------------------------------------
+// ---- fixed 2:4-sparse bf16 and FP8 operators (sp24.cu) --------------------------------------------------------------------
 // The shape checks run on the host before any CUDA call (-95); create then compresses A on the device and reports a group
 // keeping more than two elements (-96).  Every execute rejection (-97) also comes before anything is enqueued.
 struct libxsmm_b200_sp24;
@@ -1076,35 +1076,63 @@ libxsmm_b200_sp24* libxsmm_b200_sp24_create_bfloat16(int M, int K, int lda, cons
     set_error(-95, "sp24_create_bfloat16: M=%d, K=%d, lda=%d, a=%p: M and K must be at least 1, lda at least K, a not NULL", M, K, lda, (const void*)a);
     return 0;
   }
-  return (libxsmm_b200_sp24*)sp24_create(M, K, lda, (const uint16_t*)a, is_device_ptr(a));
+  return (libxsmm_b200_sp24*)sp24_create(M, K, lda, a, is_device_ptr(a), -1);
+}
+libxsmm_b200_sp24* libxsmm_b200_sp24_create_fp8(int M, int K, int lda, const unsigned char* a, int format)
+{
+  if (M < 1 || K < 1 || lda < K || 0 == a || (0 != format && 1 != format)) {
+    set_error(-95, "sp24_create_fp8: M=%d, K=%d, lda=%d, a=%p, format=%d: M and K must be at least 1, lda at least K, a not NULL, format 0 (e4m3) or 1 (e5m2)",
+              M, K, lda, (const void*)a, format);
+    return 0;
+  }
+  return (libxsmm_b200_sp24*)sp24_create(M, K, lda, a, is_device_ptr(a), format);
+}
+// the execute checks both kinds share (b_format is checked for FP8 calls only).  true: the call has work to enqueue
+static bool sp24_execute_ok(const char* who, const Sp24Op* op, bool fp8, char transb, char transc, int N, const void* d_b, int b_format,
+                            int ldb, const float* d_c, int ldc)
+{
+  if (0 == op) { set_error(-97, "%s: NULL handle", who); return false; }
+  if (fp8 != (sp24_format(op) >= 0)) {
+    set_error(-97, "%s: the handle holds a %s operator (created by sp24_create_%s)", who, fp8 ? "bf16" : "FP8", fp8 ? "bfloat16" : "fp8");
+    return false;
+  }
+  const bool tb = is_t(transb), tc = is_t(transc);
+  if (!(tb || 'N' == transb || 'n' == transb) || !(tc || 'N' == transc || 'n' == transc)) {
+    set_error(-97, "%s: transb='%c', transc='%c': each must be one of N, n, T, t", who, transb, transc);
+    return false;
+  }
+  if (fp8 && 0 != b_format && 1 != b_format) { set_error(-97, "%s: b_format=%d must be 0 (e4m3) or 1 (e5m2)", who, b_format); return false; }
+  if (N < 0) { set_error(-97, "%s: N=%d is negative", who, N); return false; }
+  const int M = sp24_rows(op), K = sp24_cols(op);
+  if (ldb < (tb ? K : N) || ldc < (tc ? M : N)) {
+    set_error(-97, "%s: ldb=%d must be at least %d (%s) and ldc=%d at least %d (%s)", who, ldb, tb ? K : N, tb ? "K" : "N", ldc, tc ? M : N, tc ? "M" : "N");
+    return false;
+  }
+  if (0 == N) return false;
+  if (0 == d_b || 0 == d_c) { set_error(-97, "%s: NULL d_b or d_c with N=%d", who, N); return false; }
+  const int ldb_unit = fp8 ? 16 : 8;     // elements in 16 bytes
+  if (0 != ((uintptr_t)d_b & 15) || 0 != (ldb % ldb_unit)) {
+    set_error(-97, "%s: d_b=%p must be 16-byte aligned and ldb=%d a multiple of %d (B is read through TMA)", who, d_b, ldb, ldb_unit);
+    return false;
+  }
+  int dev = -1;
+  if (cudaSuccess != cudaGetDevice(&dev)) { (void)cudaGetLastError(); dev = -1; }
+  if (dev != sp24_device(op)) { set_error(-97, "%s: current device %d, the operator was created on device %d", who, dev, sp24_device(op)); return false; }
+  return true;
 }
 void libxsmm_b200_sp24_execute(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
   const libxsmm_bfloat16* d_b, int ldb, float beta, float* d_c, int ldc, void* stream)
 {
-  static const char* const who = "sp24_execute";
   const Sp24Op* op = (const Sp24Op*)handle;
-  if (0 == op) { set_error(-97, "%s: NULL handle", who); return; }
-  const bool tb = is_t(transb), tc = is_t(transc);
-  if (!(tb || 'N' == transb || 'n' == transb) || !(tc || 'N' == transc || 'n' == transc)) {
-    set_error(-97, "%s: transb='%c', transc='%c': each must be one of N, n, T, t", who, transb, transc);
-    return;
-  }
-  if (N < 0) { set_error(-97, "%s: N=%d is negative", who, N); return; }
-  const int M = sp24_rows(op), K = sp24_cols(op);
-  if (ldb < (tb ? K : N) || ldc < (tc ? M : N)) {
-    set_error(-97, "%s: ldb=%d must be at least %d (%s) and ldc=%d at least %d (%s)", who, ldb, tb ? K : N, tb ? "K" : "N", ldc, tc ? M : N, tc ? "M" : "N");
-    return;
-  }
-  if (0 == N) return;
-  if (0 == d_b || 0 == d_c) { set_error(-97, "%s: NULL d_b or d_c with N=%d", who, N); return; }
-  if (0 != ((uintptr_t)d_b & 15) || 0 != (ldb & 7)) {
-    set_error(-97, "%s: d_b=%p must be 16-byte aligned and ldb=%d a multiple of 8 (B is read through TMA)", who, (const void*)d_b, ldb);
-    return;
-  }
-  int dev = -1;
-  if (cudaSuccess != cudaGetDevice(&dev)) { (void)cudaGetLastError(); dev = -1; }
-  if (dev != sp24_device(op)) { set_error(-97, "%s: current device %d, the operator was created on device %d", who, dev, sp24_device(op)); return; }
-  sp24_execute(op, tb, tc, N, (const uint16_t*)d_b, ldb, beta, d_c, ldc, (cudaStream_t)stream);
+  if (!sp24_execute_ok("sp24_execute", op, false, transb, transc, N, d_b, -2, ldb, d_c, ldc)) return;
+  sp24_execute(op, is_t(transb), is_t(transc), N, (const uint16_t*)d_b, ldb, beta, d_c, ldc, (cudaStream_t)stream);
+}
+void libxsmm_b200_sp24_execute_fp8(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const unsigned char* d_b, int b_format, int ldb, float alpha, float beta, float* d_c, int ldc, void* stream)
+{
+  const Sp24Op* op = (const Sp24Op*)handle;
+  if (!sp24_execute_ok("sp24_execute_fp8", op, true, transb, transc, N, d_b, b_format, ldb, d_c, ldc)) return;
+  sp24_execute_fp8(op, is_t(transb), is_t(transc), N, d_b, b_format, ldb, alpha, beta, d_c, ldc, (cudaStream_t)stream);
 }
 void libxsmm_b200_sp24_destroy(libxsmm_b200_sp24* handle) { sp24_destroy((Sp24Op*)handle); }
 

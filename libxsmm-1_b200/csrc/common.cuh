@@ -283,10 +283,13 @@ long long fs_soa_c_extent(const FsOperator* o);   // scalars from the first to p
 void fs_shape(const FsOperator* o, int* M, int* N, int* K, int* ldb, int* ldc, int* beta_one);
 void fs_destroy(FsOperator* op);
 
-// ---- fixed 2:4-sparse bf16 operators (sp24.cu); arguments checked by capi.cu ---------------------------------------------
+// ---- fixed 2:4-sparse bf16 and FP8 operators (sp24.cu); arguments checked by capi.cu ---------------------------------------------
 struct Sp24Op;
-Sp24Op* sp24_create(int M, int K, int lda, const uint16_t* a, bool a_on_device);
+Sp24Op* sp24_create(int M, int K, int lda, const void* a, bool a_on_device, int format);     // format: -1 bf16, 0 e4m3, 1 e5m2
 void sp24_execute(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, float beta, float* d_c, int ldc, cudaStream_t stream);
+void sp24_execute_fp8(const Sp24Op* op, bool transb, bool transc, int N, const unsigned char* d_b, int b_format, int ldb, float alpha, float beta,
+                      float* d_c, int ldc, cudaStream_t stream);
+int sp24_format(const Sp24Op* op);
 int sp24_device(const Sp24Op* op);
 int sp24_rows(const Sp24Op* op);
 int sp24_cols(const Sp24Op* op);

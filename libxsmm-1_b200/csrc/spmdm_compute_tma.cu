@@ -336,6 +336,24 @@ bool make_tensor_map_2d_sw128(CUtensorMap* map, const void* base, int elem_bytes
   return CUDA_SUCCESS == r;
 }
 
+// one-byte elements (FP8 operands), boxes of box_cols = swizzle_bytes (64 or 128) columns
+bool make_tensor_map_2d_u8(CUtensorMap* map, const void* base, unsigned long long cols, unsigned long long rows,
+                           unsigned long long row_pitch_bytes, unsigned box_cols, unsigned box_rows, int swizzle_bytes)
+{
+  EncodeTiledFn fn = encode_tiled();
+  if (0 == fn) return false;
+  if (0 != ((uintptr_t)base & 15) || 0 != (row_pitch_bytes & 15) || (int)box_cols != swizzle_bytes || box_rows > 256 ||
+      (64 != swizzle_bytes && 128 != swizzle_bytes)) return false;
+  const cuuint64_t gdim[2] = { cols, rows };
+  const cuuint64_t gstr[1] = { row_pitch_bytes };
+  const cuuint32_t box[2] = { box_cols, box_rows };
+  const cuuint32_t estr[2] = { 1, 1 };
+  const CUresult r = fn(map, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<void*>(base), gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+                        128 == swizzle_bytes ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
+                        CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+  return CUDA_SUCCESS == r;
+}
+
 template <bool BF16, int VEC, int R, int CW, int STAGES, bool PARTIAL>
 static bool launch_tma_variant(const ComputeArgs& a, cudaStream_t stream)
 {

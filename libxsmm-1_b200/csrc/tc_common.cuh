@@ -145,6 +145,16 @@ __device__ __forceinline__ void tc_mma_bf16_sp_pair(uint32_t tmem_d, uint64_t ad
     "tcgen05.mma.sp.cta_group::2.kind::f16 [%0], %1, %2, [%3], %4, p;\n\t}\n"
     ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accumulate) : "memory");
 }
+// the same with 8-bit A and B (e4m3 / e5m2, named by the instruction descriptor): K = 64 per instruction, the metadata of
+// row r in tensor-memory lane r, two columns per instruction (tools/umma_probe/probe_sp8.cu)
+__device__ __forceinline__ void tc_mma_f8_sp_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t tmem_e, uint32_t idesc, uint32_t accumulate)
+{
+  asm volatile(
+    "{\n\t.reg .pred p;\n\t"
+    "setp.ne.b32 p, %5, 0;\n\t"
+    "tcgen05.mma.sp.cta_group::2.kind::f8f6f4 [%0], %1, %2, [%3], %4, p;\n\t}\n"
+    ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(tmem_e), "r"(idesc), "r"(accumulate) : "memory");
+}
 
 __device__ __forceinline__ void tc_mma_tf32_pair(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate)
 {
