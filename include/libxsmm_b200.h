@@ -269,6 +269,25 @@ LIBXSMM_API libxsmm_b200_sp24* libxsmm_b200_sp24_create_fp8(int M, int K, int ld
 LIBXSMM_API void libxsmm_b200_sp24_execute_fp8(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
   const unsigned char* d_b, int b_format, int ldb, float alpha, float beta, float* d_c, int ldc, void* stream);
 
+/* bf16 C with an optional per-row bias, for either kind of 2:4 operator: y = x . W^T + b of a pruned linear layer in one call.
+ * acc is the fp32 accumulator the fp32-output entries produce for (m, n).  Per element of C:
+ *   1. v = acc for a bf16 operator; v = alpha * acc (one fp32 multiply, as in execute_fp8) for an FP8 operator.
+ *   2. If d_bias is not NULL, v = v + (float)d_bias[m], one fp32 addition.  If d_bias is NULL, no addition is made at all
+ *      (adding +0 would turn a -0 into +0; C stays bit-identical to rounding the fp32 entry's output).
+ *   3. If beta != 0, v = fmaf(beta, (float)C[m][n], v), where C is the old bf16 value.  If beta == 0, C is not read.
+ *   4. C[m][n] = bf16_round_to_nearest_even(v).  NaN stays NaN (the payload is not part of the contract); overflow gives +-Inf.
+ * d_bias is a DEVICE array of M bf16 values, indexed by A's row, read at execute time on stream (a graph replay reads its
+ * current contents).  transb, transc, pitches (in bf16 elements for C), N = 0 and launch behaviour as for execute.
+ * -97 (nothing launched): every case of execute / execute_fp8 (the bf16 entry rejects an FP8 handle and the FP8 entry a bf16
+ * handle), and d_c or d_bias not 2-byte aligned. */
+/* bf16 operator (sp24_create_bfloat16), bf16 C */
+LIBXSMM_API void libxsmm_b200_sp24_execute_bf16out(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const libxsmm_bfloat16* d_b, int ldb, const libxsmm_bfloat16* d_bias, float beta, libxsmm_bfloat16* d_c, int ldc, void* stream);
+/* FP8 operator (sp24_create_fp8), bf16 C */
+LIBXSMM_API void libxsmm_b200_sp24_execute_fp8_bf16out(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const unsigned char* d_b, int b_format, int ldb, float alpha, const libxsmm_bfloat16* d_bias, float beta,
+  libxsmm_bfloat16* d_c, int ldc, void* stream);
+
 /* Dense SMM dispatch for row-major operators with very many columns (SURVEY.md section 8f-3): the GPU counterpart of
  *     kernel = libxsmm_dmmdispatch(nblock, M_op, K_op, &ldb_panel, &lda_op, &ldc_panel, alpha, beta, flags, prefetch)
  *     for (i = 0; i < N; i += nblock) kernel(B_panel + i, A_op, C_panel + i)

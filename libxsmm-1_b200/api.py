@@ -61,6 +61,7 @@ ADDED_SYMBOLS = [
     "libxsmm_b200_csr_soa_execute_indexed", "libxsmm_b200_rm_soa_execute_indexed",
     "libxsmm_b200_sp24_create_bfloat16", "libxsmm_b200_sp24_execute", "libxsmm_b200_sp24_destroy",
     "libxsmm_b200_sp24_create_fp8", "libxsmm_b200_sp24_execute_fp8",
+    "libxsmm_b200_sp24_execute_bf16out", "libxsmm_b200_sp24_execute_fp8_bf16out",
 ]
 
 
@@ -877,6 +878,26 @@ def _fp8_format(x, fmt):
     return FP8_FORMATS[fmt]
 
 
+def _c_is_bf16(d_c, c_dtype):
+    """True for bf16 C: a torch bfloat16 d_c, or c_dtype="bf16" for other buffers (default fp32)"""
+    if c_dtype not in (None, "bf16", "fp32"):
+        raise ValueError("c_dtype must be 'bf16' or 'fp32', got %r" % (c_dtype,))
+    name = str(getattr(d_c, "dtype", ""))
+    if name in ("torch.bfloat16", "torch.float32"):
+        tensor_bf16 = name == "torch.bfloat16"
+        if c_dtype is not None and (c_dtype == "bf16") != tensor_bf16:
+            raise ValueError("c_dtype=%r does not match d_c's %s" % (c_dtype, name))
+        return tensor_bf16
+    return c_dtype == "bf16"
+
+
+def _check_bias(bias, M):
+    """a torch bias must hold M bf16 values; device buffers and addresses are the caller's responsibility"""
+    if hasattr(bias, "dtype") and hasattr(bias, "numel"):
+        if str(bias.dtype) != "torch.bfloat16" or bias.numel() != M or not bias.is_contiguous():
+            raise ValueError("bias must be a contiguous bfloat16 tensor of M=%d elements, got %s of %d" % (M, bias.dtype, bias.numel()))
+
+
 class Sp24:
     """A fixed 2:4-sparse operator (libxsmm_b200_sp24_*): every aligned group of four along k keeps at most two ordered
     nonzeros.  a: M x K, rows with unit stride, host or CUDA --
@@ -913,19 +934,79 @@ class Sp24:
             clear_error()
             raise ValueError("%s failed (%d): %s" % ("sp24_create_fp8" if self.fp8 else "sp24_create_bfloat16", code, msg))
 
-    def execute(self, d_b, d_c, N, ldb=None, ldc=None, beta=0.0, transb="N", transc="N", stream=None, alpha=1.0, b_fmt=None):
-        """C = alpha . (A . op(B)) + beta C (fp32 C; alpha only for FP8 operators, where it carries the per-tensor scales).
+    def execute(self, d_b, d_c, N, ldb=None, ldc=None, beta=0.0, transb="N", transc="N", stream=None, alpha=1.0, b_fmt=None,
+                bias=None, c_dtype=None):
+        """C = alpha . (A . op(B)) + beta C (alpha only for FP8 operators, where it carries the per-tensor scales).
         d_b, d_c: DEVICE memory (DeviceBuffer, torch CUDA tensor or address).  For an FP8 operator B is a torch float8 tensor,
         or device bytes with b_fmt="e4m3" | "e5m2".  transb 'N': B is K x N, 'T': B is stored N x K; transc 'N': C is M x N,
-        'T': C is stored N x M.  Pitches default to the dense extents."""
+        'T': C is stored N x M.  Pitches default to the dense extents (in elements of C).
+        C is fp32 unless d_c is a torch bfloat16 tensor or c_dtype="bf16": then C is bf16 and bias (NULL or a DEVICE array
+        of M bf16 values) is added per row before beta C, as include/libxsmm_b200.h states.  A bias with fp32 C is refused."""
         tb, tc = transb in ("T", "t"), transc in ("T", "t")
         ldb = (self.K if tb else N) if ldb is None else ldb
         ldc = (self.M if tc else N) if ldc is None else ldc
+        bf16_c = _c_is_bf16(d_c, c_dtype)
+        if bias is not None and not bf16_c:
+            raise ValueError("a bias needs bf16 C (a torch bfloat16 d_c or c_dtype='bf16'): the fp32-output entries have no bias")
+        if bias is not None:
+            _check_bias(bias, self.M)
         if self.fp8:
-            sp24_execute_fp8(self.handle, transb, transc, N, d_b, _fp8_format(d_b, b_fmt), ldb, alpha, beta, d_c, ldc, stream)
+            b_code = _fp8_format(d_b, b_fmt)
+            if bf16_c:
+                sp24_execute_fp8_bf16out(self.handle, transb, transc, N, d_b, b_code, ldb, alpha, bias, beta, d_c, ldc, stream)
+            else:
+                sp24_execute_fp8(self.handle, transb, transc, N, d_b, b_code, ldb, alpha, beta, d_c, ldc, stream)
         else:
             assert alpha == 1.0 and b_fmt is None, "alpha and b_fmt belong to FP8 operators"
-            sp24_execute(self.handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream)
+            if bf16_c:
+                sp24_execute_bf16out(self.handle, transb, transc, N, d_b, ldb, bias, beta, d_c, ldc, stream)
+            else:
+                sp24_execute(self.handle, transb, transc, N, d_b, ldb, beta, d_c, ldc, stream)
+
+    def linear(self, x, bias=None, alpha=1.0):
+        """y = x . Aᵀ (+ bias), what torch.nn.functional.linear(x, W, bias) returns for the pruned weight W = A, in bf16.
+        x: a contiguous CUDA tensor whose last dimension is K -- bfloat16 for a bf16 operator, float8_e4m3fn / float8_e5m2
+        for an FP8 one, where alpha carries scale_x * scale_w.  bias: None or a CUDA bfloat16 tensor of M elements.
+        Returns y of shape x.shape[:-1] + (M,), bfloat16, on x's device; runs on torch.cuda.current_stream() with
+        transb = transc = 'T', N = x.numel() // K and ldb = K.  Inputs the library would refuse raise ValueError here,
+        and x is never copied or padded."""
+        import torch
+        if not isinstance(x, torch.Tensor):
+            raise ValueError("x must be a torch tensor, got %s" % type(x).__name__)
+        if self.fp8:
+            if x.dtype not in (torch.float8_e4m3fn, torch.float8_e5m2):
+                raise ValueError("an FP8 operator takes x as float8_e4m3fn or float8_e5m2, got %s" % x.dtype)
+        else:
+            if x.dtype != torch.bfloat16:
+                raise ValueError("a bf16 operator takes x as bfloat16, got %s" % x.dtype)
+            if alpha != 1.0:
+                raise ValueError("alpha=%r: alpha belongs to FP8 operators" % (alpha,))
+        if x.dim() < 1 or x.shape[-1] != self.K:
+            raise ValueError("x has shape %s: its last dimension must be K=%d" % (tuple(x.shape), self.K))
+        if not x.is_contiguous():
+            raise ValueError("x must be contiguous (its rows are read through TMA with pitch K)")
+        unit = 16 if self.fp8 else 8
+        if self.K % unit:
+            raise ValueError("K=%d must be a multiple of %d: x is read through TMA with pitch K, in whole 16-byte units"
+                             % (self.K, unit))
+        if x.data_ptr() % 16:
+            raise ValueError("x must start on a 16-byte boundary (it is read through TMA)")
+        if bias is not None:
+            if not isinstance(bias, torch.Tensor):
+                raise ValueError("bias must be a torch tensor, got %s" % type(bias).__name__)
+            _check_bias(bias, self.M)
+        if x.device.type != "cuda":
+            raise ValueError("x must be a CUDA tensor, got one on %s" % x.device)
+        if bias is not None and bias.device != x.device:
+            raise ValueError("bias is on %s, x on %s" % (bias.device, x.device))
+        N = x.numel() // self.K
+        y = torch.empty(tuple(x.shape[:-1]) + (self.M,), dtype=torch.bfloat16, device=x.device)
+        if N == 0:
+            return y
+        self.execute(x, y, N, ldb=self.K, ldc=self.M, transb="T", transc="T", stream=torch.cuda.current_stream(x.device),
+                     alpha=alpha, bias=bias)
+        check()
+        return y
 
     def destroy(self):
         if self.handle:
@@ -975,6 +1056,28 @@ def sp24_execute_fp8(handle, transb, transc, N, d_b, b_fmt, ldb, alpha, beta, d_
                   ctypes.c_float, ctypes.c_float, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
     s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
     f(handle, _c(transb), _c(transc), N, _dptr(d_b), b_fmt, ldb, float(alpha), float(beta), _dptr(d_c), ldc, s)
+
+
+def sp24_execute_bf16out(handle, transb, transc, N, d_b, ldb, bias, beta, d_c, ldc, stream=None):
+    """the raw bf16-output entry of a bf16 operator (arguments checked by the library, error -97); bias None or M bf16 values"""
+    L = load()
+    f = L.libxsmm_b200_sp24_execute_bf16out
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p, ctypes.c_char, ctypes.c_char, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p,
+                  ctypes.c_float, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
+    s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
+    f(handle, _c(transb), _c(transc), N, _dptr(d_b), ldb, _dptr(bias), float(beta), _dptr(d_c), ldc, s)
+
+
+def sp24_execute_fp8_bf16out(handle, transb, transc, N, d_b, b_fmt, ldb, alpha, bias, beta, d_c, ldc, stream=None):
+    """the raw bf16-output entry of an FP8 operator (arguments checked by the library, error -97); b_fmt 0 (e4m3) / 1 (e5m2)"""
+    L = load()
+    f = L.libxsmm_b200_sp24_execute_fp8_bf16out
+    f.restype = None
+    f.argtypes = [ctypes.c_void_p, ctypes.c_char, ctypes.c_char, ctypes.c_int, ctypes.c_void_p, ctypes.c_int, ctypes.c_int,
+                  ctypes.c_float, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p]
+    s = stream.cuda_stream if hasattr(stream, "cuda_stream") else _sptr(stream)
+    f(handle, _c(transb), _c(transc), N, _dptr(d_b), b_fmt, ldb, float(alpha), _dptr(bias), float(beta), _dptr(d_c), ldc, s)
 
 
 def sp24_destroy(handle):

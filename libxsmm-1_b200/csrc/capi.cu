@@ -1087,9 +1087,10 @@ libxsmm_b200_sp24* libxsmm_b200_sp24_create_fp8(int M, int K, int lda, const uns
   }
   return (libxsmm_b200_sp24*)sp24_create(M, K, lda, a, is_device_ptr(a), format);
 }
-// the execute checks both kinds share (b_format is checked for FP8 calls only).  true: the call has work to enqueue
+// the execute checks both kinds share (b_format is checked for FP8 calls only; d_c / d_bias alignment for bf16 C only).
+// true: the call has work to enqueue
 static bool sp24_execute_ok(const char* who, const Sp24Op* op, bool fp8, char transb, char transc, int N, const void* d_b, int b_format,
-                            int ldb, const float* d_c, int ldc)
+                            int ldb, const void* d_c, int ldc, bool bf16_c = false, const void* d_bias = 0)
 {
   if (0 == op) { set_error(-97, "%s: NULL handle", who); return false; }
   if (fp8 != (sp24_format(op) >= 0)) {
@@ -1115,6 +1116,10 @@ static bool sp24_execute_ok(const char* who, const Sp24Op* op, bool fp8, char tr
     set_error(-97, "%s: d_b=%p must be 16-byte aligned and ldb=%d a multiple of %d (B is read through TMA)", who, d_b, ldb, ldb_unit);
     return false;
   }
+  if (bf16_c && (0 != ((uintptr_t)d_c & 1) || 0 != ((uintptr_t)d_bias & 1))) {
+    set_error(-97, "%s: d_c=%p and d_bias=%p must be 2-byte aligned (bf16 elements)", who, d_c, d_bias);
+    return false;
+  }
   int dev = -1;
   if (cudaSuccess != cudaGetDevice(&dev)) { (void)cudaGetLastError(); dev = -1; }
   if (dev != sp24_device(op)) { set_error(-97, "%s: current device %d, the operator was created on device %d", who, dev, sp24_device(op)); return false; }
@@ -1133,6 +1138,23 @@ void libxsmm_b200_sp24_execute_fp8(const libxsmm_b200_sp24* handle, char transb,
   const Sp24Op* op = (const Sp24Op*)handle;
   if (!sp24_execute_ok("sp24_execute_fp8", op, true, transb, transc, N, d_b, b_format, ldb, d_c, ldc)) return;
   sp24_execute_fp8(op, is_t(transb), is_t(transc), N, d_b, b_format, ldb, alpha, beta, d_c, ldc, (cudaStream_t)stream);
+}
+void libxsmm_b200_sp24_execute_bf16out(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const libxsmm_bfloat16* d_b, int ldb, const libxsmm_bfloat16* d_bias, float beta, libxsmm_bfloat16* d_c, int ldc, void* stream)
+{
+  const Sp24Op* op = (const Sp24Op*)handle;
+  if (!sp24_execute_ok("sp24_execute_bf16out", op, false, transb, transc, N, d_b, -2, ldb, d_c, ldc, true, d_bias)) return;
+  sp24_execute_bf16out(op, is_t(transb), is_t(transc), N, (const uint16_t*)d_b, ldb, (const uint16_t*)d_bias, beta, (uint16_t*)d_c, ldc,
+                       (cudaStream_t)stream);
+}
+void libxsmm_b200_sp24_execute_fp8_bf16out(const libxsmm_b200_sp24* handle, char transb, char transc, int N,
+  const unsigned char* d_b, int b_format, int ldb, float alpha, const libxsmm_bfloat16* d_bias, float beta,
+  libxsmm_bfloat16* d_c, int ldc, void* stream)
+{
+  const Sp24Op* op = (const Sp24Op*)handle;
+  if (!sp24_execute_ok("sp24_execute_fp8_bf16out", op, true, transb, transc, N, d_b, b_format, ldb, d_c, ldc, true, d_bias)) return;
+  sp24_execute_fp8_bf16out(op, is_t(transb), is_t(transc), N, d_b, b_format, ldb, alpha, (const uint16_t*)d_bias, beta, (uint16_t*)d_c, ldc,
+                           (cudaStream_t)stream);
 }
 void libxsmm_b200_sp24_destroy(libxsmm_b200_sp24* handle) { sp24_destroy((Sp24Op*)handle); }
 

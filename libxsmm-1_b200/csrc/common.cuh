@@ -289,6 +289,10 @@ Sp24Op* sp24_create(int M, int K, int lda, const void* a, bool a_on_device, int 
 void sp24_execute(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, float beta, float* d_c, int ldc, cudaStream_t stream);
 void sp24_execute_fp8(const Sp24Op* op, bool transb, bool transc, int N, const unsigned char* d_b, int b_format, int ldb, float alpha, float beta,
                       float* d_c, int ldc, cudaStream_t stream);
+void sp24_execute_bf16out(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, const uint16_t* d_bias, float beta,
+                          uint16_t* d_c, int ldc, cudaStream_t stream);
+void sp24_execute_fp8_bf16out(const Sp24Op* op, bool transb, bool transc, int N, const unsigned char* d_b, int b_format, int ldb, float alpha,
+                              const uint16_t* d_bias, float beta, uint16_t* d_c, int ldc, cudaStream_t stream);
 int sp24_format(const Sp24Op* op);
 int sp24_device(const Sp24Op* op);
 int sp24_rows(const Sp24Op* op);

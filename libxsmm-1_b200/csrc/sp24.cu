@@ -18,6 +18,9 @@
 // (tools/umma_probe/probe_sp8.cu): [column half][128 lanes][16 bytes], copied with two tcgen05.cp.  An MN-major ('N') 8-bit B
 // of 128 columns is two 64-byte SWIZZLE_64B blocks, so that the half tile's 64 columns per CTA are one block as in bf16.
 // The epilogue scales the accumulator by alpha (the per-tensor scales of A and B) before beta C is added.
+// OB (the *_bf16out entries) changes the epilogue only: v = alpha acc (F8), + bias[m] (one fp32 addition, none for a NULL
+// bias), fmaf(beta, C_old, v), rounded to bf16 to nearest even in pairs.  Its TMA store stages two 32-column chunks as one box
+// of 32 rows x 64 bf16 (128-byte rows, SWIZZLE_128B): the fp32 box's size and staging layout, half as many boxes per tile.
 #include "common.cuh"
 #include "tc_common.cuh"
 
@@ -61,11 +64,27 @@ struct Sp24F8Args : Sp24Args {
   float alpha;
   uint32_t idesc_fmt;   // instruction-descriptor bits of the A and B formats
 };
+// bf16 C (OB): c holds the address of the bf16 C, c_vec means 16-byte stores of 8 elements
+template <typename Base> struct Sp24OutArgs : Base {
+  const unsigned short* bias;   // NULL or M bf16 values, indexed by A's row
+};
+template <bool F8, bool OB> using Sp24KArgs =
+  typename std::conditional<OB, Sp24OutArgs<typename std::conditional<F8, Sp24F8Args, Sp24Args>::type>,
+                            typename std::conditional<F8, Sp24F8Args, Sp24Args>::type>::type;
 
-template <bool TB, bool F8>
+// two fp32 values rounded to bf16 (nearest even; NaN stays NaN, overflow gives +-Inf): lo in bits 0..15, hi in 16..31
+__device__ __forceinline__ uint32_t bf16x2_rn(float lo, float hi)
+{
+  uint32_t r;
+  asm("cvt.rn.bf16x2.f32 %0, %1, %2;\n" : "=r"(r) : "f"(hi), "f"(lo));
+  return r;
+}
+__device__ __forceinline__ float bf16_value(unsigned short h) { return __uint_as_float((uint32_t)h << 16); }
+
+template <bool TB, bool F8, bool OB>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(F_THREADS, 1)
 sp24_compute_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmE, const __grid_constant__ CUtensorMap tmB,
-                    const __grid_constant__ CUtensorMap tmC, const int c_tma, const typename std::conditional<F8, Sp24F8Args, Sp24Args>::type p)
+                    const __grid_constant__ CUtensorMap tmC, const int c_tma, const Sp24KArgs<F8, OB> p)
 {
   using G = Sp24Geo<F8>;
   constexpr int F_KB = G::KB, F_META = G::META;
@@ -214,6 +233,10 @@ sp24_compute_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       mbar_wait(&acc_full[acc], ((uint32_t)wi >> 1) & 1u);
       tc_fence_after();
       const size_t crow = (size_t)ct * F_BM + (size_t)row;
+      float bias_v = 0.f;      // OB: the row is fixed for the tile, so its bias is loaded once
+      if constexpr (OB) {
+        if (0 != p.bias && rvalid) bias_v = bf16_value(__ldg(p.bias + crow));
+      }
 #pragma unroll 1
       for (int cb = 0; cb < ncw; cb += 32) {
         uint32_t v[32];
@@ -222,12 +245,94 @@ sp24_compute_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
           for (int jj = 0; jj < 32; ++jj) v[jj] = __float_as_uint(p.alpha * __uint_as_float(v[jj]));
         }
+        if constexpr (OB) {    // a separate rounded addition (never contracted with alpha's multiply); none without a bias, so -0 stays
+          if (0 != p.bias) {
+#pragma unroll
+            for (int jj = 0; jj < 32; ++jj) v[jj] = __float_as_uint(__fadd_rn(__uint_as_float(v[jj]), bias_v));
+          }
+        }
         if (0 == cb) {         // columns 0..31 of this accumulator are read: the next tile's metadata may go there
           tc_fence_before();
           __syncwarp();
           if (0 == lane) mbar_arrive_cluster(lead_meta);
         }
-        if (use_tma) {
+        if constexpr (OB) {
+          unsigned short* const cc = (unsigned short*)p.c;
+          if (use_tma) {
+            // beta = 0: chunk pairs (cb, cb + 32) share one box of 32 rows x 64 bf16; chunk h fills 16-byte units 4h .. 4h + 3
+            // of each 128-byte row (XOR row % 8, SWIZZLE_128B), the second chunk stores the box
+            const int h = (cb >> 5) & 1;
+            unsigned char* sbox = stage;
+            if (wi == nwork - 1) sbox = smem + F_SMEM_A + ((warp - 2) * (F_BN / 64) + (cb >> 6)) * F_STAGE;
+            else if (0 == h) {
+              if (0 == lane) asm volatile("cp.async.bulk.wait_group.read 0;\n" ::: "memory");
+              __syncwarp();
+            }
+#pragma unroll
+            for (int u = 0; u < 4; ++u)
+              *(uint4*)(sbox + lane * 128 + (((4 * h + u) ^ (lane & 7)) << 4)) =
+                make_uint4(bf16x2_rn(__uint_as_float(v[8 * u]), __uint_as_float(v[8 * u + 1])), bf16x2_rn(__uint_as_float(v[8 * u + 2]), __uint_as_float(v[8 * u + 3])),
+                           bf16x2_rn(__uint_as_float(v[8 * u + 4]), __uint_as_float(v[8 * u + 5])), bf16x2_rn(__uint_as_float(v[8 * u + 6]), __uint_as_float(v[8 * u + 7])));
+            if (h) {
+              fence_proxy_async();
+              __syncwarp();
+              if (0 == lane) {
+                asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%1, %2}], [%3];\n"
+                             ::"l"(&tmC), "r"(n0 + cb - 32), "r"((int)(crow - (size_t)lane)), "r"(smem_u32(sbox)) : "memory");
+                asm volatile("cp.async.bulk.commit_group;\n" ::: "memory");
+              }
+            }
+          }
+          else if (rvalid) {
+            if (p.transc) {    // lanes hold consecutive m: per column the warp writes 64 contiguous bytes
+              if (0.f != p.beta) {
+#pragma unroll
+                for (int jj = 0; jj < 32; ++jj) {
+                  const int col = n0 + cb + jj;
+                  if (col < p.N) v[jj] = __float_as_uint(fmaf(p.beta, bf16_value(cc[(size_t)col * p.ldc + crow]), __uint_as_float(v[jj])));
+                }
+              }
+#pragma unroll
+              for (int jj = 0; jj < 32; jj += 2) {
+                const uint32_t w = bf16x2_rn(__uint_as_float(v[jj]), __uint_as_float(v[jj + 1]));
+                const int col = n0 + cb + jj;
+                if (col < p.N) cc[(size_t)col * p.ldc + crow] = (unsigned short)w;
+                if (col + 1 < p.N) cc[(size_t)(col + 1) * p.ldc + crow] = (unsigned short)(w >> 16);
+              }
+            }
+            else {             // 16-byte units of 8 bf16 where C allows them, element stores at the ragged end
+              unsigned short* dst = cc + crow * p.ldc + n0 + cb;
+#pragma unroll
+              for (int jj = 0; jj < 32; jj += 8) {
+                const int col = n0 + cb + jj;
+                const bool vec = p.c_vec && col + 7 < p.N;
+                if (0.f != p.beta) {
+                  if (vec) {
+                    const uint4 cin = *(const uint4*)(dst + jj);
+                    const uint32_t cw[4] = { cin.x, cin.y, cin.z, cin.w };
+#pragma unroll
+                    for (int t2 = 0; t2 < 8; ++t2)
+                      v[jj + t2] = __float_as_uint(fmaf(p.beta, bf16_value((unsigned short)(cw[t2 >> 1] >> (16 * (t2 & 1)))), __uint_as_float(v[jj + t2])));
+                  }
+                  else {
+#pragma unroll
+                    for (int t2 = 0; t2 < 8; ++t2)
+                      if (col + t2 < p.N) v[jj + t2] = __float_as_uint(fmaf(p.beta, bf16_value(dst[jj + t2]), __uint_as_float(v[jj + t2])));
+                  }
+                }
+                uint32_t w[4];
+#pragma unroll
+                for (int t2 = 0; t2 < 4; ++t2) w[t2] = bf16x2_rn(__uint_as_float(v[jj + 2 * t2]), __uint_as_float(v[jj + 2 * t2 + 1]));
+                if (vec) st_global_cs_f4((float*)(dst + jj), make_float4(__uint_as_float(w[0]), __uint_as_float(w[1]), __uint_as_float(w[2]), __uint_as_float(w[3])));
+                else {
+#pragma unroll
+                  for (int t2 = 0; t2 < 8; ++t2) if (col + t2 < p.N) dst[jj + t2] = (unsigned short)(w[t2 >> 1] >> (16 * (t2 & 1)));
+                }
+              }
+            }
+          }
+        }
+        else if (use_tma) {
           // as K4s: one box per warp, except in the pair's last tile, whose chunks each get a box in the idle ring
           unsigned char* sbox = stage;
           if (wi == nwork - 1) sbox = smem + F_SMEM_A + ((warp - 2) * (F_BN / 32) + (cb >> 5)) * F_STAGE;
@@ -435,29 +540,31 @@ void sp24_destroy(Sp24Op* op)
   delete op;
 }
 
-template <bool TB, bool F8, typename Args>
+template <bool TB, bool F8, bool OB, typename Args>
 static void launch_sp24(const Sp24Op* op, const CUtensorMap& mB, const CUtensorMap& mC, int c_tma, const Args& p, int pairs, cudaStream_t stream)
 {
-  ensure_smem_optin((const void*)sp24_compute_kernel<TB, F8>, Sp24Geo<F8>::SMEM_BYTES);
+  ensure_smem_optin((const void*)sp24_compute_kernel<TB, F8, OB>, Sp24Geo<F8>::SMEM_BYTES);
   count_launch(1);
-  note_compute_kernel(F8 ? "sp24_compute_kernel_fp8" : "sp24_compute_kernel");
-  sp24_compute_kernel<TB, F8><<<dim3(2u * (unsigned)pairs), dim3(F_THREADS), Sp24Geo<F8>::SMEM_BYTES, stream>>>(op->tmA, op->tmE, mB, mC, c_tma, p);
+  note_compute_kernel(OB ? (F8 ? "sp24_compute_kernel_fp8_bf16out" : "sp24_compute_kernel_bf16out") : (F8 ? "sp24_compute_kernel_fp8" : "sp24_compute_kernel"));
+  sp24_compute_kernel<TB, F8, OB><<<dim3(2u * (unsigned)pairs), dim3(F_THREADS), Sp24Geo<F8>::SMEM_BYTES, stream>>>(op->tmA, op->tmE, mB, mC, c_tma, p);
   XB_CUDA(cudaGetLastError());
 }
 
-// the part of the launch both kinds share: C's tensor map and the fields of Sp24Args.  false: B's map was refused (-97 set)
-static bool sp24_prepare(const Sp24Op* op, bool okb, bool transc, int N, int ldb, float beta, float* d_c, int ldc, int kb,
+// the part of the launch both kinds share: C's tensor map and the fields of Sp24Args (c_esz: 4 fp32 C, 2 bf16 C).
+// false: B's map was refused (-97 set)
+static bool sp24_prepare(const Sp24Op* op, bool okb, bool transc, int N, int ldb, float beta, void* d_c, int ldc, int c_esz, int kb,
                          CUtensorMap& mB, CUtensorMap& mC, int& c_tma, Sp24Args& p, int& pairs)
 {
   if (!okb) { set_error(-97, "sp24_execute: B (N=%d, ldb=%d) cannot be described by a tensor map", N, ldb); return false; }
-  // C leaves through TMA boxes of 32 x 32 when it is only written and stored row-major, with whole 16-byte units per row
-  // (a store box is clipped at the last column only to 16 bytes, DESIGN.md section 2)
-  const bool c_vec = !transc && 0 == ((uintptr_t)d_c & 15) && 0 == (ldc & 3);
+  // C leaves through TMA boxes of 32 rows x 128 bytes when it is only written and stored row-major, with whole 16-byte units
+  // per row (a store box is clipped at the last column only to 16 bytes, DESIGN.md section 2)
+  const bool c_vec = !transc && 0 == ((uintptr_t)d_c & 15) && 0 == (((long long)ldc * c_esz) & 15);
   c_tma = 0;
   mC = mB;
-  if (c_vec && 0.f == beta && 0 == (N & 3) && make_tensor_map_2d_sw128(&mC, d_c, 4, (unsigned long long)N, (unsigned long long)op->M, (unsigned long long)ldc * 4, 32, 32, false)) c_tma = 1;
+  if (c_vec && 0.f == beta && 0 == (((long long)N * c_esz) & 15) &&
+      make_tensor_map_2d_sw128(&mC, d_c, c_esz, (unsigned long long)N, (unsigned long long)op->M, (unsigned long long)ldc * c_esz, 128 / c_esz, 32, false)) c_tma = 1;
   else mC = mB;
-  p.c = d_c; p.ldc = ldc; p.M = op->M; p.N = N; p.nkb = op->K_pad / kb; p.ctiles_m = op->M_pad / F_BM; p.beta = beta;
+  p.c = (float*)d_c; p.ldc = ldc; p.M = op->M; p.N = N; p.nkb = op->K_pad / kb; p.ctiles_m = op->M_pad / F_BM; p.beta = beta;
   p.transc = transc ? 1 : 0; p.c_vec = c_vec ? 1 : 0;
   const int pairs_max = device_sm_count() / 2 > 0 ? device_sm_count() / 2 : 1;
   const int total = ((p.ctiles_m + 1) / 2) * ((N + F_BN - 1) / F_BN);
@@ -465,34 +572,74 @@ static bool sp24_prepare(const Sp24Op* op, bool okb, bool transc, int N, int ldb
   return true;
 }
 
+static bool sp24_map_b_bf16(CUtensorMap& mB, const Sp24Op* op, bool transb, int N, const uint16_t* d_b, int ldb)
+{
+  return transb ? make_tensor_map_2d_sw128(&mB, d_b, 2, (unsigned long long)op->K, (unsigned long long)N, (unsigned long long)ldb * 2, 64, 64, false)
+                : make_tensor_map_2d_sw128(&mB, d_b, 2, (unsigned long long)N, (unsigned long long)op->K, (unsigned long long)ldb * 2, 64, Sp24Geo<false>::KB, false);
+}
+
+// FP8: B is read as bytes, 'T' in 128-byte boxes of k (SWIZZLE_128B), 'N' in 64-column boxes (SWIZZLE_64B)
+static bool sp24_map_b_fp8(CUtensorMap& mB, const Sp24Op* op, bool transb, int N, const unsigned char* d_b, int ldb)
+{
+  return transb ? make_tensor_map_2d_u8(&mB, d_b, (unsigned long long)op->K, (unsigned long long)N, (unsigned long long)ldb, 128, 64, 128)
+                : make_tensor_map_2d_u8(&mB, d_b, (unsigned long long)N, (unsigned long long)op->K, (unsigned long long)ldb, 64, Sp24Geo<true>::KB, 64);
+}
+
 // arguments checked by the caller (capi.cu); N > 0
 void sp24_execute(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, float beta, float* d_c, int ldc, cudaStream_t stream)
 {
   CUtensorMap mB, mC;
-  const bool okb = transb ? make_tensor_map_2d_sw128(&mB, d_b, 2, (unsigned long long)op->K, (unsigned long long)N, (unsigned long long)ldb * 2, 64, 64, false)
-                          : make_tensor_map_2d_sw128(&mB, d_b, 2, (unsigned long long)N, (unsigned long long)op->K, (unsigned long long)ldb * 2, 64, Sp24Geo<false>::KB, false);
+  const bool okb = sp24_map_b_bf16(mB, op, transb, N, d_b, ldb);
   Sp24Args p;
   int c_tma = 0, pairs = 0;
-  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, Sp24Geo<false>::KB, mB, mC, c_tma, p, pairs)) return;
-  if (transb) launch_sp24<true, false>(op, mB, mC, c_tma, p, pairs, stream);
-  else launch_sp24<false, false>(op, mB, mC, c_tma, p, pairs, stream);
+  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, 4, Sp24Geo<false>::KB, mB, mC, c_tma, p, pairs)) return;
+  if (transb) launch_sp24<true, false, false>(op, mB, mC, c_tma, p, pairs, stream);
+  else launch_sp24<false, false, false>(op, mB, mC, c_tma, p, pairs, stream);
 }
 
-// FP8: B is read as bytes, 'T' in 128-byte boxes of k (SWIZZLE_128B), 'N' in 64-column boxes (SWIZZLE_64B); N > 0
 void sp24_execute_fp8(const Sp24Op* op, bool transb, bool transc, int N, const unsigned char* d_b, int b_format, int ldb, float alpha, float beta,
                       float* d_c, int ldc, cudaStream_t stream)
 {
   constexpr int KB = Sp24Geo<true>::KB;
   CUtensorMap mB, mC;
-  const bool okb = transb ? make_tensor_map_2d_u8(&mB, d_b, (unsigned long long)op->K, (unsigned long long)N, (unsigned long long)ldb, 128, 64, 128)
-                          : make_tensor_map_2d_u8(&mB, d_b, (unsigned long long)N, (unsigned long long)op->K, (unsigned long long)ldb, 64, KB, 64);
+  const bool okb = sp24_map_b_fp8(mB, op, transb, N, d_b, ldb);
   Sp24F8Args p;
   int c_tma = 0, pairs = 0;
-  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, KB, mB, mC, c_tma, p, pairs)) return;
+  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, 4, KB, mB, mC, c_tma, p, pairs)) return;
   p.alpha = alpha;
   p.idesc_fmt = ((uint32_t)op->format << 7) | ((uint32_t)b_format << 10);
-  if (transb) launch_sp24<true, true>(op, mB, mC, c_tma, p, pairs, stream);
-  else launch_sp24<false, true>(op, mB, mC, c_tma, p, pairs, stream);
+  if (transb) launch_sp24<true, true, false>(op, mB, mC, c_tma, p, pairs, stream);
+  else launch_sp24<false, true, false>(op, mB, mC, c_tma, p, pairs, stream);
+}
+
+// bf16 C with an optional per-row bias (d_bias: NULL or M bf16 values); arguments checked by capi.cu; N > 0
+void sp24_execute_bf16out(const Sp24Op* op, bool transb, bool transc, int N, const uint16_t* d_b, int ldb, const uint16_t* d_bias, float beta,
+                          uint16_t* d_c, int ldc, cudaStream_t stream)
+{
+  CUtensorMap mB, mC;
+  const bool okb = sp24_map_b_bf16(mB, op, transb, N, d_b, ldb);
+  Sp24OutArgs<Sp24Args> p;
+  int c_tma = 0, pairs = 0;
+  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, 2, Sp24Geo<false>::KB, mB, mC, c_tma, p, pairs)) return;
+  p.bias = d_bias;
+  if (transb) launch_sp24<true, false, true>(op, mB, mC, c_tma, p, pairs, stream);
+  else launch_sp24<false, false, true>(op, mB, mC, c_tma, p, pairs, stream);
+}
+
+void sp24_execute_fp8_bf16out(const Sp24Op* op, bool transb, bool transc, int N, const unsigned char* d_b, int b_format, int ldb, float alpha,
+                              const uint16_t* d_bias, float beta, uint16_t* d_c, int ldc, cudaStream_t stream)
+{
+  constexpr int KB = Sp24Geo<true>::KB;
+  CUtensorMap mB, mC;
+  const bool okb = sp24_map_b_fp8(mB, op, transb, N, d_b, ldb);
+  Sp24OutArgs<Sp24F8Args> p;
+  int c_tma = 0, pairs = 0;
+  if (!sp24_prepare(op, okb, transc, N, ldb, beta, d_c, ldc, 2, KB, mB, mC, c_tma, p, pairs)) return;
+  p.alpha = alpha;
+  p.idesc_fmt = ((uint32_t)op->format << 7) | ((uint32_t)b_format << 10);
+  p.bias = d_bias;
+  if (transb) launch_sp24<true, true, true>(op, mB, mC, c_tma, p, pairs, stream);
+  else launch_sp24<false, true, true>(op, mB, mC, c_tma, p, pairs, stream);
 }
 
 }  // namespace xb
